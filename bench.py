@@ -1,6 +1,6 @@
 """bench.py -- CTC fwd+bwd frames/s on B200 (BASELINE.json metric), one JSON line on stdout.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--workload C3] [--impl b200|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--workload C3] [--impl b200|reference] [--dump-outputs DIR]
 
 A "step" is one fused loss+gradient evaluation of one mini-batch of synthetic logits of the named shape:
 three kernels (plan -> softmax rows -> lattice, whose last CTA also sums the costs; the backward of the op is
@@ -33,6 +33,7 @@ UNIT = "frames/s"
 N_ROTATE = 16          # distinct acts/grads buffer sets cycled through the timed loop (> L2 in total)
 GROUP = 8              # steps per CUDA graph (and per all-reduce message at N > 1); 4 per graph measured 3 % slower on C3
 MIN_REGION_MS = 50.0   # N > 1: a timed region shorter than this is repeated until it adds up to it
+DUMP_GRAD_ELEMS = 1 << 23   # --dump-outputs: a larger gradient is written as this many sampled elements (32 MB)
 
 
 def parse():
@@ -44,6 +45,8 @@ def parse():
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip per_config / decoder / sharded_c5 (profiling runs)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed step to DIR/<name>.npy (see dump_outputs)")
     return ap.parse_args()
 
 
@@ -236,6 +239,24 @@ def _slice(wl, nb):
     return wl.labels[:L], wl.act_lens[:nb], wl.label_lens[:nb]
 
 
+def dump_outputs(out_dir, costs, loss_sum, grads):
+    """--dump-outputs: what a caller of the timed path receives from its last step, as float32 .npy files:
+    costs[B], loss_sum[1] and grads[T,B,V].  A gradient of more than DUMP_GRAD_ELEMS elements is written as
+    grads_sample.npy, its flat elements at np.sort(np.random.default_rng(0).choice(numel, DUMP_GRAD_ELEMS,
+    replace=False)), so that two builds run with the same arguments can be compared output for output."""
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"costs": costs, "loss_sum": loss_sum}
+    grads = torch.as_tensor(grads)
+    if grads.numel() <= DUMP_GRAD_ELEMS:
+        arrays["grads"] = grads
+    else:
+        idx = np.sort(np.random.default_rng(0).choice(grads.numel(), DUMP_GRAD_ELEMS, replace=False))
+        arrays["grads_sample"] = grads.reshape(-1)[torch.from_numpy(idx).to(grads.device)]
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), torch.as_tensor(a).detach().cpu().numpy().astype(np.float32))
+
+
 def run_reference(args):
     """--impl reference: the reference's CPU implementation of the path.  warp-ctc itself is not in
     /root/reference (un-vendored, un-pinned), so the oracle's C++/OpenMP port is timed, with all the
@@ -253,8 +274,10 @@ def run_reference(args):
         ctc_cpu.ctc_cpu(acts, wl.labels, wl.act_lens, wl.label_lens, precision="f32", num_threads=threads)
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        ctc_cpu.ctc_cpu(acts, wl.labels, wl.act_lens, wl.label_lens, precision="f32", num_threads=threads)
+        costs, grads = ctc_cpu.ctc_cpu(acts, wl.labels, wl.act_lens, wl.label_lens, precision="f32", num_threads=threads)
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, costs, np.array([costs.sum(dtype=np.float64)]), grads)
     value = frames * args.steps / dt
     total, strict, _ = workloads.algorithmic_bytes(wl)
     print(json.dumps({
@@ -305,6 +328,7 @@ class Runner:
         self.loss_groups = [torch.zeros(self.group, device=dev) for _ in range(2)]
         self.pending = [None, None]
         self.n_groups_done = 0
+        self.last_step = None                 # (buffer set, loss group, slot) of the last step run()
         self.graphs = None
         self.launches_per_step = 3            # plan, softmax rows, lattice (+ cost sum in its last CTA)
         # long steps (C4, C5: two buffer sets, 0.7-0.9 ms per step) are issued eagerly: the host needs ~0.02 ms per
@@ -357,6 +381,8 @@ class Runner:
         full, rest = divmod(steps, self.group)
         for _ in range(full):
             self._group(self.n_groups_done, eager)
+            self.last_step = ((self.n_groups_done * self.group + self.group - 1) % self.n_rot, self.n_groups_done % 2,
+                              self.group - 1)
             self.n_groups_done += 1
         if rest:
             g = self.n_groups_done % 2
@@ -367,6 +393,7 @@ class Runner:
                 self.one((self.n_groups_done * self.group + k) % self.n_rot, self.loss_groups[g][k:k + 1])
             if self.world > 1:
                 self.pending[g] = dist.all_reduce(self.loss_groups[g], async_op=True)
+            self.last_step = ((self.n_groups_done * self.group + rest - 1) % self.n_rot, g, rest - 1)
             self.n_groups_done += 1
 
     def drain(self):
@@ -627,6 +654,10 @@ def main():
         host_wall = (time.perf_counter() - t_host0) * 1e3 / repeats
     host_ms_per_step = host_wall / args.steps
     sampler.active.clear()
+    if args.dump_outputs and rank == 0:
+        # before any later pass rewrites the shared costs buffer, the loss slots or the gradient buffers
+        j, g, k = runner.last_step
+        dump_outputs(args.dump_outputs, runner.costs, runner.loss_groups[g][k:k + 1], runner.grads_dev[j])
 
     def agree_min(n):
         # every rank must take the same branch below: the extra steps contain collectives
@@ -812,4 +843,5 @@ def main():
 
 
 if __name__ == "__main__":
+    sys.dont_write_bytecode = True        # running the benchmark adds no __pycache__ to the source tree
     main()

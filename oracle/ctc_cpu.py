@@ -6,7 +6,9 @@ compiled with the host compiler: ``g++ -O3 -march=native -fopenmp -shared -fPIC`
 
 import ctypes
 import os
+import shutil
 import subprocess
+import tempfile
 
 import numpy as np
 
@@ -16,19 +18,31 @@ LIB = os.path.join(_DIR, "liboracle_ctc.so")
 _lib = None
 
 
-def build(force=False):
-    if force or not os.path.exists(LIB) or os.path.getmtime(LIB) < os.path.getmtime(SRC):
+def _stale(path):
+    return not os.path.exists(path) or os.path.getmtime(path) < os.path.getmtime(SRC)
+
+
+def build(force=False, out=LIB):
+    if force or _stale(out):
         subprocess.run(["g++", "-O3", "-march=native", "-std=c++17", "-fopenmp", "-shared", "-fPIC",
-                        SRC, "-o", LIB], check=True)
-    return LIB
+                        SRC, "-o", out], check=True)
+    return out
 
 
 def load():
     global _lib
     if _lib is None:
         # -march=native code built elsewhere may not run here: rebuild when the host differs
-        build()
-        lib = ctypes.CDLL(LIB)
+        if _stale(LIB):
+            # only build() writes into the source tree: a missing or stale library is compiled into a
+            # temporary directory (the tree may be read-only), loaded, and the directory removed
+            tmp = tempfile.mkdtemp(prefix="oracle_ctc_")
+            try:
+                lib = ctypes.CDLL(build(out=os.path.join(tmp, "liboracle_ctc.so")))
+            finally:
+                shutil.rmtree(tmp, ignore_errors=True)
+        else:
+            lib = ctypes.CDLL(LIB)
         fp = ctypes.POINTER(ctypes.c_float)
         ip = ctypes.POINTER(ctypes.c_int)
         for name in ("oracle_ctc_cpu_f32", "oracle_ctc_cpu_f64"):
