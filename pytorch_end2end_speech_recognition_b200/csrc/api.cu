@@ -144,13 +144,14 @@ int status_of(cudaError_t e) {
 int run_kernels(b200ctc_handle* h, CallParams& p, int max_L, cudaStream_t stream) {
   h->last_flags = p.flags;
   h->last_B = p.B;
-  cudaError_t e = prepare_lattice(p, max_L);
+  LatticeCfg lattice;
+  cudaError_t e = prepare_lattice(p, max_L, &lattice);
   if (e != cudaSuccess) return status_of(e);
   const bool prof = h->profiling;
   if (prof) cudaEventRecord(h->prof[0], stream);
   e = launch_softmax_rows(p, stream);
   if (prof) cudaEventRecord(h->prof[1], stream);
-  if (e == cudaSuccess) e = launch_lattice(p, max_L, stream);
+  if (e == cudaSuccess) e = launch_lattice(p, lattice, stream);
   if (prof) cudaEventRecord(h->prof[2], stream);
   if (e == cudaSuccess && p.gathered && p.grads) e = launch_apply_occupancy(p, stream);
   if (prof) {

@@ -91,10 +91,17 @@ __host__ __device__ inline int groups_of(int L) {
 }
 __host__ __device__ inline int em_width_of(int L) { return (L + 1 + 3) / 4 * 4; }
 
+// Launch geometry of the lattice kernel for one call (lattice.cu: prepare_lattice).
+struct LatticeCfg {
+  int nwmax, l_cap, depth;   // lattice windows per sweep (1, 2, 4); longest label sequence of the fast lattice; record ring depth
+  size_t smem;               // dynamic shared memory per CTA
+  bool cluster;              // two CTAs per utterance (lattice_cluster_kernel)
+};
+
 // host launchers (each in its own .cu)
 cudaError_t launch_softmax_rows(const CallParams& p, cudaStream_t stream);
-cudaError_t prepare_lattice(CallParams& p, int max_L);     // fills fast_l_cap and oth_depth; error when not even the safe lattice fits
-cudaError_t launch_lattice(const CallParams& p, int max_L, cudaStream_t stream);
+cudaError_t prepare_lattice(CallParams& p, int max_L, LatticeCfg* cfg);   // also fills fast_l_cap and oth_depth; error when not even the safe lattice fits
+cudaError_t launch_lattice(const CallParams& p, const LatticeCfg& cfg, cudaStream_t stream);
 cudaError_t launch_apply_occupancy(const CallParams& p, cudaStream_t stream);
 cudaError_t launch_plan(const CallParams& p, UttMeta* meta, int* order, int* flags, cudaStream_t stream);
 size_t edit_distance_workspace_bytes(int B, int max_ref, int max_hyp);

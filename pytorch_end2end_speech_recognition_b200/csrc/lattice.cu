@@ -10,8 +10,6 @@ namespace b200ctc {
 
 namespace {
 
-constexpr int kChunk = 4;  // frames between halo exchanges (K)
-
 // What every utterance ends with (the CTA that owns it; at least 128 threads): the label-smoothing term of the
 // utterance and, in the CTA that finishes last, the fixed-order sum of the costs (K3).
 __device__ void utterance_tail(const CallParams& p, int b, const UttMeta& m, unsigned char* smem) {
@@ -67,10 +65,10 @@ __device__ void utterance_tail(const CallParams& p, int b, const UttMeta& m, uns
 }
 
 // One CTA per utterance, longest lattice first (p.order): per side NWMAX lattice warps and kReducers
-// reducer warps (lattice_fast.cuh); NS lattice states per lane.  The block-exponent fast path runs unless
+// reducer warps (lattice_fast.cuh).  The block-exponent fast path runs unless
 // the utterance was flagged by K1 or is too long for the lattice window; when the fast path gives
 // up (range lost, zero probability) the same CTA redoes the utterance with the fp64 safe path.
-template <int K, int NWMAX, int NS>
+template <int NWMAX>
 __global__ void __launch_bounds__(2 * (NWMAX + kReducers) * 32, 1) lattice_kernel(CallParams p) {
   extern __shared__ __align__(16) unsigned char smem[];
   pdl_launch_dependents();   // the plan kernel of the next device-resident call may run underneath this kernel (plan.cu)
@@ -92,7 +90,7 @@ __global__ void __launch_bounds__(2 * (NWMAX + kReducers) * 32, 1) lattice_kerne
     if (!use_safe) {
       // prologue (no K1 output needed), then wait for K1, then the sweeps -- unless K1 flagged an extreme row
       int* abort_word = nullptr;
-      lattice_fast_utterance<K, NWMAX, NS>(p, b, smem, &abort_word);
+      lattice_fast_utterance<NWMAX>(p, b, smem, &abort_word);
       __syncthreads();
       const int why = *abort_word;
       use_safe = why != 0;
@@ -125,7 +123,7 @@ __global__ void __launch_bounds__(2 * (NWMAX + kReducers) * 32, 1) lattice_kerne
 // SMs idle.  The sides meet once, at the midpoint (a cluster barrier: everything phase 1 stored is visible to the
 // other SM afterwards), and compare their abort words through distributed shared memory at the end; the CTA of
 // rank 0 owns the utterance-level duties (safe lattice, flags, the tail).
-template <int K, int NWMAX, int NS>
+template <int NWMAX>
 __global__ void __launch_bounds__(cluster_block_warps<NWMAX>() * 32, 1) lattice_cluster_kernel(CallParams p) {
   extern __shared__ __align__(16) unsigned char smem[];
   pdl_launch_dependents();
@@ -142,7 +140,7 @@ __global__ void __launch_bounds__(cluster_block_warps<NWMAX>() * 32, 1) lattice_
     bool dirty = false;
     if (!use_safe) {
       int* abort_word = nullptr;
-      lattice_fast_utterance<K, NWMAX, NS, true>(p, b, smem, &abort_word);
+      lattice_fast_utterance<NWMAX, true>(p, b, smem, &abort_word);
       __syncthreads();
       cluster_sync_all();                                   // both sweeps are over, both abort words final
       const int why = *abort_word | ld_peer_s32(abort_word, rank ^ 1u);
@@ -171,32 +169,6 @@ __global__ void __launch_bounds__(cluster_block_warps<NWMAX>() * 32, 1) lattice_
 
 constexpr size_t kSmemBudget = 227 * 1024 - 6 * 1024;   // dynamic shared memory: 227 KB per CTA minus the kernel's static arrays (4.4 KB)
 
-// Launch geometry for a call whose longest feasible label sequence is max_L: the number of lattice windows
-// per sweep (template parameter NWMAX: 1, 2 or 4), the longest label sequence the block-exponent lattice
-// takes (l_cap: it must fit NWMAX windows AND the shared-memory budget -- in gathered mode the emission-row
-// ring grows with the label sequence, 256 * (L + 5) bytes per side), and the dynamic shared memory.
-// Longer utterances are evaluated by the fp64 safe lattice in the same launch.
-struct LatticeCfg {
-  int nwmax, l_cap, depth;   // depth: chunks in the record ring (lattice_fast.cuh)
-  size_t smem;
-  bool cluster;      // two CTAs per utterance (lattice_cluster_kernel)
-};
-template <int NWMAX>
-size_t fast_bytes_at(const CallParams& p, int L, int D) {
-  const int rw = p.gathered ? em_width_of(L) : (p.V + 3) / 4 * 4;
-  return fast_smem_bytes<kChunk, NWMAX, 8>(L, rw, p.V, D);
-}
-size_t fast_bytes(const CallParams& p, int nwmax, int L, int D) {
-  return nwmax == 1 ? fast_bytes_at<1>(p, L, D) : (nwmax == 2 ? fast_bytes_at<2>(p, L, D) : fast_bytes_at<4>(p, L, D));
-}
-template <int NWMAX>
-size_t fast_bytes_cluster_at(const CallParams& p, int L, int D) {
-  const int rw = p.gathered ? em_width_of(L) : (p.V + 3) / 4 * 4;
-  return fast_smem_bytes_cluster<kChunk, NWMAX, 8>(L, rw, p.V, D);
-}
-size_t fast_bytes_cluster(const CallParams& p, int nwmax, int L, int D) {
-  return nwmax == 1 ? fast_bytes_cluster_at<1>(p, L, D) : (nwmax == 2 ? fast_bytes_cluster_at<2>(p, L, D) : fast_bytes_cluster_at<4>(p, L, D));
-}
 // Two CTAs per utterance pay when every CTA gets an SM of its own: 2 * B <= number of SMs (B200CTC_CLUSTER=0 / 1
 // overrides the choice, for A/B measurements).
 bool want_cluster(int B) {
@@ -210,77 +182,29 @@ bool want_cluster(int B) {
 }
 int round_nw(int nw) { return nw <= 1 ? 1 : (nw <= 2 ? 2 : 4); }
 
-cudaError_t lattice_cfg(const CallParams& p, int max_L, LatticeCfg* out) {
-  const size_t safe = safe_smem_bytes(max_L) > 256 * sizeof(double) ? safe_smem_bytes(max_L) : 256 * sizeof(double);
-  if (safe > kSmemBudget) return cudaErrorInvalidConfiguration;   // not even the safe lattice holds this label sequence
-  // The deepest record ring whose shared memory still holds the longest label sequence; when none does, the
-  // shallowest (largest capacity) and the longer utterances take the safe lattice.
-  int nwmax = 1, l_cap = 0, depth = 2;
-  for (int D = kOthDepthMax; D >= 2; --D) {
-    nwmax = round_nw(fast_warps_needed<kChunk, 8>(max_L));
-    l_cap = max_L;
-    // shared memory is monotonic in L (and in the row width, which follows L in gathered mode)
-    while (l_cap > 0 && (fast_warps_needed<kChunk, 8>(l_cap) > nwmax || fast_bytes(p, nwmax, l_cap, D) > kSmemBudget)) --l_cap;
-    depth = D;
-    if (l_cap >= max_L) break;
-  }
-  nwmax = round_nw(fast_warps_needed<kChunk, 8>(l_cap));
-  const size_t fast = fast_bytes(p, nwmax, l_cap, depth);
-  out->nwmax = nwmax;
-  out->depth = depth;
-  out->l_cap = fast <= kSmemBudget ? l_cap : -1;   // -1: every utterance takes the safe lattice
-  out->smem = (out->l_cap >= 0 && fast > safe) ? fast : safe;
-  out->cluster = out->l_cap >= 0 && want_cluster(p.B);
-  if (out->cluster) {
-    // one side per CTA; at least 116 KB so that the two CTAs of a cluster cannot share an SM
-    const size_t one = fast_bytes_cluster(p, nwmax, out->l_cap, depth);
-    size_t sm = one > safe ? one : safe;
-    out->smem = sm > (size_t)116 * 1024 ? sm : (size_t)116 * 1024;
-  }
-  return cudaSuccess;
-}
-
-template <int K, int NWMAX, int NS>
-cudaError_t launch_lattice_t(const CallParams& p, size_t smem, cudaStream_t stream) {
-  if (smem > 48 * 1024) {
-    cudaError_t e = cudaFuncSetAttribute(lattice_kernel<K, NWMAX, NS>,
-                                         cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+template <int NWMAX>
+cudaError_t launch_lattice_t(const CallParams& p, const LatticeCfg& c, cudaStream_t stream) {
+  void (*kernel)(CallParams) = c.cluster ? lattice_cluster_kernel<NWMAX> : lattice_kernel<NWMAX>;
+  if (c.smem > 48 * 1024) {
+    cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)c.smem);
     if (e != cudaSuccess) return e;
   }
   // programmatic dependent launch: this kernel may start while K1 (the previous kernel in the stream) runs
   cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3((unsigned)p.B);
-  cfg.blockDim = dim3(2 * (NWMAX + kReducers) * 32);
-  cfg.dynamicSmemBytes = smem;
-  cfg.stream = stream;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[0].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = 1;
-  return cudaLaunchKernelEx(&cfg, lattice_kernel<K, NWMAX, NS>, p);
-}
-
-template <int K, int NWMAX, int NS>
-cudaError_t launch_lattice_cluster_t(const CallParams& p, size_t smem, cudaStream_t stream) {
-  cudaError_t e = cudaFuncSetAttribute(lattice_cluster_kernel<K, NWMAX, NS>,
-                                       cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-  if (e != cudaSuccess) return e;
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3((unsigned)(2 * p.B));
-  cfg.blockDim = dim3(cluster_block_warps<NWMAX>() * 32);
-  cfg.dynamicSmemBytes = smem;
+  cfg.gridDim = dim3((unsigned)(c.cluster ? 2 * p.B : p.B));
+  cfg.blockDim = dim3(c.cluster ? cluster_block_warps<NWMAX>() * 32 : 2 * (NWMAX + kReducers) * 32);
+  cfg.dynamicSmemBytes = c.smem;
   cfg.stream = stream;
   cudaLaunchAttribute attr[2];
   attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
   attr[0].val.programmaticStreamSerializationAllowed = 1;
-  attr[1].id = cudaLaunchAttributeClusterDimension;
+  attr[1].id = cudaLaunchAttributeClusterDimension;   // the cluster variant only: the two CTAs of an utterance
   attr[1].val.clusterDim.x = 2;
   attr[1].val.clusterDim.y = 1;
   attr[1].val.clusterDim.z = 1;
   cfg.attrs = attr;
-  cfg.numAttrs = 2;
-  return cudaLaunchKernelEx(&cfg, lattice_cluster_kernel<K, NWMAX, NS>, p);
+  cfg.numAttrs = c.cluster ? 2 : 1;
+  return cudaLaunchKernelEx(&cfg, kernel, p);
 }
 
 // Gathered mode, after the lattice: grads[t,b,symbol] -= s_occ * occupancy for the blank and every distinct symbol
@@ -315,30 +239,49 @@ cudaError_t launch_apply_occupancy(const CallParams& p, cudaStream_t stream) {
   return cudaGetLastError();
 }
 
-namespace {
-}  // namespace
-
-cudaError_t prepare_lattice(CallParams& p, int max_L) {
-  LatticeCfg c;
-  cudaError_t e = lattice_cfg(p, max_L, &c);
-  if (e == cudaSuccess) { p.fast_l_cap = c.l_cap; p.oth_depth = c.depth; }
-  return e;
+// Launch geometry for a call whose longest feasible label sequence is max_L: the number of lattice windows
+// per sweep (template parameter NWMAX: 1, 2 or 4), the longest label sequence the block-exponent lattice
+// takes (l_cap: it must fit NWMAX windows AND the shared-memory budget -- in gathered mode the emission-row
+// ring grows with the label sequence, 256 * (L + 5) bytes per side), and the dynamic shared memory.
+// Longer utterances are evaluated by the fp64 safe lattice in the same launch.
+cudaError_t prepare_lattice(CallParams& p, int max_L, LatticeCfg* out) {
+  const size_t safe = safe_smem_bytes(max_L) > 256 * sizeof(double) ? safe_smem_bytes(max_L) : 256 * sizeof(double);
+  if (safe > kSmemBudget) return cudaErrorInvalidConfiguration;   // not even the safe lattice holds this label sequence
+  // The deepest record ring whose shared memory still holds the longest label sequence; when none does, the
+  // shallowest (largest capacity) and the longer utterances take the safe lattice.
+  int nwmax = 1, l_cap = 0, depth = 2;
+  for (int D = kOthDepthMax; D >= 2; --D) {
+    nwmax = round_nw(fast_warps_needed(max_L));
+    l_cap = max_L;
+    // shared memory is monotonic in L (and in the row width, which follows L in gathered mode)
+    while (l_cap > 0 && (fast_warps_needed(l_cap) > nwmax || fast_smem_bytes(p, nwmax, 2, l_cap, D) > kSmemBudget)) --l_cap;
+    depth = D;
+    if (l_cap >= max_L) break;
+  }
+  nwmax = round_nw(fast_warps_needed(l_cap));
+  const size_t fast = fast_smem_bytes(p, nwmax, 2, l_cap, depth);
+  out->nwmax = nwmax;
+  out->depth = depth;
+  out->l_cap = fast <= kSmemBudget ? l_cap : -1;   // -1: every utterance takes the safe lattice
+  out->smem = (out->l_cap >= 0 && fast > safe) ? fast : safe;
+  out->cluster = out->l_cap >= 0 && want_cluster(p.B);
+  if (out->cluster) {
+    // one side per CTA; at least 116 KB so that the two CTAs of a cluster cannot share an SM
+    const size_t one = fast_smem_bytes(p, nwmax, 1, out->l_cap, depth);
+    size_t sm = one > safe ? one : safe;
+    out->smem = sm > (size_t)116 * 1024 ? sm : (size_t)116 * 1024;
+  }
+  p.fast_l_cap = out->l_cap;
+  p.oth_depth = depth;
+  return cudaSuccess;
 }
 
-cudaError_t launch_lattice(const CallParams& p, int max_L, cudaStream_t stream) {
+cudaError_t launch_lattice(const CallParams& p, const LatticeCfg& c, cudaStream_t stream) {
   if (p.B == 0) return cudaSuccess;
-  LatticeCfg c;
-  cudaError_t e = lattice_cfg(p, max_L, &c);
-  if (e != cudaSuccess) return e;
   // eight lattice states per lane; one, two or four 256-state windows per sweep
-  if (c.cluster) {
-    if (c.nwmax == 1) return launch_lattice_cluster_t<kChunk, 1, 8>(p, c.smem, stream);
-    if (c.nwmax == 2) return launch_lattice_cluster_t<kChunk, 2, 8>(p, c.smem, stream);
-    return launch_lattice_cluster_t<kChunk, 4, 8>(p, c.smem, stream);
-  }
-  if (c.nwmax == 1) return launch_lattice_t<kChunk, 1, 8>(p, c.smem, stream);
-  if (c.nwmax == 2) return launch_lattice_t<kChunk, 2, 8>(p, c.smem, stream);
-  return launch_lattice_t<kChunk, 4, 8>(p, c.smem, stream);   // longer label sequences (L > 463) take the safe lattice
+  if (c.nwmax == 1) return launch_lattice_t<1>(p, c, stream);
+  if (c.nwmax == 2) return launch_lattice_t<2>(p, c, stream);
+  return launch_lattice_t<4>(p, c, stream);   // longer label sequences (L > 463) take the safe lattice
 }
 
 #ifdef B200CTC_TRACE

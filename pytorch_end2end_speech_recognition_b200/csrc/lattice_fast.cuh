@@ -71,21 +71,12 @@ __device__ __forceinline__ void trace_event(int& cnt, int tag) {
 #define B200CTC_TRACE_EVENT(cnt, tag) do { (void)cnt; } while (0)
 #endif
 
-#ifndef B200CTC_ABLATE
-#define B200CTC_ABLATE 0   // developer timing experiments (tools/ablate_lattice.py): a bit mask, bit n = experiment n; 0 = product
-#endif
-#define B200CTC_ABL(n) (((B200CTC_ABLATE) >> (n)) & 1)
-#ifndef B200CTC_PH1_UNROLL
-#define B200CTC_PH1_UNROLL 2   // frames per unrolled iteration of the phase-1 / phase-2 frame loops
-#endif
-#ifndef B200CTC_PH2_UNROLL
-#define B200CTC_PH2_UNROLL 2
-#endif
-constexpr int kPh1Unroll = B200CTC_PH1_UNROLL, kPh2Unroll = B200CTC_PH2_UNROLL;
 constexpr int kAbortExtremeRow = 2;  // abort word: K1 flagged the utterance (nothing was written yet); 1 = redo after a lost range
 constexpr int kEZero = -(1 << 28);  // exponent of an all-zero lane
+constexpr int kChunk = 4;           // frames per chunk (K)
+constexpr int kLaneStates = 8;      // lattice states per lane (NS)
 constexpr int kRowsRing = 4;        // emission-row ring, in halo-exchange intervals (KX/K chunks each): the reducers' one, the current one, the next (landed), the one after (in flight)
-constexpr int kReducers = 4;        // reducer warps per side: warp j takes frame j of every phase-2 chunk (== K)
+constexpr int kReducers = kChunk;   // reducer warps per side: warp j takes frame j of every phase-2 chunk
 // Helper warps per side.  One CTA for both sides: kReducers warps that fetch (emission rows, records) AND reduce.
 // Cluster variant (one side per CTA, an SM to itself): the two jobs on different warps -- kReducers fetchers and
 // kReducers reducers -- because with one or two lattice windows the helper's fetch-then-reduce chain (~1500 cycles
@@ -114,10 +105,7 @@ __device__ __forceinline__ int cluster_warp_role(int warp) {
 // some chunks (B200: C3 -2 %, C5 -6 % with four, see experiments/README.md).  Chosen per launch
 // (CallParams::oth_depth, lattice.cu): the deepest of 4, 3, 2 whose shared memory still holds the longest label
 // sequence of the call -- in gathered mode the capacity is 195 / 210 / 226 labels.
-#ifndef B200CTC_OTH_DEPTH
-#define B200CTC_OTH_DEPTH 4
-#endif
-constexpr int kOthDepthMax = B200CTC_OTH_DEPTH;
+constexpr int kOthDepthMax = 4;
 
 // ---------------------------------------------------------------------------------------------
 // PTX helpers
@@ -242,30 +230,27 @@ __device__ __forceinline__ float f2_max(f2 a, f2 b) {  // max over the four floa
 }
 
 // ---------------------------------------------------------------------------------------------
-// geometry shared by host (shared-memory sizing) and device.  NS = lattice states per lane (4 or 8).
+// geometry shared by host (shared-memory sizing) and device.  NS = kLaneStates lattice states per lane.
 // ---------------------------------------------------------------------------------------------
-// Frames between two halo exchanges of neighbouring lattice windows.  Consecutive windows overlap by
+// Frames between two halo exchanges of neighbouring lattice windows (KX).  Consecutive windows overlap by
 // 2*KX positions: dependencies only point downwards (s-1, s-2), so the garbage creeping up from a window's
 // bottom stays inside the overlap for KX frames.  K (frames per chunk) sets the granularity of the
 // shared-memory buffers and of the hand-off with the helper warps; phase 1 needs neither between two
 // exchanges and runs KX/K chunks back to back without a barrier -- every barrier costs the recursion's
 // dependent chain a pipeline drain and refill (~500 cycles against 140 per frame in steady state).
-template <int K, int NS>
-__host__ __device__ constexpr int exchange_frames() { return NS == 8 ? 4 * K : K; }
+constexpr int kExchangeFrames = 4 * kChunk;
 
-template <int K, int NS>
 __host__ __device__ inline int fast_warps_needed(int L) {
-  const int P = NS * ((2 * L + 1 + NS - 1) / NS);
-  const int win = 32 * NS, own = win - 2 * exchange_frames<K, NS>();
+  const int P = kLaneStates * ((2 * L + 1 + kLaneStates - 1) / kLaneStates);
+  const int win = 32 * kLaneStates, own = win - 2 * kExchangeFrames;
   return P <= win ? 1 : 1 + (P - win + own - 1) / own;
 }
 // One frame of stored records ("frame block"), the same layout in the HBM scratch and in shared memory:
 // NS/4 planes of JG float4 (the packed mantissa pairs of every position group) followed by JG int32
 // exponents, padded to 16 bytes -- one TMA bulk copy moves a whole frame.
-template <int NS>
 __host__ __device__ inline int frame_block_bytes(int L) {
-  const int JG = (2 * L + 1 + NS - 1) / NS;
-  return (NS / 4) * JG * 16 + ((JG + 3) & ~3) * 4;
+  const int JG = (2 * L + 1 + kLaneStates - 1) / kLaneStates;
+  return (kLaneStates / 4) * JG * 16 + ((JG + 3) & ~3) * 4;
 }
 // Symbol-sorted posterior row: the label posteriors of a frame grouped by symbol (label i sits at its rank
 // in (symbol, position) order), every symbol's group padded to a multiple of four slots so that the
@@ -291,49 +276,44 @@ __host__ __device__ inline int post_stride(int L, int V) {  // floats per frame 
   return post_label_slots(L, V) + NWMAX * 32 + 4;
 }
 
-template <int K, int NWMAX, int NS>
+template <int NWMAX>
 __host__ __device__ inline size_t fast_side_bytes(int L, int RW, int V, int D) {
-  constexpr int HL = 2 * exchange_frames<K, NS>() / NS;
-  constexpr int RCH = kRowsRing * exchange_frames<K, NS>() / K;   // chunk slots of the emission-row ring
+  constexpr int HL = 2 * kExchangeFrames / kLaneStates;
+  constexpr int RCH = kRowsRing * kExchangeFrames / kChunk;   // chunk slots of the emission-row ring
   size_t b = 0;
-  b += (size_t)(D * K + 1) * frame_block_bytes<NS>(L);       // oth (+ the zero block)
-  b += (size_t)2 * NWMAX * HL * (NS / 4) * 16;               // halo_m
-  b += (size_t)RCH * K * (size_t)(RW + 4) * 4;               // rows
-  b += 2 * (size_t)K * post_stride<NWMAX>(L, V) * 4;         // post
+  b += (size_t)(D * kChunk + 1) * frame_block_bytes(L);      // oth (+ the zero block)
+  b += (size_t)2 * NWMAX * HL * (kLaneStates / 4) * 16;      // halo_m
+  b += (size_t)RCH * kChunk * (size_t)(RW + 4) * 4;          // rows
+  b += 2 * (size_t)kChunk * post_stride<NWMAX>(L, V) * 4;    // post
   b += (size_t)2 * NWMAX * HL * 4;                           // halo_e
   b += NWMAX * 8;                                            // red
   b += (size_t)kReducers * kOthDepthMax * 8 + 8;             // mbar
   return (b + 15) / 16 * 16;
 }
-#ifndef B200CTC_GROUP_SPLIT
-#define B200CTC_GROUP_SPLIT 1   // 0: one reducer group per symbol, whatever its size (A/B measurements)
-#endif
 constexpr int kReducerGroups = 64;    // reducer groups of the straight-line reducer path: two per lane
 constexpr int kUntouchedMaxV = 256;   // the small-vocabulary (non-gathered) lattice never sees a larger vocabulary
-template <int K, int NWMAX, int NS>
-__host__ __device__ inline size_t fast_smem_bytes(int L, int RW, int V, int D) {
-  // control words, lab, sorted, seg_start, seg_sym, slot_of_label, seg_slot, untouched
-  size_t common = (size_t)(16 + 6 * L + 16 + 4 * kReducerGroups + (V <= kUntouchedMaxV ? V : 0)) * 4;
+// Dynamic shared memory of the fast lattice for label sequences up to L with nwmax lattice windows and a record
+// ring D chunks deep: the utterance-wide tables (control words, lab, sorted, seg_start, seg_sym, slot_of_label,
+// seg_slot, untouched; laid out by lattice_fast_utterance) and `sides` side blocks -- 2 when one CTA runs both
+// sweeps, 1 in the cluster variant.
+inline size_t fast_smem_bytes(const CallParams& p, int nwmax, int sides, int L, int D) {
+  const int RW = p.gathered ? em_width_of(L) : (p.V + 3) / 4 * 4;
+  size_t common = (size_t)(16 + 6 * L + 16 + 4 * kReducerGroups + (p.V <= kUntouchedMaxV ? p.V : 0)) * 4;
   common = (common + 15) / 16 * 16;
-  return common + 2 * fast_side_bytes<K, NWMAX, NS>(L, RW, V, D) + 16;
+  const size_t side = nwmax == 1 ? fast_side_bytes<1>(L, RW, p.V, D)
+                    : nwmax == 2 ? fast_side_bytes<2>(L, RW, p.V, D) : fast_side_bytes<4>(L, RW, p.V, D);
+  return common + sides * side + 16;
 }
-
-template <int K, int NWMAX, int NS>
-__host__ __device__ inline size_t fast_smem_bytes_cluster(int L, int RW, int V, int D) {   // one side per CTA
-  size_t common = (size_t)(16 + 6 * L + 16 + 4 * kReducerGroups + (V <= kUntouchedMaxV ? V : 0)) * 4;
-  common = (common + 15) / 16 * 16;
-  return common + fast_side_bytes<K, NWMAX, NS>(L, RW, V, D) + 16;
-}
-template <int K, int NWMAX, int NS>
+template <int NWMAX>
 __device__ __forceinline__ FastSideSmem carve_fast_side(unsigned char* base, int L, int RW, int V, int D) {
-  constexpr int HL = 2 * exchange_frames<K, NS>() / NS;
-  constexpr int RCH = kRowsRing * exchange_frames<K, NS>() / K;
+  constexpr int HL = 2 * kExchangeFrames / kLaneStates;
+  constexpr int RCH = kRowsRing * kExchangeFrames / kChunk;
   FastSideSmem s;
   unsigned char* p = base;
-  s.oth = p;                               p += (size_t)(D * K + 1) * frame_block_bytes<NS>(L);
-  s.halo_m = reinterpret_cast<float4*>(p); p += (size_t)2 * NWMAX * HL * (NS / 4) * 16;
-  s.rows = reinterpret_cast<float*>(p);    p += (size_t)RCH * K * (size_t)(RW + 4) * 4;
-  s.post = reinterpret_cast<float*>(p);    p += 2 * (size_t)K * post_stride<NWMAX>(L, V) * 4;
+  s.oth = p;                               p += (size_t)(D * kChunk + 1) * frame_block_bytes(L);
+  s.halo_m = reinterpret_cast<float4*>(p); p += (size_t)2 * NWMAX * HL * (kLaneStates / 4) * 16;
+  s.rows = reinterpret_cast<float*>(p);    p += (size_t)RCH * kChunk * (size_t)(RW + 4) * 4;
+  s.post = reinterpret_cast<float*>(p);    p += 2 * (size_t)kChunk * post_stride<NWMAX>(L, V) * 4;
   s.halo_e = reinterpret_cast<int*>(p);    p += (size_t)2 * NWMAX * HL * 4;
   s.red_m = reinterpret_cast<float*>(p);   p += NWMAX * 4;
   s.red_e = reinterpret_cast<int*>(p);     p += NWMAX * 4;
@@ -381,21 +361,19 @@ __device__ __forceinline__ void midpoint_sync(int count) {
 // Label positions are the odd elements (forward) / even elements (backward); label slot m is element
 // 2m+1 / 2m; label pair u (pair index 2u+1 / 2u) holds label slots (u, u + NP/2).
 // ---------------------------------------------------------------------------------------------
-template <int NS>
 struct LaneConst {
-  int idxB[NS / 2]; // byte offset in the emission row of the label positions (zero slot if the position is a dummy)
-  int idxB_blank;   // byte offset of the blank
-  f2 Kf[NS / 4];    // skip-transition factors (1.0 allowed / 0.0 not) of the label pairs
-  int posB[NS / 2]; // byte offset of the label positions in the symbol-sorted posterior row (dump slot if dummy)
-  int blankB;       // byte offset of this thread's blank partial sum in the posterior row
-  int recB, expB;   // byte offsets of this lane's group in a frame block: first mantissa plane, exponent
-  bool owned;       // this lane's group belongs to the warp (not to the halo) and exists
-  int group;        // global position group (pos0 / NS)
+  int idxB[kLaneStates / 2];   // byte offset in the emission row of the label positions (zero slot if the position is a dummy)
+  int idxB_blank;              // byte offset of the blank
+  f2 Kf[kLaneStates / 4];      // skip-transition factors (1.0 allowed / 0.0 not) of the label pairs
+  int posB[kLaneStates / 2];   // byte offset of the label positions in the symbol-sorted posterior row (dump slot if dummy)
+  int blankB;                  // byte offset of this thread's blank partial sum in the posterior row
+  int recB, expB;              // byte offsets of this lane's group in a frame block: first mantissa plane, exponent
+  bool owned;                  // this lane's group belongs to the warp (not to the halo) and exists
+  int group;                   // global position group (pos0 / NS)
 };
 
-template <int NS>
 struct LaneState {
-  f2 A[NS / 2];
+  f2 A[kLaneStates / 2];
   int e;
 };
 
@@ -405,44 +383,28 @@ __device__ __forceinline__ float lds_f32(const void* base, int byte_off) {
 __device__ __forceinline__ void sts_f32(void* base, int byte_off, float v) {
   *reinterpret_cast<float*>(reinterpret_cast<char*>(base) + byte_off) = v;
 }
-template <int N>
-__device__ __forceinline__ float f2_max_all(const f2 (&v)[N]) {   // max over the 2N floats, two levels deep for N = 4
-  if (N == 4) {
-    const float t1 = fmax3(f2_lo(v[0]), f2_hi(v[0]), f2_lo(v[1]));
-    const float t2 = fmax3(f2_hi(v[1]), f2_lo(v[2]), f2_hi(v[2]));
-    const float t3 = fmaxf(f2_lo(v[N - 1]), f2_hi(v[N - 1]));
-    return fmax3(t1, t2, t3);
-  }
-  return fmaxf(fmax3(f2_lo(v[0]), f2_hi(v[0]), f2_lo(v[1])), f2_hi(v[1]));
+__device__ __forceinline__ float f2_max_all(const f2 (&v)[4]) {   // max over the 8 floats, two levels deep
+  const float t1 = fmax3(f2_lo(v[0]), f2_hi(v[0]), f2_lo(v[1]));
+  const float t2 = fmax3(f2_hi(v[1]), f2_lo(v[2]), f2_hi(v[2]));
+  const float t3 = fmaxf(f2_lo(v[3]), f2_hi(v[3]));
+  return fmax3(t1, t2, t3);
 }
 
 // One frame of the recursion for one lane.  ACC: pre-emission sums at exponent E; st: the new
 // emission-weighted state, renormalised.
-template <int SIDE, int NS>
-__device__ __forceinline__ void lattice_frame(LaneState<NS>& st, const LaneConst<NS>& lc, const void* __restrict__ row,
-                                              bool lane0, f2 (&ACC)[NS / 2], int& E) {
-  constexpr int NP = NS / 2;
+template <int SIDE>
+__device__ __forceinline__ void lattice_frame(LaneState& st, const LaneConst& lc, const void* __restrict__ row,
+                                              bool lane0, f2 (&ACC)[kLaneStates / 2], int& E) {
+  constexpr int NP = kLaneStates / 2;
   const float a_top = el_j4<SIDE>(st.A[NP - 1]), a_top2 = el_j4<SIDE>(st.A[NP - 2]);
-#if B200CTC_ABL(4)
-  const float n1 = a_top, n2 = a_top2;
-  int ne = st.e;
-#else
   const float n1 = __shfl_up_sync(0xffffffffu, a_top, 1);
   const float n2 = __shfl_up_sync(0xffffffffu, a_top2, 1);
   int ne = __shfl_up_sync(0xffffffffu, st.e, 1);
-#endif
   // emissions: one broadcast load for the blank positions, one gather per label position
-#if B200CTC_ABL(2)
-  const float yb = 0.5f;
-  float y[NP];
-#pragma unroll
-  for (int m = 0; m < NP; ++m) y[m] = 0.25f + 0.01f * m;
-#else
   const float yb = lds_f32(row, lc.idxB_blank);
   float y[NP];
 #pragma unroll
   for (int m = 0; m < NP; ++m) y[m] = lds_f32(row, lc.idxB[m]);
-#endif
   if (lane0) ne = kEZero;                      // nothing below the window: scales n1, n2 to zero
   E = max(st.e, ne);
   const float so = pow2_neg(st.e - E), sn = pow2_neg(ne - E);
@@ -470,11 +432,7 @@ __device__ __forceinline__ void lattice_frame(LaneState<NS>& st, const LaneConst
       W[j] = f2_mul(ACC[j], YB);
     }
   }
-#if B200CTC_ABL(3)
-  const float mx = 1.0f;
-#else
-  const float mx = f2_max_all<NP>(W);
-#endif
+  const float mx = f2_max_all(W);
   // renormalise: largest mantissa -> [1,2).  mx == 0 (or NaN from garbage): the lane is empty.
   const int eb = __float_as_int(mx) >> 23;                       // biased exponent
   const bool nz = mx > 0.f;
@@ -508,10 +466,9 @@ __device__ __forceinline__ void band_frames(int ws_lo, int ws_hi, int S, int T, 
 }
 
 // Everything a lattice warp carries through the sweep.
-template <int NS>
 struct SweepState {
-  LaneState<NS> st;
-  LaneConst<NS> lc;
+  LaneState st;
+  LaneConst lc;
   int act_lo, act_hi;       // steps in which the warp window intersects the reachable band (chunks outside are skipped)
   int rd_hi, wr_len;        // the other side stored this lane's record of step n iff (unsigned)(rd_hi - n) < wr_len
   float inv_mP; int eP;     // total probability P = mP * 2^eP (phase 2)
@@ -559,12 +516,12 @@ __device__ __forceinline__ void stage_row(const FastCtx<SIDE>& c, int slot, int 
 // value is 0, or the record was never written and reads as zero -- prefetch_other).
 // The fresh state is normalised to [1,2) per lane, so the one scale factor cannot push a product
 // that matters out of the fp32 range.
-template <int SIDE, int NS>
-__device__ __forceinline__ void posterior_frame(SweepState<NS>& ss, const unsigned char* __restrict__ blk, int plane_bytes,
+template <int SIDE>
+__device__ __forceinline__ void posterior_frame(SweepState& ss, const unsigned char* __restrict__ blk, int plane_bytes,
                                                 void* __restrict__ post) {
-  constexpr int NP = NS / 2, NH = NS / 4;
-  const LaneConst<NS>& lc = ss.lc;
-  const LaneState<NS>& st = ss.st;
+  constexpr int NP = kLaneStates / 2, NH = kLaneStates / 4;
+  const LaneConst& lc = ss.lc;
+  const LaneState& st = ss.st;
   f2 O[NP];
 #pragma unroll
   for (int h = 0; h < NH; ++h) {
@@ -590,7 +547,7 @@ __device__ __forceinline__ void posterior_frame(SweepState<NS>& ss, const unsign
   // dexp stays below kLostBound - 129 the bound holds whatever they are, and only the (rare) lanes beyond
   // that look at their maximum.
   if (dexp > kLostBound - 130) {
-    const float omax = f2_max_all<NP>(O);
+    const float omax = f2_max_all(O);
     ss.maxbound = max(ss.maxbound, (__float_as_int(omax) >> 23) + dexp);
   }
   {
@@ -614,13 +571,13 @@ __device__ __forceinline__ void posterior_frame(SweepState<NS>& ss, const unsign
 
 // One chunk (kc <= K frames starting at step n0; emission rows in ring slot `rslot`).  A warp whose
 // window misses the reachable band in all frames of the chunk skips it (warp-uniform).
-template <int K, bool PH2, int SIDE, int NT, int NS>
-__device__ __forceinline__ void run_chunk(const FastCtx<SIDE>& c, SweepState<NS>& ss, int rslot, int pbuf, int obuf,
+template <bool PH2, int SIDE>
+__device__ __forceinline__ void run_chunk(const FastCtx<SIDE>& c, SweepState& ss, int rslot, int pbuf, int obuf,
                                           int n0, int kc, bool write_post) {
-  constexpr int NP = NS / 2, NH = NS / 4;
-  const LaneConst<NS>& lc = ss.lc;
+  constexpr int NP = kLaneStates / 2, NH = kLaneStates / 4;
+  const LaneConst& lc = ss.lc;
   const bool lane0 = c.lane == 0;
-  const char* row = reinterpret_cast<const char*>(c.sm.rows + (size_t)rslot * K * c.RWS);
+  const char* row = reinterpret_cast<const char*>(c.sm.rows + (size_t)rslot * kChunk * c.RWS);
   const int row_bytes = c.RWS * 4;
   const bool active = n0 <= ss.act_hi && n0 + kc - 1 >= ss.act_lo;
   if (!PH2) {
@@ -632,47 +589,36 @@ __device__ __forceinline__ void run_chunk(const FastCtx<SIDE>& c, SweepState<NS>
     const int plane = c.JG * 16;
     const int eoff = ss.weoff;                                    // exponent slot relative to the first mantissa plane slot
     unsigned char* blk = ss.wblk;
-#if B200CTC_ABL(8)
-    LaneState<NS> dummy = ss.st;
-#endif
-#pragma unroll kPh1Unroll
+#pragma unroll 2
     for (int j = 0; j < kc; ++j) {
       f2 ACC[NP]; int E;
-#if B200CTC_ABL(8)
-      { f2 ACC2[NP]; int E2; lattice_frame<SIDE, NS>(dummy, lc, row, lane0, ACC2, E2); }
-#endif
-      lattice_frame<SIDE, NS>(ss.st, lc, row, lane0, ACC, E);
-      if (!B200CTC_ABL(1)) {
-        // the reader's pair j is this lane's pair NP-1-j (mirrored group, mirrored packing); lanes that
-        // own no group (halo, beyond the lattice) store into the dump block: no branch in the loop
+      lattice_frame<SIDE>(ss.st, lc, row, lane0, ACC, E);
+      // the reader's pair j is this lane's pair NP-1-j (mirrored group, mirrored packing); lanes that
+      // own no group (halo, beyond the lattice) store into the dump block: no branch in the loop
 #pragma unroll
-        for (int h = 0; h < NH; ++h)
-          asm volatile("st.global.v2.b64 [%0], {%1, %2};" ::"l"(blk + h * plane),
-                       "l"(ACC[NP - 1 - 2 * h]), "l"(ACC[NP - 2 - 2 * h]) : "memory");
-        *reinterpret_cast<int*>(blk + eoff) = E;
-      }
+      for (int h = 0; h < NH; ++h)
+        asm volatile("st.global.v2.b64 [%0], {%1, %2};" ::"l"(blk + h * plane),
+                     "l"(ACC[NP - 1 - 2 * h]), "l"(ACC[NP - 2 - 2 * h]) : "memory");
+      *reinterpret_cast<int*>(blk + eoff) = E;
       row += row_bytes;
       blk += ss.wstep;
     }
     ss.wblk = blk;
-#if B200CTC_ABL(8)
-    if (dummy.e == 12345) ss.maxbound = 1 << 20;   // keep the duplicate chain alive
-#endif
   } else {
     // cost-only calls (no gradient buffer) walk phase 2 for the range check: their posteriors land in one dump row
-    char* post = reinterpret_cast<char*>(c.sm.post + (size_t)pbuf * K * c.PS);
+    char* post = reinterpret_cast<char*>(c.sm.post + (size_t)pbuf * kChunk * c.PS);
     const int post_bytes = write_post ? c.PS * 4 : 0;
     const bool store = write_post;
     if (active) {
-      const unsigned char* blk = c.sm.oth + (size_t)obuf * K * c.FB;
-      const unsigned char* zero_blk = c.sm.oth + (size_t)c.D * K * c.FB;
+      const unsigned char* blk = c.sm.oth + (size_t)obuf * kChunk * c.FB;
+      const unsigned char* zero_blk = c.sm.oth + (size_t)c.D * kChunk * c.FB;
       const int plane = c.JG * 16;
-#pragma unroll kPh2Unroll
+#pragma unroll 2
       for (int j = 0; j < kc; ++j) {
         f2 ACC[NP]; int E;
-        lattice_frame<SIDE, NS>(ss.st, lc, row, lane0, ACC, E);
+        lattice_frame<SIDE>(ss.st, lc, row, lane0, ACC, E);
         const bool wr = (unsigned)(ss.rd_hi - (n0 + j)) < (unsigned)ss.wr_len;   // did the other side store this record?
-        if (!B200CTC_ABL(5)) posterior_frame<SIDE, NS>(ss, wr ? blk : zero_blk, plane, post);
+        posterior_frame<SIDE>(ss, wr ? blk : zero_blk, plane, post);
         row += row_bytes;
         post += post_bytes;
         blk += c.FB;
@@ -692,13 +638,13 @@ __device__ __forceinline__ void run_chunk(const FastCtx<SIDE>& c, SweepState<NS>
 // Chunk boundary of the lattice warps: publish the halo lanes, ONE barrier with the side's lattice and
 // helper warps (after it the helpers' prefetch for the next chunk has landed and the posterior buffer
 // of the previous chunk is consumed), import the halo.
-template <int K, int NWMAX, int SIDE, int NS, int HW>   // HW: helper warps of the side
-__device__ __forceinline__ void chunk_boundary(const FastCtx<SIDE>& c, SweepState<NS>& ss, int cc, int* abort_flag, int& tc,
-                                               bool exchange = true, bool sync = true) {
-  constexpr int NH = NS / 4, HL = 2 * exchange_frames<K, NS>() / NS;
-  static_assert(HL * NS == 2 * exchange_frames<K, NS>() && HL >= 1, "the halo must be whole lanes");
+template <int NWMAX, int SIDE, int HW>   // HW: helper warps of the side
+__device__ __forceinline__ void chunk_boundary(const FastCtx<SIDE>& c, SweepState& ss, int cc, int* abort_flag, int& tc,
+                                               bool exchange = true) {
+  constexpr int NH = kLaneStates / 4, HL = 2 * kExchangeFrames / kLaneStates;
+  static_assert(HL * kLaneStates == 2 * kExchangeFrames && HL >= 1, "the halo must be whole lanes");
   const int hb = cc & 1, NW = c.NW, w = c.w, lane = c.lane;
-  LaneState<NS>& st = ss.st;
+  LaneState& st = ss.st;
   if (exchange && w + 1 < NW && lane >= 32 - HL) {
     const int slot = (hb * NWMAX + w) * HL + (lane - (32 - HL));
 #pragma unroll
@@ -708,7 +654,7 @@ __device__ __forceinline__ void chunk_boundary(const FastCtx<SIDE>& c, SweepStat
   }
   if (ss.lc.owned && ss.maxbound > kLostBound) *abort_flag = 1;
   B200CTC_TRACE_EVENT(tc, 30);
-  if (sync) named_bar_sync(bar_chunk(SIDE), (NW + HW) * 32);
+  named_bar_sync(bar_chunk(SIDE), (NW + HW) * 32);
   B200CTC_TRACE_EVENT(tc, 31);
   if (exchange && w > 0 && lane < HL) {
     const int slot = (hb * NWMAX + (w - 1)) * HL + lane;
@@ -739,19 +685,19 @@ __device__ __forceinline__ bool total_probability(const FastSideSmem& sm, int NW
   return true;
 }
 
-template <int K, int NWMAX, int SIDE, int NS>
+template <int NWMAX, int SIDE>
 __device__ __forceinline__ void fill_ctx(FastCtx<SIDE>& c, const CallParams& p, int b, const UttMeta& m,
                                          unsigned char* side_smem, int w, int lane) {
   c.p = &p; c.b = b;
-  c.T = m.T; c.L = m.L; c.S = 2 * m.L + 1; c.JG = (c.S + NS - 1) / NS; c.FB = frame_block_bytes<NS>(m.L); c.P = NS * c.JG;
-  c.NW = fast_warps_needed<K, NS>(m.L);
+  c.T = m.T; c.L = m.L; c.S = 2 * m.L + 1; c.JG = (c.S + kLaneStates - 1) / kLaneStates; c.FB = frame_block_bytes(m.L); c.P = kLaneStates * c.JG;
+  c.NW = fast_warps_needed(m.L);
   c.RW = p.gathered ? m.W : (p.V + 3) / 4 * 4;
   c.RWS = c.RW + 4;
   c.PS = post_stride<NWMAX>(m.L, p.V);
   c.RC = c.PS - NWMAX * 32 - 4;                 // label slots come first, then the blank partials, then the dump slot
   c.w = w; c.lane = lane; c.tid_side = w * 32 + lane;
   c.D = p.oth_depth;
-  c.sm = carve_fast_side<K, NWMAX, NS>(side_smem, m.L, c.RW, p.V, c.D);
+  c.sm = carve_fast_side<NWMAX>(side_smem, m.L, c.RW, p.V, c.D);
   c.scr = p.scratch + m.scratch_off * kGroupBytes;
   const float* row_src; long long row_stride; int row_vec;
   if (p.gathered) {
@@ -771,12 +717,11 @@ __device__ __forceinline__ void fill_ctx(FastCtx<SIDE>& c, const CallParams& p, 
 struct SidePlan {
   int M_side, nc1, nc2, n_chunks;
 };
-template <int K, int SIDE>
-__device__ __forceinline__ SidePlan side_plan(int T) {
+__device__ __forceinline__ SidePlan side_plan(int T, int side) {
   SidePlan s;
-  s.M_side = SIDE ? (T / 2) : (T - T / 2);      // frames this side covers in phase 1
-  s.nc1 = (s.M_side + K - 1) / K;
-  s.nc2 = (T - s.M_side + K - 1) / K;
+  s.M_side = side ? (T / 2) : (T - T / 2);      // frames this side covers in phase 1
+  s.nc1 = (s.M_side + kChunk - 1) / kChunk;
+  s.nc2 = (T - s.M_side + kChunk - 1) / kChunk;
   s.n_chunks = s.nc1 + s.nc2;
   return s;
 }
@@ -786,30 +731,28 @@ __device__ __forceinline__ SidePlan side_plan(int T) {
 // ---------------------------------------------------------------------------------------------
 // CL: the two sides are the two CTAs of a thread-block cluster; the one rendezvous of the sides (midpoint) then is
 // a cluster barrier instead of a named barrier.
-template <int K, int NWMAX, int SIDE, int NS, bool CL>
+template <int NWMAX, int SIDE, bool CL>
 __device__ void fast_side_sweep(const CallParams& p, int b, const UttMeta& m, const FastCommon& cm,
                                 unsigned char* side_smem, int w, int lane) {
-  constexpr int NP = NS / 2, NH = NS / 4;
-  constexpr int KX = exchange_frames<K, NS>();
-  constexpr int H = 2 * KX;         // halo positions
-  constexpr int RCH = kRowsRing * KX / K;   // chunk slots of the emission-row ring
-  constexpr int HL = H / NS;        // halo lanes
-  constexpr int WIN = 32 * NS;      // positions per warp window
+  constexpr int NP = kLaneStates / 2, NH = kLaneStates / 4;
+  constexpr int H = 2 * kExchangeFrames;                     // halo positions
+  constexpr int RCH = kRowsRing * kExchangeFrames / kChunk;   // chunk slots of the emission-row ring
+  constexpr int HL = H / kLaneStates;                         // halo lanes
+  constexpr int WIN = 32 * kLaneStates;                       // positions per warp window
   constexpr int OWN = WIN - H;
-  constexpr int OWNG = OWN / NS;    // owned groups per warp
-  constexpr int NT = NWMAX * 32;
+  constexpr int OWNG = OWN / kLaneStates;                     // owned groups per warp
 
   FastCtx<SIDE> c;
-  fill_ctx<K, NWMAX, SIDE, NS>(c, p, b, m, side_smem, w, lane);
+  fill_ctx<NWMAX, SIDE>(c, p, b, m, side_smem, w, lane);
   const int T = c.T, S = c.S, JG = c.JG, P = c.P, NW = c.NW;
   const int* lab = cm.lab;
 
   // ---- per-lane constants ----
-  SweepState<NS> ss;
-  LaneConst<NS>& lc = ss.lc;
+  SweepState ss;
+  LaneConst& lc = ss.lc;
   const int base_w = w * OWN;
-  const int pos0 = base_w + NS * lane;
-  lc.group = pos0 / NS;
+  const int pos0 = base_w + kLaneStates * lane;
+  lc.group = pos0 / kLaneStates;
   lc.owned = ((w == 0) || (lane >= HL)) && (lc.group < JG);
   lc.idxB_blank = 4 * (p.gathered ? 0 : p.blank);
   lc.blankB = 4 * (lc.owned ? c.RC + c.tid_side : c.PS - 4);
@@ -861,22 +804,22 @@ __device__ void fast_side_sweep(const CallParams& p, int b, const UttMeta& m, co
     int nb = min(SIDE ? t1 : T - 1 - t0, M_other - 1);
     ss.rd_hi = 0; ss.wr_len = 0;
     if (t0 <= t1 && na <= nb && lc.group < JG) {
-      na = na / K * K;
-      nb = nb / K * K + K - 1;
+      na = na / kChunk * kChunk;
+      nb = nb / kChunk * kChunk + kChunk - 1;
       ss.rd_hi = T - 1 - na;                                  // writer step n' = T-1-n for a reader at step n
       ss.wr_len = nb - na + 1;
     }
   }
   // ---- initial state: delta on the first lattice state of this side's sweep ----
   {
-    float v[NS];
+    float v[kLaneStates];
 #pragma unroll
-    for (int i = 0; i < NS; ++i) v[i] = 0.f;
+    for (int i = 0; i < kLaneStates; ++i) v[i] = 0.f;
     ss.st.e = kEZero;
     const int q_start = SIDE ? (P - S) : 0;   // backward: NS*JG - S dummy positions come first
-    if (w == 0 && q_start >= pos0 && q_start < pos0 + NS) {
+    if (w == 0 && q_start >= pos0 && q_start < pos0 + kLaneStates) {
 #pragma unroll
-      for (int i = 0; i < NS; ++i) if (q_start - pos0 == i) v[i] = 1.f;
+      for (int i = 0; i < kLaneStates; ++i) if (q_start - pos0 == i) v[i] = 1.f;
       ss.st.e = 0;
     }
 #pragma unroll
@@ -892,14 +835,14 @@ __device__ void fast_side_sweep(const CallParams& p, int b, const UttMeta& m, co
   B200CTC_TRACE_DECL(tc);
   B200CTC_TRACE_EVENT(tc, 10);
 
-  const SidePlan pl = side_plan<K, SIDE>(T);
+  const SidePlan pl = side_plan(T, SIDE);
   const int M_side = pl.M_side, nc2 = pl.nc2;
   int* abort_flag = cm.abort_flag;
 
   // the all-zero frame block (stands in for records the other side never wrote)
-  for (int i = c.tid_side; i < c.FB / 4; i += NW * 32) reinterpret_cast<int*>(c.sm.oth + (size_t)c.D * K * c.FB)[i] = (i >= NH * JG * 4) ? kEZero : 0;
+  for (int i = c.tid_side; i < c.FB / 4; i += NW * 32) reinterpret_cast<int*>(c.sm.oth + (size_t)c.D * kChunk * c.FB)[i] = (i >= NH * JG * 4) ? kEZero : 0;
   // zero slots of the row buffers (the helper warps stage the rows themselves)
-  for (int i = c.tid_side; i < RCH * K; i += NW * 32) {
+  for (int i = c.tid_side; i < RCH * kChunk; i += NW * 32) {
     float* z = c.sm.rows + (size_t)i * c.RWS + c.RW;
     z[0] = 0.f; z[1] = 0.f; z[2] = 0.f; z[3] = 0.f;
   }
@@ -918,14 +861,14 @@ __device__ void fast_side_sweep(const CallParams& p, int b, const UttMeta& m, co
   // runs frames outside its band only writes records the reader never looks at, record_window).
   int cc = 0, xc = 0;
   for (int n0 = 0; n0 < M_side; ++xc) {
-    const int kc = min(KX, M_side - n0), nch = (kc + K - 1) / K;
+    const int kc = min(kExchangeFrames, M_side - n0), nch = (kc + kChunk - 1) / kChunk;
     B200CTC_TRACE_EVENT(tc, 2);
-    run_chunk<K, false, SIDE, NT, NS>(c, ss, rs, 0, 0, n0, kc, false);
+    run_chunk<false, SIDE>(c, ss, rs, 0, 0, n0, kc, false);
     B200CTC_TRACE_EVENT(tc, 3);
     rs = (rs + nch) & (RCH - 1);
     n0 += kc;
     cc += nch;
-    chunk_boundary<K, NWMAX, SIDE, NS, HW>(c, ss, xc, abort_flag, tc);
+    chunk_boundary<NWMAX, SIDE, HW>(c, ss, xc, abort_flag, tc);
   }
 
   // ================================ midpoint ================================
@@ -939,15 +882,15 @@ __device__ void fast_side_sweep(const CallParams& p, int b, const UttMeta& m, co
   // ---- total probability P = sum_s alpha_t(s) beta'_t(s) at the first phase-2 frame (state copy) ----
   {
     const int n0 = M_side;
-    LaneState<NS> tmp = ss.st;
+    LaneState tmp = ss.st;
     float part = 0.f; int pe = kEZero;
-    if (n0 <= ss.act_hi && n0 + min(K, T - M_side) - 1 >= ss.act_lo) {   // same rule as run_chunk: the warp runs this chunk
+    if (n0 <= ss.act_hi && n0 + min(kChunk, T - M_side) - 1 >= ss.act_lo) {   // same rule as run_chunk: the warp runs this chunk
       f2 ACC[NP]; int E;
-      lattice_frame<SIDE, NS>(tmp, lc, c.sm.rows + (size_t)rs * K * c.RWS, lane == 0, ACC, E);
+      lattice_frame<SIDE>(tmp, lc, c.sm.rows + (size_t)rs * kChunk * c.RWS, lane == 0, ACC, E);
       if (lc.owned) {
         // no band masks: outside the band one of the two factors is exactly zero (posterior_frame)
         const bool wr = (unsigned)(ss.rd_hi - n0) < (unsigned)ss.wr_len;
-        const unsigned char* blk = c.sm.oth + (wr ? (size_t)0 : (size_t)c.D * K * c.FB);
+        const unsigned char* blk = c.sm.oth + (wr ? (size_t)0 : (size_t)c.D * kChunk * c.FB);
         float sum = 0.f;
 #pragma unroll
         for (int h = 0; h < NH; ++h) {
@@ -978,15 +921,15 @@ __device__ void fast_side_sweep(const CallParams& p, int b, const UttMeta& m, co
 
   // ================================ phase 2 ================================
   int k2 = 0, ob = 0;                                  // ob: ring slot of the chunk's records, k2 mod D
-  for (int n0 = M_side; n0 < T; n0 += K, ++k2, ++cc) {
-    const int kc = min(K, T - n0), par = k2 & 1;
+  for (int n0 = M_side; n0 < T; n0 += kChunk, ++k2, ++cc) {
+    const int kc = min(kChunk, T - n0), par = k2 & 1;
     B200CTC_TRACE_EVENT(tc, 13);
-    run_chunk<K, true, SIDE, NT, NS>(c, ss, rs, par, ob, n0, kc, write_post);
+    run_chunk<true, SIDE>(c, ss, rs, par, ob, n0, kc, write_post);
     ob = ob + 1 == c.D ? 0 : ob + 1;
     B200CTC_TRACE_EVENT(tc, 14);
     // the barrier with the helpers is per chunk; the halo is good for KX frames after an exchange
-    const bool exchange = (k2 + 1) % (KX / K) == 0;
-    chunk_boundary<K, NWMAX, SIDE, NS, HW>(c, ss, xc, abort_flag, tc, exchange, !B200CTC_ABL(7) || exchange);
+    const bool exchange = (k2 + 1) % (kExchangeFrames / kChunk) == 0;
+    chunk_boundary<NWMAX, SIDE, HW>(c, ss, xc, abort_flag, tc, exchange);
     rs = (rs + 1) & (RCH - 1);
     xc += exchange ? 1 : 0;
   }
@@ -1100,15 +1043,15 @@ __device__ __forceinline__ void reduce_frame(const CallParams& p, const FastComm
 // of chunk c+1 needs (emission row; in phase 2 the other side's records of all position groups) and,
 // in phase 2, reduces the posteriors the lattice warps produced for its frame of chunk c-1 into the
 // gradient row.  It meets the lattice warps at the one barrier per chunk.
-template <int K, int NWMAX, int SIDE, int NS, bool CL, bool SPLIT, int ROLE>
+template <int NWMAX, int SIDE, bool CL, bool SPLIT, int ROLE>
 __device__ void fast_side_helper(const CallParams& p, int b, const UttMeta& m, const FastCommon& cm,
                                  unsigned char* side_smem, int hj, int lane) {
-  static_assert(kReducers == K, "one helper warp per frame of a chunk");
+  static_assert(kReducers == kChunk, "one helper warp per frame of a chunk");
   constexpr bool FETCH = ROLE != kReduceOnly, REDUCE = ROLE != kFetchOnly;
   FastCtx<SIDE> c;
-  fill_ctx<K, NWMAX, SIDE, NS>(c, p, b, m, side_smem, NWMAX + hj, lane);
+  fill_ctx<NWMAX, SIDE>(c, p, b, m, side_smem, NWMAX + hj, lane);
   const int T = c.T, NW = c.NW, V = p.V;
-  const SidePlan pl = side_plan<K, SIDE>(T);
+  const SidePlan pl = side_plan(T, SIDE);
   const int M_side = pl.M_side;
   const int nbar = (NW + helper_warps<CL>()) * 32;
   B200CTC_TRACE_DECL(tc);
@@ -1123,15 +1066,15 @@ __device__ void fast_side_helper(const CallParams& p, int b, const UttMeta& m, c
 
   // Emission rows are staged two barrier intervals ahead (ring slot = chunk & (RCH - 1)), so that the
   // global-memory latency of a row never sits between the lattice warps and a barrier.
-  constexpr int KX = exchange_frames<K, NS>(), M = KX / K, RCH = kRowsRing * M;
+  constexpr int M = kExchangeFrames / kChunk, RCH = kRowsRing * M;
   const int nc1 = pl.nc1, n_chunks = pl.n_chunks;
-  auto chunk_start = [&](int cc) { return cc < nc1 ? cc * K : M_side + (cc - nc1) * K; };
+  auto chunk_start = [&](int cc) { return cc < nc1 ? cc * kChunk : M_side + (cc - nc1) * kChunk; };
   int staged = 0;                                    // chunks [0, staged) have been requested
   auto stage_upto = [&](int end) {                   // one cp.async group: this warp's row of chunks [staged, end)
     if (FETCH) {
       for (; staged < min(end, n_chunks); ++staged) {
         const int n = chunk_start(staged) + hj;
-        if (n < T) stage_row<SIDE>(c, (staged & (RCH - 1)) * K + hj, n);   // a row past a short chunk is harmless
+        if (n < T) stage_row<SIDE>(c, (staged & (RCH - 1)) * kChunk + hj, n);   // a row past a short chunk is harmless
       }
       cp_async_commit();
     }
@@ -1158,11 +1101,11 @@ __device__ void fast_side_helper(const CallParams& p, int b, const UttMeta& m, c
   // chunks go into slots 0 .. D - 2 here; the loop below keeps its slot and phase counters incrementally.
   const int nc2 = pl.nc2;
   for (int q = 0; FETCH && q < D - 1; ++q) {
-    const int n = M_side + q * K + hj;
-    if (!B200CTC_ABL(10) && q < nc2 && n < T) prefetch_other<SIDE>(c, q * K + hj, n, mbar + q);
+    const int n = M_side + q * kChunk + hj;
+    if (q < nc2 && n < T) prefetch_other<SIDE>(c, q * kChunk + hj, n, mbar + q);
   }
   auto landed = [&](int n, int slot, unsigned phase) {       // the copy for step n (if there was one) has arrived
-    if (FETCH && !B200CTC_ABL(10) && !B200CTC_ABL(11) && n < T)
+    if (FETCH && n < T)
       if (!mbar_wait(mbar + slot, phase) && lane == 0) *cm.abort_flag = 1;   // never observed; the safe lattice would redo the utterance
   };
   landed(M_side + hj, 0, 0u);
@@ -1172,7 +1115,7 @@ __device__ void fast_side_helper(const CallParams& p, int b, const UttMeta& m, c
     float inv_mP; int eP; double log2P;
     if (!total_probability(c.sm, NW, inv_mP, eP, log2P)) return;
   }
-  const bool reduce = REDUCE && p.grads != nullptr && !B200CTC_ABL(9);   // ablation 9: helpers do not reduce (timing only)
+  const bool reduce = REDUCE && p.grads != nullptr;
 
   const int n_seg = *cm.ix.n_seg, max_n4 = cm.max_n4[0];
   ReducerLane rl;                                     // this lane's reducer groups (lane, lane + 32)
@@ -1200,26 +1143,26 @@ __device__ void fast_side_helper(const CallParams& p, int b, const UttMeta& m, c
   // By now every chunk phase 1's look-ahead requested is a phase-2 chunk or the last chunk of phase 1.
   const int sgn = SIDE ? -1 : 1;
   // (a) emission rows: chunk `staged` is the next one to request (at most one per iteration)
-  const int st_adv = sgn * K * c.st_stride;
+  const int st_adv = sgn * kChunk * c.st_stride;
   const char* st_src = c.st_src + (long long)c.frame_of(chunk_start(staged) + hj) * c.st_stride;
   int st_n = chunk_start(staged) + hj;
   // (b) the opposite side's records: chunk k2 + D - 1 goes into ring slot (k2 - 1) mod D; chunk k2 + 1 is awaited
-  const int rec_adv = sgn * K * c.FB;
-  int rec_n = M_side + (D - 1) * K + hj;
+  const int rec_adv = sgn * kChunk * c.FB;
+  int rec_n = M_side + (D - 1) * kChunk + hj;
   int f_slot = D - 1;                                          // slot of chunk k2 + D - 1
-  int l_slot = 1 % D, l_n = M_side + K + hj;                   // slot, step and mbarrier phase of chunk k2 + 1
+  int l_slot = 1 % D, l_n = M_side + kChunk + hj;              // slot, step and mbarrier phase of chunk k2 + 1
   unsigned l_phase = D == 1 ? 1u : 0u;
   const unsigned char* rec_src = c.scr + (long long)c.frame_of(rec_n) * c.FB;
   // (c) the row reduce_frame updates: the gradient row of the frame, or (gathered mode) the frame's emission row in
   // the workspace, which nobody reads any more once its posteriors exist and which becomes its occupancy row
   const long long out_stride = p.gathered ? (long long)m.W : (long long)p.B * V;
   float* out = (p.gathered ? p.em + m.em_off : p.grads + (long long)b * V) + (long long)c.frame_of(M_side + hj) * out_stride;
-  const long long out_adv = sgn * K * out_stride;
+  const long long out_adv = sgn * kChunk * out_stride;
   const unsigned zero16 = smem_u32(c.sm.rows + c.RW);          // the zero slot of emission row 0
   const float* post_hj = c.sm.post + (size_t)hj * c.PS;
-  const int post_half = K * c.PS;                               // floats per posterior buffer
+  const int post_half = kChunk * c.PS;                          // floats per posterior buffer
   const float* rows_hj = c.sm.rows + (size_t)hj * c.RWS;
-  const int row_chunk = K * c.RWS;                              // floats per chunk slot of the row ring
+  const int row_chunk = kChunk * c.RWS;                         // floats per chunk slot of the row ring
   const unsigned st_dst_hj = c.st_dst + (unsigned)(hj * c.RWS * 4);
 
   int k2 = 0;
@@ -1227,15 +1170,15 @@ __device__ void fast_side_helper(const CallParams& p, int b, const UttMeta& m, c
     B200CTC_TRACE_EVENT(tc, 7);
     if (FETCH && staged < cc + 3 && staged < n_chunks) {   // chunk cc+2 (nothing to do while phase 1's look-ahead lasts)
       if (st_n < T) stage_row_at<SIDE>(c, st_dst_hj + (unsigned)((staged & (RCH - 1)) * row_chunk * 4), st_src);   // a row past a short chunk is harmless
-      ++staged; st_n += K; st_src += st_adv;
+      ++staged; st_n += kChunk; st_src += st_adv;
     }
     if (FETCH) cp_async_commit();
-    if (FETCH && !B200CTC_ABL(10) && rec_n < T && lane == 0) {
+    if (FETCH && rec_n < T && lane == 0) {
       unsigned long long* mb = mbar + f_slot;
       mbar_expect_tx(mb, (unsigned)c.FB);
-      bulk_g2s(c.sm.oth + (size_t)(f_slot * K + hj) * c.FB, rec_src, (unsigned)c.FB, mb);
+      bulk_g2s(c.sm.oth + (size_t)(f_slot * kChunk + hj) * c.FB, rec_src, (unsigned)c.FB, mb);
     }
-    rec_n += K; rec_src += rec_adv;
+    rec_n += kChunk; rec_src += rec_adv;
     f_slot = f_slot + 1 == D ? 0 : f_slot + 1;
     B200CTC_TRACE_EVENT(tc, 8);
     if (reduce && k2 >= 1) {                          // frame hj of the previous chunk (it was a full chunk)
@@ -1247,12 +1190,12 @@ __device__ void fast_side_helper(const CallParams& p, int b, const UttMeta& m, c
     B200CTC_TRACE_EVENT(tc, 9);
     if (FETCH) cp_async_wait<1>();
     landed(l_n, l_slot, l_phase);
-    l_n += K;
+    l_n += kChunk;
     if (++l_slot == D) { l_slot = 0; l_phase ^= 1u; }
-    if (!B200CTC_ABL(7) || (k2 + 1) % (KX / K) == 0) named_bar_sync(bar_chunk(SIDE), nbar);
+    named_bar_sync(bar_chunk(SIDE), nbar);
   }
   // the last chunk
-  if (reduce && M_side + (k2 - 1) * K + hj < T) {
+  if (reduce && M_side + (k2 - 1) * kChunk + hj < T) {
     const float* post_row = post_hj + ((k2 - 1) & 1) * post_half;
     const float* y_row = rows_hj + ((cc - 1) & (RCH - 1)) * row_chunk;
     reduce_frame<NWMAX, SPLIT>(p, cm, post_row, y_row, out, zero16, c.RC, NW, n_seg, max_n4, rl, lane);
@@ -1265,7 +1208,7 @@ __device__ void fast_side_helper(const CallParams& p, int b, const UttMeta& m, c
 // caller reads it after a __syncthreads()).
 // CL (cluster variant): the CTA holds ONE side -- the one its rank in the two-CTA cluster names -- with NWMAX
 // lattice warps and kReducers helper warps; both CTAs run the (cheap) prologue.
-template <int K, int NWMAX, int NS, bool CL = false>
+template <int NWMAX, bool CL = false>
 __device__ void lattice_fast_utterance(const CallParams& p, int b, unsigned char* smem, int** smem_abort) {
   const UttMeta m = p.meta[b];
   const int L = m.L;
@@ -1274,7 +1217,7 @@ __device__ void lattice_fast_utterance(const CallParams& p, int b, unsigned char
   // the shuffles of the frame loops need no convergence check (BRA.DIV) in front of them: measured on B200, C3
   // (four windows) 0.1967 -> 0.1930 ms per step, C2 (two windows) 0.2674 -> 0.2652, but C1 (one window, where
   // ptxas then allocates 91 registers instead of 105) 0.138 -> 0.156 -- hence only for NWMAX > 1.
-  const int NW = NWMAX > 1 ? __shfl_sync(0xffffffffu, fast_warps_needed<K, NS>(L), 0) : fast_warps_needed<K, NS>(L);
+  const int NW = NWMAX > 1 ? __shfl_sync(0xffffffffu, fast_warps_needed(L), 0) : fast_warps_needed(L);
   const int warp = NWMAX > 1 ? __shfl_sync(0xffffffffu, (int)(threadIdx.x >> 5), 0) : (int)(threadIdx.x >> 5);
   const int lane = threadIdx.x & 31;
   const int side = CL ? (int)cluster_ctarank() : warp / (NWMAX + kReducers);
@@ -1305,7 +1248,7 @@ __device__ void lattice_fast_utterance(const CallParams& p, int b, unsigned char
   size_t common = (size_t)(reinterpret_cast<unsigned char*>(ip) - smem);
   common = (common + 15) / 16 * 16;
   const int RW = p.gathered ? m.W : (p.V + 3) / 4 * 4;
-  const size_t side_bytes = fast_side_bytes<K, NWMAX, NS>(L, RW, p.V, p.oth_depth);
+  const size_t side_bytes = fast_side_bytes<NWMAX>(L, RW, p.V, p.oth_depth);
   *smem_abort = cm.abort_flag;
 
   // ---- prologue (all threads of the CTA) ----
@@ -1318,8 +1261,8 @@ __device__ void lattice_fast_utterance(const CallParams& p, int b, unsigned char
   {
     const int PS = post_stride<NWMAX>(L, p.V);
     for (int sd = 0; sd < (CL ? 1 : 2); ++sd) {
-      FastSideSmem s = carve_fast_side<K, NWMAX, NS>(smem + common + sd * side_bytes, L, RW, p.V, p.oth_depth);
-      for (int i = threadIdx.x; i < 2 * K * PS; i += blockDim.x) s.post[i] = 0.f;
+      FastSideSmem s = carve_fast_side<NWMAX>(smem + common + sd * side_bytes, L, RW, p.V, p.oth_depth);
+      for (int i = threadIdx.x; i < 2 * kChunk * PS; i += blockDim.x) s.post[i] = 0.f;
     }
   }
   __syncthreads();
@@ -1368,7 +1311,7 @@ __device__ void lattice_fast_utterance(const CallParams& p, int b, unsigned char
         const int cost0 = slots0 * mx4 * 8;
         auto split_cost = [](int slots, int r, int pm) { return slots * r * 8 + (pm - 1) * 12 + 16; };
         int lo = max(1, (tot4 + limit - 1) / limit), hi = mx4 - 1;
-        if (B200CTC_GROUP_SPLIT && lo <= hi && mx4 <= 128 && 4 * split_cost(1, lo, 2) <= 3 * cost0) {
+        if (lo <= hi && mx4 <= 128 && 4 * split_cost(1, lo, 2) <= 3 * cost0) {
           auto pieces = [&](int r, int& pm) {
             const unsigned m = 65536u / (unsigned)r + 1u;
             const int p0 = (int)(((unsigned)(g4[0] + r - 1) * m) >> 16), p1 = (int)(((unsigned)(g4[1] + r - 1) * m) >> 16);
@@ -1468,33 +1411,33 @@ __device__ void lattice_fast_utterance(const CallParams& p, int b, unsigned char
   }
   unsigned char* side_smem = smem + common + (CL ? 0 : side) * side_bytes;
   if (w >= 0 && w < NW) {
-    if (side == 0) fast_side_sweep<K, NWMAX, 0, NS, CL>(p, b, m, cm, side_smem, w, lane);
-    else           fast_side_sweep<K, NWMAX, 1, NS, CL>(p, b, m, cm, side_smem, w, lane);
+    if (side == 0) fast_side_sweep<NWMAX, 0, CL>(p, b, m, cm, side_smem, w, lane);
+    else           fast_side_sweep<NWMAX, 1, CL>(p, b, m, cm, side_smem, w, lane);
   } else if (CL && w >= NWMAX) {
     // cluster variant: helper warps NWMAX .. NWMAX + 3 fetch, NWMAX + 4 .. NWMAX + 7 reduce (frame hj of every chunk each)
-    const bool split = B200CTC_GROUP_SPLIT && __builtin_expect(cm.max_n4[2] > 1, 0);
+    const bool split = __builtin_expect(cm.max_n4[2] > 1, 0);
     const int hw = w - NWMAX;
     if (hw < kReducers) {
-      if (side == 0) fast_side_helper<K, NWMAX, 0, NS, CL, false, kFetchOnly>(p, b, m, cm, side_smem, hw, lane);
-      else           fast_side_helper<K, NWMAX, 1, NS, CL, false, kFetchOnly>(p, b, m, cm, side_smem, hw, lane);
+      if (side == 0) fast_side_helper<NWMAX, 0, CL, false, kFetchOnly>(p, b, m, cm, side_smem, hw, lane);
+      else           fast_side_helper<NWMAX, 1, CL, false, kFetchOnly>(p, b, m, cm, side_smem, hw, lane);
     } else if (!split) {
-      if (side == 0) fast_side_helper<K, NWMAX, 0, NS, CL, false, kReduceOnly>(p, b, m, cm, side_smem, hw - kReducers, lane);
-      else           fast_side_helper<K, NWMAX, 1, NS, CL, false, kReduceOnly>(p, b, m, cm, side_smem, hw - kReducers, lane);
+      if (side == 0) fast_side_helper<NWMAX, 0, CL, false, kReduceOnly>(p, b, m, cm, side_smem, hw - kReducers, lane);
+      else           fast_side_helper<NWMAX, 1, CL, false, kReduceOnly>(p, b, m, cm, side_smem, hw - kReducers, lane);
     } else {
-      if (side == 0) fast_side_helper<K, NWMAX, 0, NS, CL, true, kReduceOnly>(p, b, m, cm, side_smem, hw - kReducers, lane);
-      else           fast_side_helper<K, NWMAX, 1, NS, CL, true, kReduceOnly>(p, b, m, cm, side_smem, hw - kReducers, lane);
+      if (side == 0) fast_side_helper<NWMAX, 0, CL, true, kReduceOnly>(p, b, m, cm, side_smem, hw - kReducers, lane);
+      else           fast_side_helper<NWMAX, 1, CL, true, kReduceOnly>(p, b, m, cm, side_smem, hw - kReducers, lane);
     }
   } else if (w >= NWMAX) {
     // (a second instantiation of the helper rather than a branch in its loop: the combination of split symbol
     // groups costs the unsplit case 5 % of the step by merely being in the loop body; out of line -- __noinline__ --
     // it costs every case 10-15 %: a 448-byte stack frame and the call ABI's register constraints)
-    const bool split = B200CTC_GROUP_SPLIT && __builtin_expect(cm.max_n4[2] > 1, 0);
+    const bool split = __builtin_expect(cm.max_n4[2] > 1, 0);
     if (!split) {
-      if (side == 0) fast_side_helper<K, NWMAX, 0, NS, CL, false, kFetchAndReduce>(p, b, m, cm, side_smem, w - NWMAX, lane);
-      else           fast_side_helper<K, NWMAX, 1, NS, CL, false, kFetchAndReduce>(p, b, m, cm, side_smem, w - NWMAX, lane);
+      if (side == 0) fast_side_helper<NWMAX, 0, CL, false, kFetchAndReduce>(p, b, m, cm, side_smem, w - NWMAX, lane);
+      else           fast_side_helper<NWMAX, 1, CL, false, kFetchAndReduce>(p, b, m, cm, side_smem, w - NWMAX, lane);
     } else {
-      if (side == 0) fast_side_helper<K, NWMAX, 0, NS, CL, true, kFetchAndReduce>(p, b, m, cm, side_smem, w - NWMAX, lane);
-      else           fast_side_helper<K, NWMAX, 1, NS, CL, true, kFetchAndReduce>(p, b, m, cm, side_smem, w - NWMAX, lane);
+      if (side == 0) fast_side_helper<NWMAX, 0, CL, true, kFetchAndReduce>(p, b, m, cm, side_smem, w - NWMAX, lane);
+      else           fast_side_helper<NWMAX, 1, CL, true, kFetchAndReduce>(p, b, m, cm, side_smem, w - NWMAX, lane);
     }
   } else if (CL) {
     cluster_sync_all();          // an idle warp: the midpoint rendezvous counts every thread of the cluster
