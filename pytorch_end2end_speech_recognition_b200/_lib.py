@@ -1,4 +1,5 @@
-"""ctypes binding of the C-ABI library (include/b200ctc.h).
+"""ctypes binding of the C-ABI library (include/b200ctc.h) for the decoders, evaluation and diagnostics; the
+loss goes through the PyTorch extension (csrc/torch_binding.cpp).
 
 The shared library is built in-tree by ``build.py`` (``lib/libb200ctc.so``).  There is no
 fallback implementation: if the library cannot be loaded every product entry point raises.
@@ -38,18 +39,14 @@ EXPORTED_SYMBOLS = (
 )
 
 
-class Options(ctypes.Structure):
-    """b200ctc_options (include/b200ctc.h): fused call-site arithmetic of the device-resident call."""
-    _fields_ = [("logit_scale", ctypes.c_float), ("label_smoothing", ctypes.c_float),
-                ("loss_scale", ctypes.c_float), ("grad_scale", ctypes.c_float)]
-
-
 class B200CTCError(RuntimeError):
     """Raised for every non-zero status of the C ABI (a RuntimeError, so the reference's
     skip-mini-batch guard, utils/training/training_loop.py:69-76, keeps working)."""
 
 
-def _declare(lib):
+def declare(lib):
+    """Set the ctypes signatures of ``lib``'s entry points (any build of the library, variants included) and
+    return it.  b200ctc_loss_and_grad_dev is left undeclared: only the PyTorch extension calls it."""
     c_int_p = ctypes.POINTER(ctypes.c_int)
     lib.b200ctc_version.restype = ctypes.c_int
     lib.b200ctc_version.argtypes = []
@@ -75,17 +72,6 @@ def _declare(lib):
     lib.b200ctc_get_workspace_bound.restype = ctypes.c_int
     lib.b200ctc_get_workspace_bound.argtypes = [ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_int,
                                                 ctypes.POINTER(ctypes.c_size_t)]
-    lib.b200ctc_loss_and_grad_dev.restype = ctypes.c_int
-    lib.b200ctc_loss_and_grad_dev.argtypes = [
-        ctypes.c_void_p,                                   # handle
-        ctypes.c_void_p, ctypes.c_int64, ctypes.c_int64,   # acts, stride_t, stride_b
-        ctypes.c_void_p,                                   # grads
-        ctypes.c_void_p, ctypes.c_int, ctypes.c_void_p, ctypes.c_void_p,   # labels, label_stride, label_lens, act_lens (device)
-        ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_int,  # T, V, B, max_label_len, blank
-        ctypes.POINTER(Options),                           # opts (nullable)
-        ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, # costs, loss_sum, ls_costs (device)
-        ctypes.c_void_p, ctypes.c_size_t, ctypes.c_void_p  # workspace, bytes, stream
-    ]
     lib.b200ctc_get_plan_cache_stats.restype = ctypes.c_int
     lib.b200ctc_get_plan_cache_stats.argtypes = [ctypes.c_void_p, ctypes.POINTER(ctypes.c_longlong),
                                                  ctypes.POINTER(ctypes.c_longlong)]
@@ -143,7 +129,7 @@ def load(build_if_missing=True):
                 if not os.path.exists(path):
                     raise B200CTCError("cannot build libb200ctc.so: %s" % exc)
         try:
-            _LIB = _declare(ctypes.CDLL(path))
+            _LIB = declare(ctypes.CDLL(path))
         except OSError as exc:
             raise B200CTCError("cannot load %s: %s" % (path, exc))
         return _LIB

@@ -14,7 +14,8 @@ PKG_DIR = os.path.dirname(os.path.abspath(__file__))
 REPO_DIR = os.path.dirname(PKG_DIR)
 CSRC = os.path.join(PKG_DIR, "csrc")
 LIB_DIR = os.path.join(PKG_DIR, "lib")
-LIB_PATH = os.environ.get("B200CTC_LIB") or os.path.join(LIB_DIR, "libb200ctc.so")   # B200CTC_LIB: developer variants
+LIB_DEFAULT = os.path.join(LIB_DIR, "libb200ctc.so")       # what build_library() builds
+LIB_PATH = os.environ.get("B200CTC_LIB") or LIB_DEFAULT    # what the package loads; B200CTC_LIB: a developer variant
 
 SOURCES = ["api.cu", "plan.cu", "softmax_rows.cu", "lattice.cu", "greedy.cu", "beam.cu", "eval.cu"]
 
@@ -56,15 +57,24 @@ def _stale(target, deps, flags=()):
         return True
 
 
+def _link(objs, out):
+    # the link step names the architecture too: without it nvcc adds an (empty) sm_52 device-link stub.  Every
+    # build, variants included, is named libb200ctc.so (SONAME): the extension's dependency on libb200ctc.so then
+    # resolves to whichever copy the process loaded first, so B200CTC_LIB redirects the whole process.
+    subprocess.run([_nvcc(), "-shared", "-gencode", "arch=compute_100a,code=sm_100a", "-Xlinker", "-soname=libb200ctc.so",
+                    "-o", out] + objs + ["-Xcompiler", "-fPIC"], check=True)
+
+
 def build_library(force=False, verbose=False, extra_flags=(), lib_path=None):
     """Compile csrc/*.cu into lib/libb200ctc.so (no-op when up to date).  ``extra_flags`` /
-    ``lib_path`` build a developer variant next to it (tools/trace_lattice.py: -DB200CTC_TRACE)."""
+    ``lib_path`` build a developer variant next to it (tools/trace_lattice.py: -DB200CTC_TRACE).
+    B200CTC_LIB never names the output: it selects what is loaded, not what is built."""
     os.makedirs(LIB_DIR, exist_ok=True)
     if lib_path is not None:
         return _build_variant(list(extra_flags), lib_path, verbose)
     deps = [os.path.join(CSRC, f) for f in os.listdir(CSRC)] + [os.path.join(REPO_DIR, "include", "b200ctc.h")]
-    if not force and not _stale(LIB_PATH, deps, NVCC_FLAGS):
-        return LIB_PATH
+    if not force and not _stale(LIB_DEFAULT, deps, NVCC_FLAGS):
+        return LIB_DEFAULT
     objs = []
     for src in SOURCES:
         obj = os.path.join(LIB_DIR, src.replace(".cu", ".o"))
@@ -75,12 +85,10 @@ def build_library(force=False, verbose=False, extra_flags=(), lib_path=None):
             print(" ".join(cmd), file=sys.stderr)
         subprocess.run(cmd, check=True)
         objs.append(obj)
-    # the link step names the architecture too: without it nvcc adds an (empty) sm_52 device-link stub
-    cmd = [_nvcc(), "-shared", "-gencode", "arch=compute_100a,code=sm_100a", "-o", LIB_PATH] + objs + ["-Xcompiler", "-fPIC"]
-    subprocess.run(cmd, check=True)
-    with open(LIB_PATH + ".srchash", "w") as f:
+    _link(objs, LIB_DEFAULT)
+    with open(LIB_DEFAULT + ".srchash", "w") as f:
         f.write(_source_hash(deps, NVCC_FLAGS))
-    return LIB_PATH
+    return LIB_DEFAULT
 
 
 def _build_variant(extra_flags, lib_path, verbose):
@@ -94,8 +102,7 @@ def _build_variant(extra_flags, lib_path, verbose):
             print(" ".join(cmd), file=sys.stderr)
         subprocess.run(cmd, check=True)
         objs.append(obj)
-    subprocess.run([_nvcc(), "-shared", "-gencode", "arch=compute_100a,code=sm_100a", "-o", lib_path] + objs +
-                   ["-Xcompiler", "-fPIC"], check=True)
+    _link(objs, lib_path)
     return lib_path
 
 
@@ -110,11 +117,10 @@ def extension_path():
 
 def build_extension(force=False, verbose=False):
     """Compile csrc/torch_binding.cpp -- the thin PyTorch C++ extension over the C ABI -- in-tree with the host
-    compiler against this interpreter's torch headers, linked to lib/libb200ctc.so (rpath $ORIGIN/..).
+    compiler against this interpreter's torch headers, linked to the in-tree lib/libb200ctc.so (rpath $ORIGIN/..).
     Returns the path of the extension module; a no-op when its source hash is unchanged."""
     import sysconfig
     import torch
-    from torch.utils import cpp_extension
     build_library()
     os.makedirs(EXT_DIR, exist_ok=True)
     src = os.path.join(CSRC, "torch_binding.cpp")
@@ -123,6 +129,7 @@ def build_extension(force=False, verbose=False):
     flags = ["torch=" + torch.__version__, "py=" + sys.version.split()[0]]
     if not force and not _stale(out, deps, flags):
         return out
+    from torch.utils import cpp_extension
     cuda_home = os.environ.get("CUDA_HOME", "/usr/local/cuda")
     inc = ["-I" + p for p in cpp_extension.include_paths()] + ["-I" + os.path.join(cuda_home, "include"),
            "-I" + sysconfig.get_paths()["include"], "-I" + os.path.join(REPO_DIR, "include")]

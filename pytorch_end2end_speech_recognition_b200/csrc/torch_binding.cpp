@@ -1,8 +1,8 @@
 // Thin PyTorch C++ extension over the C ABI (include/b200ctc.h): what replaces warp-ctc's pytorch_binding
 // (tools/install_warpctc_pytorch.sh:12-18 builds `pytorch_binding/setup.py install`; reference call site
 // models/pytorch_v3/ctc/ctc.py:35,39-45).  PyTorch supplies device memory, the current stream and the tensor
-// checks; every computation happens behind the C ABI in libb200ctc.so.  The Python layer (ctc.py) uses this
-// module when it is built and the ctypes binding (_lib.py) otherwise: both call the same entry points.
+// checks; every computation happens behind the C ABI in libb200ctc.so.  It is the one binding of the loss
+// (ctc.py); the ctypes binding (_lib.py) serves the decoders, evaluation and diagnostics on the same handles.
 #include <torch/extension.h>
 #include <ATen/cuda/CUDAContext.h>
 #include <c10/cuda/CUDAGuard.h>

@@ -16,81 +16,60 @@ Native additions: ``ctc_loss_and_grad`` (device-resident results, no host sync) 
 """
 
 import ctypes
+import importlib.util
 import os
 
 import numpy as np
 import torch
 
 from . import _lib
+from . import build as _build
 from ._lib import B200CTCError
 
 _HANDLES = {}
-_WORKSPACES = {}     # (device index, stream handle) -> growing uint8 workspace tensor
-_EXT = None          # the PyTorch C++ extension over the C ABI (csrc/torch_binding.cpp), False when not built
+_EXT = None          # the PyTorch C++ extension over the C ABI (csrc/torch_binding.cpp), once loaded
 
 
 def _ext():
-    """The thin PyTorch C++ extension (north_star: "a thin PyTorch C++/CUDA extension over a C-ABI"), built
-    in-tree by ``__graft_entry__.build()`` / ``build.build_extension()``.  When it is not built (or
-    ``B200CTC_BINDING=ctypes``) the ctypes binding calls the same C entry points."""
+    """The thin PyTorch C++ extension (north_star: "a thin PyTorch C++/CUDA extension over a C-ABI"): the one
+    binding of the loss.  Built in-tree by ``__graft_entry__.build()``, and here when it is missing or stale, as
+    ``_lib.load()`` builds the library -- unless ``B200CTC_LIB`` selects a developer variant of the library, in
+    which case nothing is built on demand.  Raises B200CTCError when the extension cannot be built or imported."""
     global _EXT
     if _EXT is None:
-        _EXT = False
-        if os.environ.get("B200CTC_BINDING", "ext") != "ctypes":
+        # The library first: every build of it is named libb200ctc.so, so the extension's dependency on that name
+        # resolves to the copy already loaded (B200CTC_LIB's variant included) and the loss and the ctypes
+        # diagnostics share one library, and one set of handles, per process.
+        _lib.load()
+        path = _build.extension_path()
+        if not os.environ.get("B200CTC_LIB"):
             try:
-                import importlib.util
-                from . import build as _build
-                _lib.load()                                   # libb200ctc.so first (also builds it when missing)
-                path = _build.extension_path()
-                if os.path.exists(path):
-                    spec = importlib.util.spec_from_file_location(_build.EXT_NAME, path)
-                    mod = importlib.util.module_from_spec(spec)
-                    spec.loader.exec_module(mod)
-                    _EXT = mod
-            except Exception:                                 # an extension built for another torch / python: fall back
-                _EXT = False
+                _build.build_extension()
+            except Exception as exc:      # no host compiler: an extension that exists is used, as for the library
+                if not os.path.exists(path):
+                    raise B200CTCError("cannot build the PyTorch extension %s: %s" % (path, exc)) from exc
+        try:
+            spec = importlib.util.spec_from_file_location(_build.EXT_NAME, path)
+            mod = importlib.util.module_from_spec(spec)
+            spec.loader.exec_module(mod)
+        except Exception as exc:          # missing, or built for another torch / python
+            raise B200CTCError("cannot import the PyTorch extension %s: %s" % (path, exc)) from exc
+        _EXT = mod
     return _EXT
 
 
-def binding():
-    """'extension' or 'ctypes': which binding ``ctc_loss_and_grad`` goes through."""
-    return "extension" if _ext() else "ctypes"
-
-
 def _handle(device_index):
-    """One library handle per device (the handle serialises its calls with a mutex, include/b200ctc.h);
-    shared between the extension and the ctypes entry points (diagnostics, decoders)."""
+    """One library handle per device (the handle serialises its calls with a mutex, include/b200ctc.h), created
+    by the extension and shared with the ctypes entry points (diagnostics, decoders)."""
     h = _HANDLES.get(device_index)
     if h is None:
-        ext = _ext()
-        if ext:
-            hp = ctypes.c_void_p(ext.handle_address(int(device_index)))
-        else:
-            lib = _lib.load()
-            hp = ctypes.c_void_p()
-            _lib.check(lib.b200ctc_create(ctypes.byref(hp), int(device_index)), "b200ctc_create")
-        h = _HANDLES[device_index] = hp
+        h = _HANDLES[device_index] = ctypes.c_void_p(_ext().handle_address(int(device_index)))
     return h
-
-
-def _workspace(dev_index, stream, nbytes):
-    """Workspace of the calls issued on one stream of one device: allocated once and grown on demand (no
-    caching-allocator round trip per call).  Calls on one stream are ordered, so they can share it; calls on
-    another stream get their own -- which is also what keeps the buffer alive and un-recycled while kernels
-    of that stream still use it (no record_stream needed)."""
-    key = (dev_index, stream)
-    ws = _WORKSPACES.get(key)
-    if ws is None or ws.numel() < nbytes:
-        ws = torch.empty(max(int(nbytes * 1.25), 1 << 20), dtype=torch.uint8, device=torch.device("cuda", dev_index))
-        _WORKSPACES[key] = ws
-    return ws
 
 
 def release_workspaces():
     """Drop the cached workspaces (they are re-allocated on the next call)."""
-    _WORKSPACES.clear()
-    if _ext():
-        _ext().release_workspaces()
+    _ext().release_workspaces()
 
 
 def set_profiling(enable, device_index=None):
@@ -185,30 +164,6 @@ def workspace_bound(T, V, B, max_label_len):
     return n.value
 
 
-def _outputs(T, B, V, dev, grads, need_grad, costs, loss_sum):
-    if need_grad:
-        if grads is None:
-            grads = torch.empty((T, B, V), dtype=torch.float32, device=dev)
-        elif (not grads.is_cuda or grads.dtype != torch.float32 or tuple(grads.shape) != (T, B, V)
-              or not grads.is_contiguous()):
-            raise B200CTCError("grads must be a contiguous CUDA float32 tensor shaped like acts")
-    else:
-        grads = None
-    if costs is None:
-        costs = torch.empty(B, dtype=torch.float32, device=dev)
-    if loss_sum is None:
-        loss_sum = torch.empty(1, dtype=torch.float32, device=dev)
-    return grads, costs, loss_sum
-
-
-def _dev_i32(x, name, dev):
-    if not (isinstance(x, torch.Tensor) and x.is_cuda):
-        raise B200CTCError("%s must be a CUDA tensor when the labels are device-resident" % name)
-    if x.dtype != torch.int32 or not x.is_contiguous() or x.device != dev:
-        x = x.to(device=dev, dtype=torch.int32).contiguous()
-    return x
-
-
 def ctc_loss_and_grad(acts, labels, act_lens, label_lens, blank=0, grads=None, need_grad=True,
                       costs=None, loss_sum=None, max_label_len=None, logit_scale=1.0, label_smoothing=0.0,
                       loss_scale=1.0, grad_scale=1.0, ls_costs=None):
@@ -230,90 +185,21 @@ def ctc_loss_and_grad(acts, labels, act_lens, label_lens, blank=0, grads=None, n
     """
     _require_cuda(acts)
     ext = _ext()
-    if ext:
-        try:
-            if isinstance(labels, torch.Tensor) and labels.is_cuda:
-                return ext.loss_and_grad_dev(acts, labels, act_lens, label_lens, int(blank), grads, bool(need_grad), costs,
-                                             loss_sum, -1 if max_label_len is None else int(max_label_len),
-                                             float(logit_scale), float(label_smoothing), float(loss_scale),
-                                             float(grad_scale), ls_costs)
-            if logit_scale != 1.0 or label_smoothing != 0.0 or loss_scale != 1.0 or grad_scale != 1.0:
-                raise B200CTCError("logit_scale / label_smoothing / loss_scale / grad_scale need device-resident labels "
-                                   "(the warp-ctc style call has no such arguments); see ctc_loss_from_padded")
-            return ext.loss_and_grad_host(acts, _as_cpu_tensor(labels), _as_cpu_tensor(act_lens), _as_cpu_tensor(label_lens),
-                                          int(blank), grads, bool(need_grad), costs, loss_sum)
-        except B200CTCError:
-            raise
-        except (RuntimeError, TypeError) as exc:
-            raise B200CTCError(str(exc).split("\n")[0])
-    lib = _lib.load()
-    if acts.stride(2) != 1 and acts.size(2) > 1:
-        acts = acts.contiguous()
-    T, B, V = acts.shape
-    dev = acts.device
-    dev_index = dev.index if dev.index is not None else torch.cuda.current_device()
-    switch = torch.cuda.current_device() != dev_index
-    if switch:
-        prev_dev = torch.cuda.current_device()
-        torch.cuda.set_device(dev_index)
     try:
-        grads, costs, loss_sum = _outputs(T, B, V, dev, grads, need_grad, costs, loss_sum)
-        stream = torch.cuda.current_stream(dev).cuda_stream
         if isinstance(labels, torch.Tensor) and labels.is_cuda:
-            if labels.dim() != 2 or labels.size(0) != B:
-                raise B200CTCError("device-resident labels must be a padded [B, Lmax] tensor")
-            labels = labels if (labels.dtype == torch.int32 and labels.stride(1) == 1) else labels.to(torch.int32).contiguous()
-            act_lens_d = _dev_i32(act_lens, "act_lens", dev)
-            label_lens_d = _dev_i32(label_lens, "label_lens", dev)
-            if act_lens_d.numel() != B or label_lens_d.numel() != B:
-                raise B200CTCError("act_lens and label_lens must have one entry per utterance (B=%d)" % B)
-            Lmax = labels.size(1) if max_label_len is None else int(max_label_len)
-            if Lmax > labels.size(1):
-                raise B200CTCError("max_label_len exceeds the padded label width")
-            nbytes = ctypes.c_size_t()
-            _lib.check(lib.b200ctc_get_workspace_bound(T, V, B, Lmax, ctypes.byref(nbytes)), "b200ctc_get_workspace_bound")
-            workspace = _workspace(dev_index, stream, nbytes.value)
-            opts = None
-            if logit_scale != 1.0 or label_smoothing != 0.0 or loss_scale != 1.0 or grad_scale != 1.0:
-                opts = ctypes.byref(_lib.Options(float(logit_scale), float(label_smoothing), float(loss_scale),
-                                                 float(grad_scale)))
-            st = lib.b200ctc_loss_and_grad_dev(
-                _handle(dev_index), acts.data_ptr(), acts.stride(0), acts.stride(1),
-                grads.data_ptr() if grads is not None else None,
-                labels.data_ptr(), labels.stride(0) if B > 0 and labels.size(1) > 0 else Lmax,
-                label_lens_d.data_ptr(), act_lens_d.data_ptr(),
-                T, V, B, Lmax, int(blank), opts, costs.data_ptr(), loss_sum.data_ptr(),
-                ls_costs.data_ptr() if ls_costs is not None else None,
-                workspace.data_ptr(), workspace.numel(), stream)
-            _lib.check(st, "b200ctc_loss_and_grad_dev")
-            return costs, loss_sum, grads
+            return ext.loss_and_grad_dev(acts, labels, act_lens, label_lens, int(blank), grads, bool(need_grad), costs,
+                                         loss_sum, -1 if max_label_len is None else int(max_label_len),
+                                         float(logit_scale), float(label_smoothing), float(loss_scale),
+                                         float(grad_scale), ls_costs)
         if logit_scale != 1.0 or label_smoothing != 0.0 or loss_scale != 1.0 or grad_scale != 1.0:
             raise B200CTCError("logit_scale / label_smoothing / loss_scale / grad_scale need device-resident labels "
                                "(the warp-ctc style call has no such arguments); see ctc_loss_from_padded")
-        labels = _host_i32(labels, "labels")
-        act_lens = _host_i32(act_lens, "act_lens")
-        label_lens = _host_i32(label_lens, "label_lens")
-        if len(act_lens) != B or len(label_lens) != B:
-            raise B200CTCError("act_lens and label_lens must have one entry per utterance (B=%d)" % B)
-        if int(label_lens.sum()) != len(labels):
-            raise B200CTCError("sum(label_lens)=%d does not match len(labels)=%d" % (int(label_lens.sum()), len(labels)))
-        nbytes = ctypes.c_size_t()
-        _lib.check(lib.b200ctc_get_workspace_size(_i32_ptr(label_lens), _i32_ptr(act_lens), T, V, B,
-                                                  ctypes.byref(nbytes)), "b200ctc_get_workspace_size")
-        workspace = _workspace(dev_index, stream, nbytes.value)
-        st = lib.b200ctc_loss_and_grad(
-            _handle(dev_index),
-            acts.data_ptr(), acts.stride(0), acts.stride(1),
-            grads.data_ptr() if grads is not None else None,
-            _i32_ptr(labels), _i32_ptr(label_lens), _i32_ptr(act_lens),
-            T, V, B, int(blank),
-            costs.data_ptr(), loss_sum.data_ptr(),
-            workspace.data_ptr(), workspace.numel(), stream)
-        _lib.check(st, "b200ctc_loss_and_grad")
-    finally:
-        if switch:
-            torch.cuda.set_device(prev_dev)
-    return costs, loss_sum, grads
+        return ext.loss_and_grad_host(acts, _as_cpu_tensor(labels), _as_cpu_tensor(act_lens), _as_cpu_tensor(label_lens),
+                                      int(blank), grads, bool(need_grad), costs, loss_sum)
+    except B200CTCError:
+        raise
+    except (RuntimeError, TypeError) as exc:
+        raise B200CTCError(str(exc).split("\n")[0])
 
 
 # ------------------------------------------------------------------------------------------------

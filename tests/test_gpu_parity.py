@@ -1,5 +1,5 @@
-"""GPU parity tests proper: the CUDA path, called through the C ABI (ctypes binding), against the
-CPU oracle on identical inputs.  Tolerances are the ones BASELINE.json's north_star states:
+"""GPU parity tests proper: the CUDA path, called through the C ABI (the PyTorch extension for the loss,
+ctypes for the decoders), against the CPU oracle on identical inputs.  Tolerances are the ones BASELINE.json's north_star states:
 per-utterance loss within 1e-5 relative, gradients within 1e-4 absolute (fp32), decoded label
 sequences bit-exact."""
 import os

@@ -171,16 +171,47 @@ def test_evaluation_entry_points_have_no_cpu_path():
     assert lib.b200ctc_get_workspace_bound(100, 30, 4, 20, ctypes.byref(n)) == 0 and n.value > 0
 
 
-def test_torch_extension_builds_in_tree_and_loads():
+def test_torch_extension_builds_in_tree_and_is_the_loss_binding():
     """The thin PyTorch C++ extension over the C ABI: built next to the library (not into site-packages), so
-    that it travels with the repository snapshot and shows up as loaded native code."""
+    that it travels with the repository snapshot and shows up as loaded native code; the loss calls go through
+    that very module."""
     path = build.build_extension()
     assert path.startswith(ROOT) and os.path.exists(path)
     from pytorch_end2end_speech_recognition_b200 import ctc
-    if os.environ.get("B200CTC_BINDING", "ext") != "ctypes":
-        assert ctc.binding() == "extension"
-        with pytest.raises(RuntimeError):
-            ctc._ext().loss_and_grad_host(torch.zeros(2, 1, 3), torch.zeros(1), torch.zeros(1), torch.zeros(1))
+    assert os.path.samefile(ctc._ext().__file__, path)
+    with pytest.raises(RuntimeError):
+        ctc._ext().loss_and_grad_host(torch.zeros(2, 1, 3), torch.zeros(1), torch.zeros(1), torch.zeros(1))
+
+
+def test_library_variant_is_the_only_copy_in_the_process(tmp_path):
+    """B200CTC_LIB redirects the whole process: the extension's dependency on libb200ctc.so resolves, by SONAME,
+    to the variant the package loaded, so the loss and the ctypes diagnostics run one copy of the library."""
+    import shutil
+    import subprocess
+    import sys
+    build.build_extension()
+    variant = os.path.realpath(str(tmp_path / "libb200ctc_variant.so"))     # /proc/self/maps shows real paths
+    shutil.copy(build.LIB_DEFAULT, variant)
+    code = ("import sys; sys.path.insert(0, %r)\n"
+            "from pytorch_end2end_speech_recognition_b200 import ctc\n"
+            "ctc._ext()\n"
+            "print(sorted({l.split()[-1] for l in open('/proc/self/maps') if 'libb200ctc' in l}))\n" % ROOT)
+    env = dict(os.environ, B200CTC_LIB=variant)
+    out = subprocess.run([sys.executable, "-c", code], env=env, cwd=ROOT, check=True, capture_output=True, text=True)
+    assert out.stdout.strip().splitlines()[-1] == repr([variant])
+
+
+def test_extension_that_cannot_be_built_raises(monkeypatch, tmp_path):
+    """No fallback: when the extension can be neither built nor imported, the loss raises."""
+    from pytorch_end2end_speech_recognition_b200 import ctc
+
+    def fail(*args, **kwargs):
+        raise OSError("no host compiler")
+    monkeypatch.setattr(build, "build_extension", fail)
+    monkeypatch.setattr(build, "extension_path", lambda: str(tmp_path / "missing.so"))
+    monkeypatch.setattr(ctc, "_EXT", None)
+    with pytest.raises(b200.B200CTCError):
+        ctc._ext()
 
 
 def test_both_bench_arms_describe_the_same_config():

@@ -9,7 +9,7 @@ import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
-from pytorch_end2end_speech_recognition_b200 import workloads  # noqa: E402
+from pytorch_end2end_speech_recognition_b200 import _lib, workloads  # noqa: E402
 
 libs = [a for a in sys.argv[1:] if a.endswith(".so")]
 keys = [a for a in sys.argv[1:] if not a.endswith(".so")] or ["C1", "C3"]
@@ -21,18 +21,13 @@ for key in keys:
     grads = [torch.empty_like(a) for a in acts]
     costs, loss = torch.empty(wl.B, device="cuda"), torch.empty(1, device="cuda")
     for path in libs:
-        lib = ctypes.CDLL(path)
+        lib = _lib.declare(ctypes.CDLL(path))
         h = ctypes.c_void_p()
-        lib.b200ctc_create.argtypes = [ctypes.POINTER(ctypes.c_void_p), ctypes.c_int]
         assert lib.b200ctc_create(ctypes.byref(h), 0) == 0
-        lib.b200ctc_get_workspace_size.argtypes = [ip, ip, ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.POINTER(ctypes.c_size_t)]
         n = ctypes.c_size_t()
         ll, al, lab = wl.label_lens.ctypes.data_as(ip), wl.act_lens.ctypes.data_as(ip), wl.labels.ctypes.data_as(ip)
         assert lib.b200ctc_get_workspace_size(ll, al, wl.T, wl.V, wl.B, ctypes.byref(n)) == 0
         ws = torch.empty(n.value, dtype=torch.uint8, device="cuda")
-        lib.b200ctc_loss_and_grad.argtypes = [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int64, ctypes.c_int64, ctypes.c_void_p,
-                                              ip, ip, ip, ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_int,
-                                              ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_size_t, ctypes.c_void_p]
         stream = torch.cuda.current_stream().cuda_stream
 
         def step(i):
