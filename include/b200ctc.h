@@ -61,6 +61,13 @@ typedef enum {
 
 typedef struct b200ctc_handle b200ctc_handle;
 
+/* Element type of the logits (and of the gradient) of b200ctc_loss_and_grad_dev_typed. */
+typedef enum {
+  B200CTC_FLOAT32 = 0,
+  B200CTC_BFLOAT16 = 1,
+  B200CTC_FLOAT16 = 2
+} b200ctc_dtype_t;
+
 /*
  * Arithmetic of the reference's loss call site fused into the kernels (SURVEY 8(f) ranks 1-2), for
  * b200ctc_loss_and_grad_dev.  With z = logit_scale * acts and y = softmax(z):
@@ -177,6 +184,34 @@ B200CTC_API int b200ctc_loss_and_grad_dev(b200ctc_handle* handle,
                               void* workspace, size_t workspace_bytes, void* stream);
 
 /*
+ * b200ctc_loss_and_grad_dev for logits of element type `acts_dtype` (b200ctc_dtype_t); `grads` has the same element
+ * type.  A bfloat16 / float16 logit is widened to fp32 when it is loaded, and everything after that is the fp32
+ * evaluation of b200ctc_loss_and_grad_dev.  The gradient rows are formed in fp32 in a staging region of the
+ * workspace and rounded once, to nearest even, into `grads`; rows t >= act_lens[b] and rows of rejected or
+ * infeasible utterances are exact zeros.  costs, loss_sum and ls_costs stay fp32.  With B200CTC_FLOAT32 this is
+ * exactly b200ctc_loss_and_grad_dev.
+ *   workspace   DEVICE, >= b200ctc_get_workspace_bound_typed(T, V, B, max_label_len, acts_dtype, grads != NULL) bytes
+ */
+B200CTC_API int b200ctc_loss_and_grad_dev_typed(b200ctc_handle* handle, const void* acts, int64_t acts_stride_t, int64_t acts_stride_b, int acts_dtype, void* grads, const int* labels, int label_stride, const int* label_lens, const int* act_lens, int T, int V, int B, int max_label_len, int blank, const b200ctc_options* opts, float* costs, float* loss_sum, float* ls_costs, void* workspace, size_t workspace_bytes, void* stream);
+
+/*
+ * Workspace of b200ctc_loss_and_grad_dev_typed.  For B200CTC_FLOAT32, or without a gradient (need_grad == 0), it
+ * equals b200ctc_get_workspace_bound; a bfloat16 / float16 call with a gradient adds the fp32 [T,B,V] staging region
+ * (4 * T * B * V bytes, rounded up to 256).
+ */
+B200CTC_API int b200ctc_get_workspace_bound_typed(int T, int V, int B, int max_label_len, int dtype, int need_grad, size_t* bytes);
+
+/*
+ * Backward of a loss on bfloat16 / float16 logits: out[t,b,v] = grads[t,b,v] * scale[s], multiplied in fp32 and rounded
+ * once, to nearest even, to `dtype`; s = 0 when n_scale == 1 (one grad_output for the whole loss), s = b when
+ * n_scale == B (one per utterance).
+ *   grads, out  DEVICE [T,B,V] contiguous, of type dtype (B200CTC_BFLOAT16 or B200CTC_FLOAT16); may be the same buffer
+ *   scale       DEVICE fp32 [n_scale]
+ * One kernel launch on `stream`.
+ */
+B200CTC_API int b200ctc_scale_grads(const void* grads, void* out, int dtype, int T, int B, int V, const float* scale, int n_scale, void* stream);
+
+/*
  * Batched best-path decoder; replaces the numpy loops of
  * models/pytorch_v3/ctc/decoders/greedy_decoder.py:32-45 (per-frame argmax with
  * first-index tie break, collapse repeats, then drop blanks).
@@ -245,7 +280,9 @@ B200CTC_API int b200ctc_softmax_temperature(const float* logits, int64_t stride_
  * Measurement hooks (no counterpart in the reference; used by bench.py for the roofline line).
  * With profiling enabled every b200ctc_loss_and_grad call on this handle brackets each of its
  * kernels with CUDA events on `stream`; b200ctc_get_last_kernel_ms waits for the last call and
- * returns the device time of {softmax rows, lattice, cost sum} in milliseconds.
+ * returns the device time of {softmax rows, lattice, gradient completion} in milliseconds.  The third
+ * slot holds the occupancy pass of large vocabularies and, for bfloat16 / float16 logits, the pass
+ * that rounds the fp32 staged gradient into the caller's buffer.
  */
 B200CTC_API int b200ctc_set_profiling(b200ctc_handle* handle, int enable);
 B200CTC_API int b200ctc_get_last_kernel_ms(b200ctc_handle* handle, float* ms3);

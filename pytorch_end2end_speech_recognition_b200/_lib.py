@@ -15,6 +15,7 @@ _LOCK = threading.Lock()
 _LIB = None
 
 STATUS_SUCCESS = 0
+FLOAT32, BFLOAT16, FLOAT16 = 0, 1, 2     # b200ctc_dtype_t
 
 # every symbol include/b200ctc.h declares (tests check that the library exports all of them)
 EXPORTED_SYMBOLS = (
@@ -26,6 +27,9 @@ EXPORTED_SYMBOLS = (
     "b200ctc_get_workspace_bound",
     "b200ctc_loss_and_grad",
     "b200ctc_loss_and_grad_dev",
+    "b200ctc_loss_and_grad_dev_typed",
+    "b200ctc_get_workspace_bound_typed",
+    "b200ctc_scale_grads",
     "b200ctc_greedy_decode",
     "b200ctc_beam_search_workspace",
     "b200ctc_beam_search",
@@ -72,6 +76,23 @@ def declare(lib):
     lib.b200ctc_get_workspace_bound.restype = ctypes.c_int
     lib.b200ctc_get_workspace_bound.argtypes = [ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_int,
                                                 ctypes.POINTER(ctypes.c_size_t)]
+    lib.b200ctc_get_workspace_bound_typed.restype = ctypes.c_int
+    lib.b200ctc_get_workspace_bound_typed.argtypes = [ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_int,
+                                                      ctypes.c_int, ctypes.c_int, ctypes.POINTER(ctypes.c_size_t)]
+    lib.b200ctc_loss_and_grad_dev_typed.restype = ctypes.c_int
+    lib.b200ctc_loss_and_grad_dev_typed.argtypes = [
+        ctypes.c_void_p,                                                 # handle
+        ctypes.c_void_p, ctypes.c_int64, ctypes.c_int64, ctypes.c_int,   # acts, stride_t, stride_b, acts_dtype
+        ctypes.c_void_p,                                                 # grads (acts_dtype)
+        ctypes.c_void_p, ctypes.c_int, ctypes.c_void_p, ctypes.c_void_p,   # labels, label_stride, label_lens, act_lens
+        ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_int,  # T, V, B, max_label_len, blank
+        ctypes.c_void_p,                                                 # options or NULL
+        ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p,               # costs, loss_sum, ls_costs (device fp32)
+        ctypes.c_void_p, ctypes.c_size_t, ctypes.c_void_p                # workspace, bytes, stream
+    ]
+    lib.b200ctc_scale_grads.restype = ctypes.c_int
+    lib.b200ctc_scale_grads.argtypes = [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int, ctypes.c_int, ctypes.c_int,
+                                        ctypes.c_int, ctypes.c_void_p, ctypes.c_int, ctypes.c_void_p]
     lib.b200ctc_get_plan_cache_stats.restype = ctypes.c_int
     lib.b200ctc_get_plan_cache_stats.argtypes = [ctypes.c_void_p, ctypes.POINTER(ctypes.c_longlong),
                                                  ctypes.POINTER(ctypes.c_longlong)]

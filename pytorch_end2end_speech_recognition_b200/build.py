@@ -17,7 +17,7 @@ LIB_DIR = os.path.join(PKG_DIR, "lib")
 LIB_DEFAULT = os.path.join(LIB_DIR, "libb200ctc.so")       # what build_library() builds
 LIB_PATH = os.environ.get("B200CTC_LIB") or LIB_DEFAULT    # what the package loads; B200CTC_LIB: a developer variant
 
-SOURCES = ["api.cu", "plan.cu", "softmax_rows.cu", "lattice.cu", "greedy.cu", "beam.cu", "eval.cu"]
+SOURCES = ["api.cu", "plan.cu", "softmax_rows.cu", "lattice.cu", "narrow_grads.cu", "greedy.cu", "beam.cu", "eval.cu"]
 
 NVCC_FLAGS = [
     "-O3", "-std=c++17",

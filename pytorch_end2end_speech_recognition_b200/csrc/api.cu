@@ -20,6 +20,7 @@ constexpr int kStagingSlots = 4;
 constexpr int kGatherMinV = 129;  // V above this: the lattice reads gathered emission rows
 
 inline size_t align_up(size_t x) { return (x + kAlign - 1) / kAlign * kAlign; }
+inline bool valid_dtype(int d) { return d == B200CTC_FLOAT32 || d == B200CTC_BFLOAT16 || d == B200CTC_FLOAT16; }
 
 // The call's host-prepared tables (utterance metadata, launch order, flags, labels: ~160 KB for C3) are
 // written into a pinned staging slot and copied to a device slot of the handle on the handle's own COPY
@@ -32,6 +33,7 @@ struct WorkspaceLayout {
   size_t blob_bytes;   // meta + order + flags + labels
   size_t off_meta, off_order, off_flags, off_labels;
   size_t off_lse, off_xe_rows, off_xe_costs, off_symtab, off_nseg, off_em, off_scratch;
+  size_t off_staging;  // fp32 [T,B,V] gradient rows of a bfloat16 / float16 call (empty otherwise)
   size_t total;
 };
 
@@ -66,8 +68,9 @@ BatchTotals totals_from_bound(int T, int B, int max_label_len) {
 // `tables_in_workspace`: the device-resident call keeps meta/order/flags in the workspace (plan_kernel writes
 // them); the host call keeps them, with the labels, in the handle's staging slots.
 // Small vocabularies never run the lattice in gathered mode: the `em` region then holds the softmax rows of a
-// cost-only call (no gradient buffer to leave them in).
-WorkspaceLayout make_layout(const BatchTotals& t, int T, int B, int V, long long symtab_ints) {
+// cost-only call (no gradient buffer to leave them in).  `staged`: a bfloat16 / float16 call with a gradient, whose
+// kernels write fp32 rows into the staging region at the end; fp32 calls do not have it.
+WorkspaceLayout make_layout(const BatchTotals& t, int T, int B, int V, long long symtab_ints, bool staged = false) {
   WorkspaceLayout w;
   size_t off = 0;
   w.off_meta = off;   off += align_up((size_t)B * sizeof(UttMeta));
@@ -83,6 +86,7 @@ WorkspaceLayout make_layout(const BatchTotals& t, int T, int B, int V, long long
   const size_t em_floats = V >= kGatherMinV ? (size_t)t.em_floats : (size_t)T * B * V;
   w.off_em = off;     off += align_up(em_floats * sizeof(float));
   w.off_scratch = off; off += align_up((size_t)t.scratch_units * kGroupBytes);
+  w.off_staging = off; off += staged ? align_up((size_t)T * B * V * sizeof(float)) : 0;
   w.total = off;
   return w;
 }
@@ -140,8 +144,9 @@ int status_of(cudaError_t e) {
                                                                             : B200CTC_STATUS_EXECUTION_FAILED;
 }
 
-// K1 -> K2 (whose last CTA also writes loss_sum) on `stream`, bracketed by the profiling events.
-int run_kernels(b200ctc_handle* h, CallParams& p, int max_L, cudaStream_t stream) {
+// K1 -> K2 (whose last CTA also writes loss_sum) on `stream`, bracketed by the profiling events.  `narrow_to`: the
+// caller's gradient buffer of a bfloat16 / float16 call, into which the fp32 rows at p.grads are rounded last.
+int run_kernels(b200ctc_handle* h, CallParams& p, int max_L, cudaStream_t stream, void* narrow_to = nullptr) {
   h->last_flags = p.flags;
   h->last_B = p.B;
   LatticeCfg lattice;
@@ -154,6 +159,7 @@ int run_kernels(b200ctc_handle* h, CallParams& p, int max_L, cudaStream_t stream
   if (e == cudaSuccess) e = launch_lattice(p, lattice, stream);
   if (prof) cudaEventRecord(h->prof[2], stream);
   if (e == cudaSuccess && p.gathered && p.grads) e = launch_apply_occupancy(p, stream);
+  if (e == cudaSuccess && narrow_to) e = launch_narrow_grads(p.grads, narrow_to, (long long)p.T * p.B * p.V, p.acts_dtype, stream);
   if (prof) {
     cudaEventRecord(h->prof[3], stream);
     h->prof_valid = true;
@@ -161,7 +167,7 @@ int run_kernels(b200ctc_handle* h, CallParams& p, int max_L, cudaStream_t stream
   return status_of(e);
 }
 
-void fill_common(CallParams& p, const float* acts, int64_t as_t, int64_t as_b, float* grads, int T, int V, int B,
+void fill_common(CallParams& p, const void* acts, int64_t as_t, int64_t as_b, float* grads, int T, int V, int B,
                  int blank, float* costs, float* loss_sum, unsigned char* ws, const WorkspaceLayout& lay,
                  const b200ctc_options* o = nullptr, float* ls_costs = nullptr) {
   // fused call-site arithmetic (include/b200ctc.h, b200ctc_options); the defaults leave every result bit-identical
@@ -197,6 +203,7 @@ void fill_common(CallParams& p, const float* acts, int64_t as_t, int64_t as_b, f
   p.dev_act_lens = nullptr;
   p.label_stride = 0;
   p.max_label_len = 0;
+  p.acts_dtype = B200CTC_FLOAT32;
 }
 
 }  // namespace
@@ -260,8 +267,13 @@ int b200ctc_get_workspace_size(const int* label_lens, const int* act_lens, int T
 }
 
 int b200ctc_get_workspace_bound(int T, int V, int B, int max_label_len, size_t* bytes) {
-  if (!bytes || T < 0 || V < 1 || B < 0 || max_label_len < 0) return B200CTC_STATUS_INVALID_VALUE;
-  *bytes = make_layout(totals_from_bound(T, B, max_label_len), T, B, V, (long long)B * max_label_len).total + kAlign;
+  return b200ctc_get_workspace_bound_typed(T, V, B, max_label_len, B200CTC_FLOAT32, 1, bytes);
+}
+
+int b200ctc_get_workspace_bound_typed(int T, int V, int B, int max_label_len, int dtype, int need_grad, size_t* bytes) {
+  if (!bytes || T < 0 || V < 1 || B < 0 || max_label_len < 0 || !valid_dtype(dtype)) return B200CTC_STATUS_INVALID_VALUE;
+  const bool staged = dtype != B200CTC_FLOAT32 && need_grad;
+  *bytes = make_layout(totals_from_bound(T, B, max_label_len), T, B, V, (long long)B * max_label_len, staged).total + kAlign;
   return B200CTC_STATUS_SUCCESS;
 }
 
@@ -432,7 +444,18 @@ int b200ctc_loss_and_grad_dev(b200ctc_handle* h, const float* acts, int64_t acts
                               int max_label_len, int blank, const b200ctc_options* opts, float* costs,
                               float* loss_sum, float* ls_costs, void* workspace, size_t workspace_bytes,
                               void* stream_v) {
-  if (!h || T < 0 || V < 1 || B < 0 || blank < 0 || blank >= V || max_label_len < 0 || label_stride < max_label_len)
+  return b200ctc_loss_and_grad_dev_typed(h, acts, acts_stride_t, acts_stride_b, B200CTC_FLOAT32, grads, labels,
+                                         label_stride, label_lens, act_lens, T, V, B, max_label_len, blank, opts, costs,
+                                         loss_sum, ls_costs, workspace, workspace_bytes, stream_v);
+}
+
+int b200ctc_loss_and_grad_dev_typed(b200ctc_handle* h, const void* acts, int64_t acts_stride_t, int64_t acts_stride_b,
+                                    int acts_dtype, void* grads, const int* labels, int label_stride,
+                                    const int* label_lens, const int* act_lens, int T, int V, int B, int max_label_len,
+                                    int blank, const b200ctc_options* opts, float* costs, float* loss_sum,
+                                    float* ls_costs, void* workspace, size_t workspace_bytes, void* stream_v) {
+  if (!h || T < 0 || V < 1 || B < 0 || blank < 0 || blank >= V || max_label_len < 0 || label_stride < max_label_len ||
+      !valid_dtype(acts_dtype))
     return B200CTC_STATUS_INVALID_VALUE;
   if (opts && (!(opts->logit_scale > 0.f) || !(opts->label_smoothing >= 0.f) || !(opts->label_smoothing < 1.f) ||
                opts->grad_scale != opts->grad_scale || opts->loss_scale != opts->loss_scale))
@@ -450,14 +473,19 @@ int b200ctc_loss_and_grad_dev(b200ctc_handle* h, const float* acts, int64_t acts
     return B200CTC_STATUS_INVALID_VALUE;
   if ((long long)B * V * 4 > 0x7fffffffLL || (long long)B * label_stride > 0x7fffffffLL || B > 65536)
     return B200CTC_STATUS_UNSUPPORTED;
-  const WorkspaceLayout lay = make_layout(totals_from_bound(T, B, max_label_len), T, B, V, (long long)B * max_label_len);
+  const bool staged = acts_dtype != B200CTC_FLOAT32 && grads;
+  const WorkspaceLayout lay =
+      make_layout(totals_from_bound(T, B, max_label_len), T, B, V, (long long)B * max_label_len, staged);
   unsigned char* ws = reinterpret_cast<unsigned char*>(
       (reinterpret_cast<uintptr_t>(workspace) + kAlign - 1) / kAlign * kAlign);
   const size_t lost = (size_t)(ws - reinterpret_cast<unsigned char*>(workspace));
   if (workspace_bytes < lay.total + lost) return B200CTC_STATUS_WORKSPACE_TOO_SMALL;
 
   CallParams p;
-  fill_common(p, acts, acts_stride_t, acts_stride_b, grads, T, V, B, blank, costs, loss_sum, ws, lay, opts, ls_costs);
+  // a bfloat16 / float16 gradient is formed in fp32 in the staging region and rounded into `grads` by the last kernel
+  float* rows = staged ? reinterpret_cast<float*>(ws + lay.off_staging) : static_cast<float*>(grads);
+  fill_common(p, acts, acts_stride_t, acts_stride_b, rows, T, V, B, blank, costs, loss_sum, ws, lay, opts, ls_costs);
+  p.acts_dtype = acts_dtype;
   UttMeta* meta = reinterpret_cast<UttMeta*>(ws + lay.off_meta);
   int* order = reinterpret_cast<int*>(ws + lay.off_order);
   int* flags = reinterpret_cast<int*>(ws + lay.off_flags);
@@ -474,7 +502,17 @@ int b200ctc_loss_and_grad_dev(b200ctc_handle* h, const float* acts, int64_t acts
   // everything below is kernel launches on `stream`: the call can be captured into a CUDA graph
   cudaError_t e = launch_plan(p, meta, order, flags, stream);
   if (e != cudaSuccess) return status_of(e);
-  return run_kernels(h, p, max_label_len, stream);
+  return run_kernels(h, p, max_label_len, stream, staged ? grads : nullptr);
+}
+
+int b200ctc_scale_grads(const void* grads, void* out, int dtype, int T, int B, int V, const float* scale, int n_scale,
+                        void* stream_v) {
+  if (T < 0 || B < 0 || V < 1 || (dtype != B200CTC_BFLOAT16 && dtype != B200CTC_FLOAT16) ||
+      (n_scale != 1 && n_scale != B))
+    return B200CTC_STATUS_INVALID_VALUE;
+  if ((long long)T * B == 0) return B200CTC_STATUS_SUCCESS;
+  if (!grads || !out || !scale) return B200CTC_STATUS_INVALID_VALUE;
+  return status_of(launch_scale_grads(grads, out, dtype, T, B, V, scale, n_scale, reinterpret_cast<cudaStream_t>(stream_v)));
 }
 
 int b200ctc_set_profiling(b200ctc_handle* h, int enable) {

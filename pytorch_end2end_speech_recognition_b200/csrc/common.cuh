@@ -1,6 +1,8 @@
 // Shared definitions for the B200 CTC engine (internal; the public boundary is include/b200ctc.h).
 #pragma once
 
+#include <cuda_bf16.h>
+#include <cuda_fp16.h>
 #include <cuda_runtime.h>
 #include <stdint.h>
 
@@ -28,9 +30,10 @@ struct UttMeta {
 
 // Device views of one call, shared by all kernels.
 struct CallParams {
-  const float* acts;      // [T,B,V] logits, element (t,b,v) at acts[t*as_t + b*as_b + v]
+  const void* acts;       // [T,B,V] logits of type acts_dtype, element (t,b,v) at acts[t*as_t + b*as_b + v]
   long long as_t, as_b;
-  float* grads;           // [T,B,V] contiguous or nullptr (cost only)
+  float* grads;           // [T,B,V] contiguous fp32 or nullptr (cost only): the caller's buffer, or the staging region of a
+                          // bfloat16 / float16 call, which launch_narrow_grads rounds into the caller's buffer
   float* yrows;           // [T,B,V] where K1 leaves the softmax rows: == grads, or a workspace buffer in a cost-only call
   int T, B, V, blank;
   const UttMeta* meta;    // [B]
@@ -44,6 +47,7 @@ struct CallParams {
   float* costs;           // [B]
   float* loss_sum;        // [1] or nullptr
   int gathered;           // 1: lattice reads emissions from `em`, 0: from the softmax rows in `yrows`
+  int acts_dtype;         // b200ctc_dtype_t of acts (fills what was padding: the offsets of the other fields stay)
   // Gathered mode leaves the per-symbol occupancy of frame t in the emission row em[t] it no longer needs
   // ([0] blank, [1 + u] distinct symbol u) instead of one RED per (frame, symbol) into gradient rows that have
   // long left the L2; apply_occupancy_kernel subtracts them afterwards, all frames in parallel.
@@ -103,6 +107,11 @@ cudaError_t launch_softmax_rows(const CallParams& p, cudaStream_t stream);
 cudaError_t prepare_lattice(CallParams& p, int max_L, LatticeCfg* cfg);   // also fills fast_l_cap and oth_depth; error when not even the safe lattice fits
 cudaError_t launch_lattice(const CallParams& p, const LatticeCfg& cfg, cudaStream_t stream);
 cudaError_t launch_apply_occupancy(const CallParams& p, cudaStream_t stream);
+// dst[i] = src[i] rounded to nearest even in `dtype` (B200CTC_BFLOAT16 / B200CTC_FLOAT16), i < n
+cudaError_t launch_narrow_grads(const float* src, void* dst, long long n, int dtype, cudaStream_t stream);
+// out = grads * scale[0] (n_scale == 1) or grads[t,b,:] * scale[b] (n_scale == B), in fp32, rounded once to `dtype`
+cudaError_t launch_scale_grads(const void* grads, void* out, int dtype, int T, int B, int V, const float* scale,
+                               int n_scale, cudaStream_t stream);
 cudaError_t launch_plan(const CallParams& p, UttMeta* meta, int* order, int* flags, cudaStream_t stream);
 size_t edit_distance_workspace_bytes(int B, int max_ref, int max_hyp);
 cudaError_t launch_edit_distance(const int* refs, int ref_stride, const int* ref_lens, const int* hyps, int hyp_stride,
@@ -136,6 +145,21 @@ __device__ __forceinline__ float warp_sum(float v) {
   for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
   return v;
 }
+// Logit element types: every kernel widens a logit to fp32 when it loads it and computes in fp32 from there on.
+__device__ __forceinline__ float widen(float x) { return x; }
+__device__ __forceinline__ float widen(__nv_bfloat16 x) { return __bfloat162float(x); }
+__device__ __forceinline__ float widen(__half x) { return __half2float(x); }
+__device__ __forceinline__ float2 widen2(__nv_bfloat162 x) { return __bfloat1622float2(x); }
+__device__ __forceinline__ float2 widen2(__half2 x) { return __half22float2(x); }
+
+// Logit (t,b,v) of any element type, for code that is not specialised on it (the safe lattice); `i` is the element
+// offset t*as_t + b*as_b + v.
+__device__ __forceinline__ float load_act(const CallParams& p, long long i) {
+  if (p.acts_dtype == B200CTC_BFLOAT16) return widen(static_cast<const __nv_bfloat16*>(p.acts)[i]);
+  if (p.acts_dtype == B200CTC_FLOAT16) return widen(static_cast<const __half*>(p.acts)[i]);
+  return static_cast<const float*>(p.acts)[i];
+}
+
 __device__ __forceinline__ double warp_sum(double v) {
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);

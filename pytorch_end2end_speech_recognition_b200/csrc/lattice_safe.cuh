@@ -6,7 +6,8 @@
 // lattice window.  It follows SURVEY Appendix A literally: alpha over all frames (stored to the
 // scratch as doubles), log-likelihood from the last frame, then beta fused with the occupancy
 // update of the gradient rows.  Emissions are log-probabilities acts[t,b,k] - lse[t,b] with the
-// row log-sum-exp from K1, evaluated in double.
+// row log-sum-exp from K1, evaluated in double.  Logits of every element type are read through load_act
+// (common.cuh), which widens them to fp32 as K1 does.
 #pragma once
 
 #include "lattice_common.cuh"
@@ -67,7 +68,7 @@ __device__ void lattice_safe_utterance(const CallParams& p, int b, unsigned char
   __syncthreads();
   build_symbol_index(sm.lab, L, V, sm.ix);
 
-  const float* acts_b = p.acts + (long long)b * p.as_b;
+  const long long acts_b = (long long)b * p.as_b;   // element offset of the utterance's logits
   double* alpha = reinterpret_cast<double*>(p.scratch + m.scratch_off * kGroupBytes);
   const long long frame_stride = 4LL * m.J;  // doubles per frame in the scratch
 
@@ -77,10 +78,10 @@ __device__ void lattice_safe_utterance(const CallParams& p, int b, unsigned char
   const float ls = p.logit_scale;
   if ((rows_dirty || (p.rescale && !p.gathered)) && p.grads) {
     for (int t = 0; t < T; ++t) {
-      const float* arow = acts_b + (long long)t * p.as_t;
+      const long long arow = acts_b + (long long)t * p.as_t;
       float* grow = p.grads + ((long long)t * p.B + b) * V;
       const float lse = p.lse[(long long)t * p.B + b];
-      for (int v = tid; v < V; v += nt) grow[v] = fmaf(p.s_y, expf(arow[v] * ls - lse), -p.c_ls);
+      for (int v = tid; v < V; v += nt) grow[v] = fmaf(p.s_y, expf(load_act(p, arow + v) * ls - lse), -p.c_ls);
     }
     __threadfence();
     __syncthreads();
@@ -92,7 +93,7 @@ __device__ void lattice_safe_utterance(const CallParams& p, int b, unsigned char
   for (int s = tid; s < S; s += nt) prev[s] = (s == 0) ? 0.0 : -INFINITY;  // virtual frame -1
   __syncthreads();
   for (int t = 0; t < T; ++t) {
-    const float* arow = acts_b + (long long)t * p.as_t;
+    const long long arow = acts_b + (long long)t * p.as_t;
     const double lse = (double)p.lse[(long long)t * p.B + b];
     for (int s = tid; s < S; s += nt) {
       const int sym = (s & 1) ? sm.lab[s >> 1] : blank;
@@ -100,7 +101,7 @@ __device__ void lattice_safe_utterance(const CallParams& p, int b, unsigned char
       const double x0 = prev[s];
       const double x1 = (s >= 1) ? prev[s - 1] : -INFINITY;
       const double x2 = skip ? prev[s - 2] : -INFINITY;
-      const double v = log_sum_exp3(x0, x1, x2) + ((double)(arow[sym] * ls) - lse);
+      const double v = log_sum_exp3(x0, x1, x2) + ((double)(load_act(p, arow + sym) * ls) - lse);
       cur[s] = v;
       alpha[t * frame_stride + s] = v;
     }
@@ -132,7 +133,7 @@ __device__ void lattice_safe_utterance(const CallParams& p, int b, unsigned char
   const int n_seg = *sm.ix.n_seg;
   const int warp = tid >> 5, lane = tid & 31, n_warps = nt >> 5;
   for (int t = T - 1; t >= 0; --t) {
-    const float* arow = acts_b + (long long)t * p.as_t;
+    const long long arow = acts_b + (long long)t * p.as_t;
     const double lse = (double)p.lse[(long long)t * p.B + b];
     for (int s = tid; s < S; s += nt) {
       const int sym = (s & 1) ? sm.lab[s >> 1] : blank;
@@ -140,7 +141,7 @@ __device__ void lattice_safe_utterance(const CallParams& p, int b, unsigned char
       const double x0 = prev[s];
       const double x1 = (s + 1 < S) ? prev[s + 1] : -INFINITY;
       const double x2 = skip ? prev[s + 2] : -INFINITY;
-      const double lp = (double)(arow[sym] * ls) - lse;
+      const double lp = (double)(load_act(p, arow + sym) * ls) - lse;
       const double v = log_sum_exp3(x0, x1, x2) + lp;
       cur[s] = v;
       const double q = alpha[t * frame_stride + s] + v - lp - ll;

@@ -45,11 +45,24 @@ at::Tensor workspace_of(int device, void* stream, size_t bytes) {
   return it->second;
 }
 
-void check_acts(const at::Tensor& acts) {
+// `reduced`: the device-label call also takes bfloat16 and float16 logits; the host-label (warp-ctc) call is fp32 only
+void check_acts(const at::Tensor& acts, bool reduced) {
   TORCH_CHECK(acts.is_cuda(), "acts must be a CUDA tensor: this engine has no CPU path");
-  TORCH_CHECK(acts.scalar_type() == at::kFloat, "acts must be float32");
+  const auto t = acts.scalar_type();
+  TORCH_CHECK(t == at::kFloat || (reduced && (t == at::kBFloat16 || t == at::kHalf)),
+              reduced ? "acts must be float32, bfloat16 or float16" : "acts must be float32");
   TORCH_CHECK(acts.dim() == 3, "acts must be [T, B, V]");
 }
+
+int dtype_of(const at::Tensor& acts) {
+  switch (acts.scalar_type()) {
+    case at::kBFloat16: return B200CTC_BFLOAT16;
+    case at::kHalf: return B200CTC_FLOAT16;
+    default: return B200CTC_FLOAT32;
+  }
+}
+
+// The gradient has the logits' element type; costs and the loss sum are fp32 whatever it is.
 
 std::tuple<at::Tensor, at::Tensor, at::Tensor> outputs(const at::Tensor& acts, const c10::optional<at::Tensor>& grads,
                                                        bool need_grad, const c10::optional<at::Tensor>& costs,
@@ -59,26 +72,27 @@ std::tuple<at::Tensor, at::Tensor, at::Tensor> outputs(const at::Tensor& acts, c
   if (need_grad) {
     if (grads.has_value()) {
       g = *grads;
-      TORCH_CHECK(g.is_cuda() && g.scalar_type() == at::kFloat && g.is_contiguous() && g.sizes() == acts.sizes(),
-                  "grads must be a contiguous CUDA float32 tensor shaped like acts");
+      TORCH_CHECK(g.is_cuda() && g.scalar_type() == acts.scalar_type() && g.is_contiguous() && g.sizes() == acts.sizes(),
+                  "grads must be a contiguous CUDA tensor shaped like acts, of its dtype");
     } else {
       g = at::empty({T, B, V}, acts.options().memory_format(at::MemoryFormat::Contiguous));
     }
   }
-  at::Tensor c = costs.has_value() ? *costs : at::empty({B}, acts.options());
-  at::Tensor l = loss_sum.has_value() ? *loss_sum : at::empty({1}, acts.options());
+  at::Tensor c = costs.has_value() ? *costs : at::empty({B}, acts.options().dtype(at::kFloat));
+  at::Tensor l = loss_sum.has_value() ? *loss_sum : at::empty({1}, acts.options().dtype(at::kFloat));
   return {c, l, g};
 }
 
 }  // namespace
 
-// Device-resident labels / lengths (b200ctc_loss_and_grad_dev): kernel launches only, CUDA-graph capturable.
+// Device-resident labels / lengths (b200ctc_loss_and_grad_dev_typed): kernel launches only, CUDA-graph capturable.
+// fp32, bfloat16 or float16 logits; the gradient is returned in their dtype.
 std::tuple<at::Tensor, at::Tensor, c10::optional<at::Tensor>> loss_and_grad_dev(
     at::Tensor acts, at::Tensor labels, at::Tensor act_lens, at::Tensor label_lens, int64_t blank,
     c10::optional<at::Tensor> grads, bool need_grad, c10::optional<at::Tensor> costs, c10::optional<at::Tensor> loss_sum,
     int64_t max_label_len, double logit_scale, double label_smoothing, double loss_scale, double grad_scale,
     c10::optional<at::Tensor> ls_costs) {
-  check_acts(acts);
+  check_acts(acts, true);
   if (acts.stride(2) != 1 && acts.size(2) > 1) acts = acts.contiguous();
   const int T = (int)acts.size(0), B = (int)acts.size(1), V = (int)acts.size(2);
   TORCH_CHECK(labels.is_cuda() && labels.dim() == 2 && labels.size(0) == B, "labels must be a padded CUDA [B, Lmax] tensor");
@@ -94,18 +108,20 @@ std::tuple<at::Tensor, at::Tensor, c10::optional<at::Tensor>> loss_and_grad_dev(
   auto [c, l, g] = outputs(acts, grads, need_grad, costs, loss_sum);
   cudaStream_t stream = at::cuda::getCurrentCUDAStream(device).stream();
   size_t bytes = 0;
-  check(b200ctc_get_workspace_bound(T, V, B, Lmax, &bytes), "b200ctc_get_workspace_bound");
+  const int dtype = dtype_of(acts);
+  check(b200ctc_get_workspace_bound_typed(T, V, B, Lmax, dtype, need_grad ? 1 : 0, &bytes),
+        "b200ctc_get_workspace_bound_typed");
   at::Tensor ws = workspace_of(device, (void*)stream, bytes);
   b200ctc_options o{(float)logit_scale, (float)label_smoothing, (float)loss_scale, (float)grad_scale};
   const bool plain = logit_scale == 1.0 && label_smoothing == 0.0 && loss_scale == 1.0 && grad_scale == 1.0;
-  check(b200ctc_loss_and_grad_dev(handle_of(device), acts.data_ptr<float>(), acts.stride(0), acts.stride(1),
-                                  need_grad ? g.data_ptr<float>() : nullptr, labels.data_ptr<int>(),
+  check(b200ctc_loss_and_grad_dev_typed(handle_of(device), acts.data_ptr(), acts.stride(0), acts.stride(1), dtype,
+                                  need_grad ? g.data_ptr() : nullptr, labels.data_ptr<int>(),
                                   (B > 0 && labels.size(1) > 0) ? (int)labels.stride(0) : Lmax,
                                   label_lens.data_ptr<int>(), act_lens.data_ptr<int>(), T, V, B, Lmax, (int)blank,
                                   plain ? nullptr : &o, c.data_ptr<float>(), l.data_ptr<float>(),
                                   ls_costs.has_value() ? ls_costs->data_ptr<float>() : nullptr, ws.data_ptr(),
                                   (size_t)ws.numel(), (void*)stream),
-        "b200ctc_loss_and_grad_dev");
+        "b200ctc_loss_and_grad_dev_typed");
   return {c, l, need_grad ? c10::optional<at::Tensor>(g) : c10::nullopt};
 }
 
@@ -113,7 +129,7 @@ std::tuple<at::Tensor, at::Tensor, c10::optional<at::Tensor>> loss_and_grad_dev(
 std::tuple<at::Tensor, at::Tensor, c10::optional<at::Tensor>> loss_and_grad_host(
     at::Tensor acts, at::Tensor labels, at::Tensor act_lens, at::Tensor label_lens, int64_t blank,
     c10::optional<at::Tensor> grads, bool need_grad, c10::optional<at::Tensor> costs, c10::optional<at::Tensor> loss_sum) {
-  check_acts(acts);
+  check_acts(acts, false);
   if (acts.stride(2) != 1 && acts.size(2) > 1) acts = acts.contiguous();
   const int T = (int)acts.size(0), B = (int)acts.size(1), V = (int)acts.size(2);
   auto host_i32 = [](at::Tensor x, const char* name) {
@@ -141,6 +157,25 @@ std::tuple<at::Tensor, at::Tensor, c10::optional<at::Tensor>> loss_and_grad_host
   return {c, l, need_grad ? c10::optional<at::Tensor>(g) : c10::nullopt};
 }
 
+// Backward of a loss on bfloat16 / float16 logits (b200ctc_scale_grads): grads * scale in fp32, rounded once; `scale`
+// holds one value or one per utterance.
+at::Tensor scale_grads(at::Tensor grads, at::Tensor scale) {
+  const auto t = grads.scalar_type();
+  TORCH_CHECK(grads.is_cuda() && (t == at::kBFloat16 || t == at::kHalf) && grads.is_contiguous() && grads.dim() == 3,
+              "grads must be a contiguous CUDA bfloat16 or float16 [T, B, V] tensor");
+  const int T = (int)grads.size(0), B = (int)grads.size(1), V = (int)grads.size(2);
+  scale = scale.to(at::kFloat).contiguous();
+  TORCH_CHECK(scale.is_cuda() && scale.get_device() == grads.get_device() && (scale.numel() == 1 || scale.numel() == B),
+              "scale must be a CUDA tensor on the gradient's device with one value or one per utterance");
+  c10::cuda::CUDAGuard guard(grads.device());
+  at::Tensor out = at::empty_like(grads);
+  cudaStream_t stream = at::cuda::getCurrentCUDAStream(grads.get_device()).stream();
+  check(b200ctc_scale_grads(grads.data_ptr(), out.data_ptr(), dtype_of(grads), T, B, V, scale.data_ptr<float>(),
+                            (int)scale.numel(), (void*)stream),
+        "b200ctc_scale_grads");
+  return out;
+}
+
 int64_t handle_address(int64_t device) { return (int64_t)(intptr_t)handle_of((int)device); }
 
 void release_workspaces() {
@@ -160,6 +195,8 @@ PYBIND11_MODULE(TORCH_EXTENSION_NAME, m) {
         py::arg("acts"), py::arg("labels"), py::arg("act_lens"), py::arg("label_lens"), py::arg("blank") = 0,
         py::arg("grads") = py::none(), py::arg("need_grad") = true, py::arg("costs") = py::none(),
         py::arg("loss_sum") = py::none());
+  m.def("scale_grads", &scale_grads, "grads * scale in fp32, rounded once to the bfloat16 / float16 gradient's dtype",
+        py::arg("grads"), py::arg("scale"));
   m.def("handle_address", &handle_address, "address of the device's b200ctc_handle (shared with the ctypes diagnostics)");
   m.def("release_workspaces", &release_workspaces);
 }

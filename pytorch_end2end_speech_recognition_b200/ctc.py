@@ -12,7 +12,8 @@ Surface kept (same names, argument order and meaning):
         is inherited from here.
   * ``CTCLoss(size_average=False, length_average=False, blank=0)``  nn.Module front end.
 Native additions: ``ctc_loss_and_grad`` (device-resident results, no host sync) and
-``ctc_loss`` (autograd, device scalar).
+``ctc_loss`` (autograd, device scalar).  With device-resident labels these, and ``ctc_loss_from_padded``, also take
+bfloat16 and float16 logits (``torch.autocast``): the gradient comes back in the logits' dtype, the costs in fp32.
 """
 
 import ctypes
@@ -136,12 +137,17 @@ def _i32_ptr(arr):
     return arr.ctypes.data_as(ctypes.POINTER(ctypes.c_int))
 
 
-def _require_cuda(acts):
+_REDUCED = (torch.bfloat16, torch.float16)
+
+
+def _require_cuda(acts, reduced=False):
+    """``reduced``: bfloat16 / float16 logits are accepted too (the device-resident loss)."""
     if not isinstance(acts, torch.Tensor) or not acts.is_cuda:
         raise B200CTCError("acts must be a CUDA tensor: this engine has no CPU path "
                            "(the CPU restatement lives in oracle/ for tests only)")
-    if acts.dtype != torch.float32:
-        raise B200CTCError("acts must be float32, got %s" % acts.dtype)
+    if acts.dtype != torch.float32 and not (reduced and acts.dtype in _REDUCED):
+        raise B200CTCError("acts must be %s, got %s" % ("float32, bfloat16 or float16" if reduced else "float32",
+                                                        acts.dtype))
     if acts.dim() != 3:
         raise B200CTCError("acts must be [T, B, V]")
 
@@ -164,13 +170,29 @@ def workspace_bound(T, V, B, max_label_len):
     return n.value
 
 
+def _scale_grads(grads, scale):
+    """``grads * scale`` for backward; ``scale`` is grad_output: a 0-dim tensor, or ``[B]`` (one per utterance).  A
+    bfloat16 / float16 gradient is multiplied in fp32 and rounded once, in one pass of b200ctc_scale_grads: a plain
+    ``grads * scale`` would round the fp32 ``scale`` to the gradient's dtype first (a GradScaler's 2^16 is inf in
+    float16)."""
+    if grads.dtype == torch.float32:
+        return grads * (scale.reshape(1, -1, 1) if scale.dim() else scale)
+    try:
+        return _ext().scale_grads(grads, scale)
+    except RuntimeError as exc:
+        raise B200CTCError(str(exc).split("\n")[0])
+
+
 def ctc_loss_and_grad(acts, labels, act_lens, label_lens, blank=0, grads=None, need_grad=True,
                       costs=None, loss_sum=None, max_label_len=None, logit_scale=1.0, label_smoothing=0.0,
                       loss_scale=1.0, grad_scale=1.0, ls_costs=None):
     """One fused cost-and-gradient evaluation on the current CUDA stream.
 
     acts [T,B,V] CUDA fp32 logits (any strides with a unit vocabulary stride, e.g. the
-    ``logits.transpose(0, 1)`` view the reference passes, ctc.py:319 -- no copy is made).
+    ``logits.transpose(0, 1)`` view the reference passes, ctc.py:319 -- no copy is made).  With device-resident
+    labels bfloat16 and float16 logits are accepted as well: they are widened to fp32 as they are loaded, the
+    gradient is formed in fp32 and rounded once into a tensor of their dtype, and the costs stay fp32.  The result
+    is the fp32 evaluation of ``acts.float()`` with its gradient cast by ``.to(acts.dtype)``.
     Two forms of labels / lengths:
       * host-resident (the warp-ctc contract, ctc.py:295-297,321): flat int32 ``labels`` and ``act_lens`` /
         ``label_lens`` as CPU tensors, numpy arrays or lists -- planned on the host, tables copied by the call;
@@ -183,7 +205,7 @@ def ctc_loss_and_grad(acts, labels, act_lens, label_lens, blank=0, grads=None, n
     (ctc.py:323,329-337), grads = grad_scale * d(loss_sum/loss_scale)/d(scaled logits).
     Returns device tensors ``(costs[B], loss_sum[1], grads[T,B,V] or None)``; nothing synchronises the host.
     """
-    _require_cuda(acts)
+    _require_cuda(acts, reduced=True)
     ext = _ext()
     try:
         if isinstance(labels, torch.Tensor) and labels.is_cuda:
@@ -194,6 +216,9 @@ def ctc_loss_and_grad(acts, labels, act_lens, label_lens, blank=0, grads=None, n
         if logit_scale != 1.0 or label_smoothing != 0.0 or loss_scale != 1.0 or grad_scale != 1.0:
             raise B200CTCError("logit_scale / label_smoothing / loss_scale / grad_scale need device-resident labels "
                                "(the warp-ctc style call has no such arguments); see ctc_loss_from_padded")
+        if acts.dtype != torch.float32:
+            raise B200CTCError("%s logits need device-resident labels (CUDA tensors); the warp-ctc style call with "
+                               "host labels takes float32 only" % acts.dtype)
         return ext.loss_and_grad_host(acts, _as_cpu_tensor(labels), _as_cpu_tensor(act_lens), _as_cpu_tensor(label_lens),
                                       int(blank), grads, bool(need_grad), costs, loss_sum)
     except B200CTCError:
@@ -296,16 +321,17 @@ class _CTCDevice(torch.autograd.Function):
     @staticmethod
     def backward(ctx, grad_output):
         if ctx.reduction == "none":
-            g = ctx.grads * grad_output.reshape(1, -1, 1)
+            g = _scale_grads(ctx.grads, grad_output.reshape(-1))
         elif ctx.reduction == "mean":
-            g = ctx.grads * (grad_output.reshape(-1)[0] / ctx.grads.size(1))
+            g = _scale_grads(ctx.grads, grad_output.reshape(-1)[0] / ctx.grads.size(1))
         else:
-            g = ctx.grads * grad_output.reshape(-1)[0]
+            g = _scale_grads(ctx.grads, grad_output.reshape(-1)[0])
         return g, None, None, None, None, None
 
 
 def ctc_loss(acts, labels, act_lens, label_lens, blank=0, reduction="sum"):
-    """Device-resident CTC loss: returns a CUDA tensor ([1] for 'sum'/'mean', [B] for 'none')."""
+    """Device-resident CTC loss: returns a CUDA tensor ([1] for 'sum'/'mean', [B] for 'none').  ``acts`` may be
+    fp32, bfloat16 or float16; the loss is fp32 and the gradient has the dtype of ``acts``."""
     if reduction not in ("sum", "mean", "none"):
         raise B200CTCError("reduction must be 'sum', 'mean' or 'none'")
     return _CTCDevice.apply(acts, labels, act_lens, label_lens, blank, reduction)
@@ -345,7 +371,7 @@ class _CTCFromPadded(torch.autograd.Function):
 
     @staticmethod
     def backward(ctx, grad_output):
-        g = ctx.grads * grad_output.reshape(-1)[0]        # [T, B, V]
+        g = _scale_grads(ctx.grads, grad_output.reshape(-1)[0])        # [T, B, V]
         return g.transpose(0, 1), None, None, None, None, None, None
 
 
@@ -373,11 +399,12 @@ def ctc_loss_from_padded(logits, ys, x_lens, y_lens, label_offset=1, logits_temp
     ``average=True`` its ``/ len(xs)`` (ctc.py:323), ``label_smoothing`` its ``ls_prob`` (ctc.py:329-337 with
     models/pytorch_v3/criterion.py:51-80): all three are evaluated inside the kernels, not as tensor passes.
     Returns a CUDA tensor ``[1]``:  ``(1-ls) * sum_b cost_b / B + ls/V * sum_b sum_{t<x_lens[b]} sum_k -lp[b,t,k] / B``
-    that back-propagates into ``logits``.
+    that back-propagates into ``logits``.  ``logits`` may be fp32, bfloat16 or float16 (the output of a projection
+    under ``torch.autocast``): the loss is fp32 and the gradient has the dtype of ``logits``.
     """
     if logits.dim() != 3:
         raise B200CTCError("logits must be [B, T, V]")
-    _require_cuda(logits)
+    _require_cuda(logits, reduced=True)
     dev = logits.device
     ys_d, y_lens_d = _dev_padded_labels(ys, y_lens, dev, label_offset)
     x_lens_d = (x_lens if isinstance(x_lens, torch.Tensor) else torch.as_tensor(np.asarray(x_lens))).to(
