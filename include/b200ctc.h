@@ -61,7 +61,8 @@ typedef enum {
 
 typedef struct b200ctc_handle b200ctc_handle;
 
-/* Element type of the logits (and of the gradient) of b200ctc_loss_and_grad_dev_typed. */
+/* Element type of the logits (and of the gradient) of b200ctc_loss_and_grad_dev_typed, and of the input of
+   b200ctc_greedy_decode_typed, b200ctc_beam_search_typed and b200ctc_softmax_temperature_typed. */
 typedef enum {
   B200CTC_FLOAT32 = 0,
   B200CTC_BFLOAT16 = 1,
@@ -228,6 +229,16 @@ B200CTC_API int b200ctc_greedy_decode(const float* logits, int64_t stride_b, int
                           int* out_tokens, int* out_lens, void* stream);
 
 /*
+ * b200ctc_greedy_decode for logits of element type `dtype` (b200ctc_dtype_t); the other parameters are the same and the
+ * outputs stay int32.  A bfloat16 / float16 call gives, bit for bit, what the fp32 call gives on the logits widened to
+ * fp32 (widening is exact and monotone: the same arg-max, ties and NaN included), and reads half the bytes.  With
+ * B200CTC_FLOAT32 this is exactly b200ctc_greedy_decode.  An unknown dtype returns B200CTC_STATUS_INVALID_VALUE.
+ */
+B200CTC_API int b200ctc_greedy_decode_typed(const void* logits, int dtype, int64_t stride_b, int64_t stride_t,
+                          const int* lens, int T, int V, int B, int blank,
+                          int* out_tokens, int* out_lens, void* stream);
+
+/*
  * Batched CTC prefix beam search without a language model; replaces the python loops of
  * models/pytorch_v3/ctc/decoders/beam_search_decoder.py:33-124 (called with beam_width 10 for every published
  * error rate and with beam_width 2 by every reference test).  One CTA per utterance; scores are accumulated in
@@ -244,6 +255,17 @@ B200CTC_API int b200ctc_greedy_decode(const float* logits, int64_t stride_b, int
  */
 B200CTC_API int b200ctc_beam_search_workspace(int B, int T, int V, int beam_width, size_t* bytes);
 B200CTC_API int b200ctc_beam_search(const float* log_probs, int64_t stride_b, int64_t stride_t,
+                        const int* lens, int T, int V, int B, int blank, int beam_width,
+                        int* out_tokens, int* out_lens, float* out_scores,
+                        void* workspace, size_t workspace_bytes, void* stream);
+/*
+ * b200ctc_beam_search for log-probabilities of element type `dtype` (b200ctc_dtype_t); the other parameters and the
+ * workspace size are the same, tokens and lengths stay int32 and scores fp32.  The arithmetic is float64 on the
+ * widened values, so a bfloat16 / float16 call gives, bit for bit, the tokens, lengths and scores of the fp32 call on
+ * the log-probabilities widened to fp32.  With B200CTC_FLOAT32 this is exactly b200ctc_beam_search.  An unknown dtype
+ * returns B200CTC_STATUS_INVALID_VALUE.
+ */
+B200CTC_API int b200ctc_beam_search_typed(const void* log_probs, int dtype, int64_t stride_b, int64_t stride_t,
                         const int* lens, int T, int V, int B, int blank, int beam_width,
                         int* out_tokens, int* out_lens, float* out_scores,
                         void* workspace, size_t workspace_bytes, void* stream);
@@ -274,6 +296,14 @@ B200CTC_API int b200ctc_edit_distance(const int* refs, int ref_stride, const int
  * logits[b*stride_b + t*stride_t + v]; probs: DEVICE fp32 [B,T,V] contiguous.
  */
 B200CTC_API int b200ctc_softmax_temperature(const float* logits, int64_t stride_b, int64_t stride_t,
+                                int T, int V, int B, float temperature, float* probs, void* stream);
+/*
+ * b200ctc_softmax_temperature for logits of element type `dtype` (b200ctc_dtype_t); `probs` stays fp32 [B,T,V] for
+ * every type.  A bfloat16 / float16 call gives, bit for bit, the probabilities of the fp32 call on the logits widened
+ * to fp32 (same element-to-lane assignment and summation order).  With B200CTC_FLOAT32 this is exactly
+ * b200ctc_softmax_temperature.  An unknown dtype returns B200CTC_STATUS_INVALID_VALUE.
+ */
+B200CTC_API int b200ctc_softmax_temperature_typed(const void* logits, int dtype, int64_t stride_b, int64_t stride_t,
                                 int T, int V, int B, float temperature, float* probs, void* stream);
 
 /*

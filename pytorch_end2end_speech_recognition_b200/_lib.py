@@ -31,11 +31,14 @@ EXPORTED_SYMBOLS = (
     "b200ctc_get_workspace_bound_typed",
     "b200ctc_scale_grads",
     "b200ctc_greedy_decode",
+    "b200ctc_greedy_decode_typed",
     "b200ctc_beam_search_workspace",
     "b200ctc_beam_search",
+    "b200ctc_beam_search_typed",
     "b200ctc_edit_distance_workspace",
     "b200ctc_edit_distance",
     "b200ctc_softmax_temperature",
+    "b200ctc_softmax_temperature_typed",
     "b200ctc_set_profiling",
     "b200ctc_get_last_kernel_ms",
     "b200ctc_get_last_fallbacks",
@@ -101,6 +104,11 @@ def declare(lib):
         ctypes.c_void_p, ctypes.c_int64, ctypes.c_int64, ctypes.c_void_p,
         ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_int,
         ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p]
+    lib.b200ctc_greedy_decode_typed.restype = ctypes.c_int
+    lib.b200ctc_greedy_decode_typed.argtypes = [
+        ctypes.c_void_p, ctypes.c_int, ctypes.c_int64, ctypes.c_int64, ctypes.c_void_p,
+        ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_int,
+        ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p]
     lib.b200ctc_beam_search_workspace.restype = ctypes.c_int
     lib.b200ctc_beam_search_workspace.argtypes = [ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_int,
                                                   ctypes.POINTER(ctypes.c_size_t)]
@@ -108,6 +116,11 @@ def declare(lib):
     lib.b200ctc_beam_search.argtypes = [
         ctypes.c_void_p, ctypes.c_int64, ctypes.c_int64, ctypes.c_void_p, ctypes.c_int, ctypes.c_int, ctypes.c_int,
         ctypes.c_int, ctypes.c_int, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p,
+        ctypes.c_size_t, ctypes.c_void_p]
+    lib.b200ctc_beam_search_typed.restype = ctypes.c_int
+    lib.b200ctc_beam_search_typed.argtypes = [
+        ctypes.c_void_p, ctypes.c_int, ctypes.c_int64, ctypes.c_int64, ctypes.c_void_p, ctypes.c_int, ctypes.c_int,
+        ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p,
         ctypes.c_size_t, ctypes.c_void_p]
     lib.b200ctc_edit_distance_workspace.restype = ctypes.c_int
     lib.b200ctc_edit_distance_workspace.argtypes = [ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.POINTER(ctypes.c_size_t)]
@@ -119,6 +132,10 @@ def declare(lib):
     lib.b200ctc_softmax_temperature.argtypes = [
         ctypes.c_void_p, ctypes.c_int64, ctypes.c_int64, ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_float,
         ctypes.c_void_p, ctypes.c_void_p]
+    lib.b200ctc_softmax_temperature_typed.restype = ctypes.c_int
+    lib.b200ctc_softmax_temperature_typed.argtypes = [
+        ctypes.c_void_p, ctypes.c_int, ctypes.c_int64, ctypes.c_int64, ctypes.c_int, ctypes.c_int, ctypes.c_int,
+        ctypes.c_float, ctypes.c_void_p, ctypes.c_void_p]
     lib.b200ctc_set_profiling.restype = ctypes.c_int
     lib.b200ctc_set_profiling.argtypes = [ctypes.c_void_p, ctypes.c_int]
     lib.b200ctc_get_last_kernel_ms.restype = ctypes.c_int

@@ -573,12 +573,19 @@ int b200ctc_beam_search_workspace(int B, int T, int V, int beam_width, size_t* b
 int b200ctc_beam_search(const float* log_probs, int64_t stride_b, int64_t stride_t, const int* lens, int T, int V,
                         int B, int blank, int beam_width, int* out_tokens, int* out_lens, float* out_scores,
                         void* workspace, size_t workspace_bytes, void* stream_v) {
-  if (T < 0 || V < 1 || B < 0 || blank < 0 || blank >= V || beam_width < 1 || beam_width > 64)
+  return b200ctc_beam_search_typed(log_probs, B200CTC_FLOAT32, stride_b, stride_t, lens, T, V, B, blank, beam_width,
+                                   out_tokens, out_lens, out_scores, workspace, workspace_bytes, stream_v);
+}
+
+int b200ctc_beam_search_typed(const void* log_probs, int dtype, int64_t stride_b, int64_t stride_t, const int* lens, int T,
+                              int V, int B, int blank, int beam_width, int* out_tokens, int* out_lens, float* out_scores,
+                              void* workspace, size_t workspace_bytes, void* stream_v) {
+  if (T < 0 || V < 1 || B < 0 || blank < 0 || blank >= V || beam_width < 1 || beam_width > 64 || !valid_dtype(dtype))
     return B200CTC_STATUS_INVALID_VALUE;
   if (B == 0) return B200CTC_STATUS_SUCCESS;
   if (!lens || !out_lens || !workspace || (T > 0 && (!log_probs || !out_tokens))) return B200CTC_STATUS_INVALID_VALUE;
   if (workspace_bytes < beam_search_workspace_bytes(B, T, V, beam_width)) return B200CTC_STATUS_WORKSPACE_TOO_SMALL;
-  return status_of(launch_beam_search(log_probs, stride_b, stride_t, lens, T, V, B, blank, beam_width, out_tokens,
+  return status_of(launch_beam_search(log_probs, dtype, stride_b, stride_t, lens, T, V, B, blank, beam_width, out_tokens,
                                       out_lens, out_scores, workspace, reinterpret_cast<cudaStream_t>(stream_v)));
 }
 
@@ -602,20 +609,32 @@ int b200ctc_edit_distance(const int* refs, int ref_stride, const int* ref_lens, 
 
 int b200ctc_softmax_temperature(const float* logits, int64_t stride_b, int64_t stride_t, int T, int V, int B,
                                 float temperature, float* probs, void* stream_v) {
-  if (T < 0 || V < 1 || B < 0 || !(temperature > 0.f)) return B200CTC_STATUS_INVALID_VALUE;
+  return b200ctc_softmax_temperature_typed(logits, B200CTC_FLOAT32, stride_b, stride_t, T, V, B, temperature, probs,
+                                           stream_v);
+}
+
+int b200ctc_softmax_temperature_typed(const void* logits, int dtype, int64_t stride_b, int64_t stride_t, int T, int V,
+                                      int B, float temperature, float* probs, void* stream_v) {
+  if (T < 0 || V < 1 || B < 0 || !(temperature > 0.f) || !valid_dtype(dtype)) return B200CTC_STATUS_INVALID_VALUE;
   if ((long long)B * T == 0) return B200CTC_STATUS_SUCCESS;
   if (!logits || !probs) return B200CTC_STATUS_INVALID_VALUE;
-  return status_of(launch_softmax_temperature(logits, stride_b, stride_t, T, V, B, 1.0f / temperature, probs,
+  return status_of(launch_softmax_temperature(logits, dtype, stride_b, stride_t, T, V, B, 1.0f / temperature, probs,
                                               reinterpret_cast<cudaStream_t>(stream_v)));
 }
 
 int b200ctc_greedy_decode(const float* logits, int64_t stride_b, int64_t stride_t, const int* lens,
                           int T, int V, int B, int blank, int* out_tokens, int* out_lens,
                           void* stream_v) {
-  if (T < 0 || V < 1 || B < 0) return B200CTC_STATUS_INVALID_VALUE;
+  return b200ctc_greedy_decode_typed(logits, B200CTC_FLOAT32, stride_b, stride_t, lens, T, V, B, blank, out_tokens,
+                                     out_lens, stream_v);
+}
+
+int b200ctc_greedy_decode_typed(const void* logits, int dtype, int64_t stride_b, int64_t stride_t, const int* lens, int T,
+                                int V, int B, int blank, int* out_tokens, int* out_lens, void* stream_v) {
+  if (T < 0 || V < 1 || B < 0 || !valid_dtype(dtype)) return B200CTC_STATUS_INVALID_VALUE;
   if (B == 0) return B200CTC_STATUS_SUCCESS;
   if (!lens || !out_lens || (T > 0 && (!logits || !out_tokens))) return B200CTC_STATUS_INVALID_VALUE;
-  return status_of(launch_greedy(logits, stride_b, stride_t, lens, T, V, B, blank, out_tokens, out_lens,
+  return status_of(launch_greedy(logits, dtype, stride_b, stride_t, lens, T, V, B, blank, out_tokens, out_lens,
                                  reinterpret_cast<cudaStream_t>(stream_v)));
 }
 

@@ -43,8 +43,11 @@ __device__ __forceinline__ bool better(const Best& a, const Best& b) {   // a be
   return a.seq < b.seq;
 }
 
+// E: the log-probabilities' type (float, __nv_bfloat16, __half).  A 16-bit value widens exactly to the float64 the
+// arithmetic uses, so the result is the fp32 kernel's on the widened values.
+template <typename E>
 __global__ void __launch_bounds__(kBeamThreads) beam_search_kernel(
-    const float* __restrict__ log_probs, long long stride_b, long long stride_t, const int* __restrict__ lens,
+    const E* __restrict__ log_probs, long long stride_b, long long stride_t, const int* __restrict__ lens,
     int T, int V, int blank, int beam_width, double* __restrict__ cand_all, int2* __restrict__ nodes_all,
     int* __restrict__ out_tokens, int* __restrict__ out_lens, float* __restrict__ out_scores) {
   __shared__ double s_pb[2][kMaxBeam], s_pnb[2][kMaxBeam];      // current / next beam
@@ -58,7 +61,7 @@ __global__ void __launch_bounds__(kBeamThreads) beam_search_kernel(
 
   const int b = blockIdx.x, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const int n_frames = min(max(lens[b], 0), T);
-  const float* lp_b = log_probs + (long long)b * stride_b;
+  const E* lp_b = log_probs + (long long)b * stride_b;
   double* cand = cand_all + (long long)b * kMaxBeam * V;
   int2* nodes = nodes_all + (long long)b * ((long long)T * beam_width + 1);
   int cur = 0, W = 1;
@@ -70,14 +73,14 @@ __global__ void __launch_bounds__(kBeamThreads) beam_search_kernel(
   __syncthreads();
 
   for (int t = 0; t < n_frames; ++t) {
-    const float* lp = lp_b + (long long)t * stride_t;
+    const E* lp = lp_b + (long long)t * stride_t;
     const int nxt = cur ^ 1;
     // ---- extension candidates (prefix i, symbol c != blank): beam_search_decoder.py:86-101 ----
     for (int k = tid; k < W * V; k += kBeamThreads) {
       const int i = k / V, c = k - i * V;
       double v = INFINITY;                              // +inf: not a candidate
       if (c != blank) {
-        const double p_t = (double)lp[c];
+        const double p_t = (double)widen(lp[c]);
         v = (c != s_last[cur][i]) ? logaddexp64(s_pb[cur][i] + p_t, s_pnb[cur][i] + p_t) : s_pb[cur][i] + p_t;
       }
       cand[k] = v;
@@ -94,7 +97,7 @@ __global__ void __launch_bounds__(kBeamThreads) beam_search_kernel(
     // ---- stay candidates: :75-81 (blank) and :105-109 (repeated last symbol), merged with the extension of the parent ----
     if (tid < W) {
       const int j = tid, e = s_last[cur][j];
-      const double p_blank = (double)lp[blank];
+      const double p_blank = (double)widen(lp[blank]);
       const double n_pb = logaddexp64(s_pb[cur][j] + p_blank, s_pnb[cur][j] + p_blank);
       double n_pnb = -INFINITY;
       long long seq = ((long long)blank * W + j) * 2;
@@ -106,7 +109,7 @@ __global__ void __launch_bounds__(kBeamThreads) beam_search_kernel(
           cand[pi * V + e] = INFINITY;                  // that extension IS this prefix
           seq = min(seq, ((long long)e * W + pi) * 2);
         }
-        n_pnb = logaddexp64(n_pnb, s_pnb[cur][j] + (double)lp[e]);
+        n_pnb = logaddexp64(n_pnb, s_pnb[cur][j] + (double)widen(lp[e]));
         seq = min(seq, ((long long)e * W + j) * 2 + 1);
       }
       s_stay_pb[j] = n_pb; s_stay_pnb[j] = n_pnb;
@@ -189,16 +192,27 @@ size_t beam_search_workspace_bytes(int B, int T, int V, int beam_width) {
   return (cand + 255) / 256 * 256 + nodes;
 }
 
-cudaError_t launch_beam_search(const float* log_probs, long long stride_b, long long stride_t, const int* lens, int T,
-                               int V, int B, int blank, int beam_width, int* out_tokens, int* out_lens,
+cudaError_t launch_beam_search(const void* log_probs, int dtype, long long stride_b, long long stride_t, const int* lens,
+                               int T, int V, int B, int blank, int beam_width, int* out_tokens, int* out_lens,
                                float* out_scores, void* workspace, cudaStream_t stream) {
   if (B == 0) return cudaSuccess;
   if (beam_width < 1 || beam_width > kMaxBeam) return cudaErrorInvalidValue;
   unsigned char* ws = reinterpret_cast<unsigned char*>(workspace);
   const size_t cand = ((size_t)B * kMaxBeam * (size_t)V * sizeof(double) + 255) / 256 * 256;
-  beam_search_kernel<<<B, kBeamThreads, 0, stream>>>(log_probs, stride_b, stride_t, lens, T, V, blank, beam_width,
-                                                     reinterpret_cast<double*>(ws), reinterpret_cast<int2*>(ws + cand),
-                                                     out_tokens, out_lens, out_scores);
+  double* cand_all = reinterpret_cast<double*>(ws);
+  int2* nodes_all = reinterpret_cast<int2*>(ws + cand);
+  if (dtype == B200CTC_BFLOAT16)
+    beam_search_kernel<<<B, kBeamThreads, 0, stream>>>(static_cast<const __nv_bfloat16*>(log_probs), stride_b, stride_t,
+                                                       lens, T, V, blank, beam_width, cand_all, nodes_all, out_tokens,
+                                                       out_lens, out_scores);
+  else if (dtype == B200CTC_FLOAT16)
+    beam_search_kernel<<<B, kBeamThreads, 0, stream>>>(static_cast<const __half*>(log_probs), stride_b, stride_t, lens, T,
+                                                       V, blank, beam_width, cand_all, nodes_all, out_tokens, out_lens,
+                                                       out_scores);
+  else
+    beam_search_kernel<<<B, kBeamThreads, 0, stream>>>(static_cast<const float*>(log_probs), stride_b, stride_t, lens, T,
+                                                       V, blank, beam_width, cand_all, nodes_all, out_tokens, out_lens,
+                                                       out_scores);
   return cudaGetLastError();
 }
 

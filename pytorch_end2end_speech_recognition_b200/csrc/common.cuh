@@ -117,15 +117,15 @@ size_t edit_distance_workspace_bytes(int B, int max_ref, int max_hyp);
 cudaError_t launch_edit_distance(const int* refs, int ref_stride, const int* ref_lens, const int* hyps, int hyp_stride,
                                  const int* hyp_lens, int B, int max_ref, int max_hyp, int* out4, void* workspace,
                                  cudaStream_t stream);
-cudaError_t launch_softmax_temperature(const float* logits, long long stride_b, long long stride_t, int T, int V, int B,
-                                       float inv_temperature, float* probs, cudaStream_t stream);
+// the decoders and the posterior softmax read logits / log-probabilities of element type `dtype` (b200ctc_dtype_t)
+cudaError_t launch_softmax_temperature(const void* logits, int dtype, long long stride_b, long long stride_t, int T, int V,
+                                       int B, float inv_temperature, float* probs, cudaStream_t stream);
 size_t beam_search_workspace_bytes(int B, int T, int V, int beam_width);
-cudaError_t launch_beam_search(const float* log_probs, long long stride_b, long long stride_t, const int* lens, int T,
-                               int V, int B, int blank, int beam_width, int* out_tokens, int* out_lens,
+cudaError_t launch_beam_search(const void* log_probs, int dtype, long long stride_b, long long stride_t, const int* lens,
+                               int T, int V, int B, int blank, int beam_width, int* out_tokens, int* out_lens,
                                float* out_scores, void* workspace, cudaStream_t stream);
-cudaError_t launch_greedy(const float* logits, long long stride_b, long long stride_t, const int* lens,
-                          int T, int V, int B, int blank, int* out_tokens, int* out_lens,
-                          cudaStream_t stream);
+cudaError_t launch_greedy(const void* logits, int dtype, long long stride_b, long long stride_t, const int* lens,
+                          int T, int V, int B, int blank, int* out_tokens, int* out_lens, cudaStream_t stream);
 
 // ---------------------------------------------------------------------------------------------
 // small device helpers

@@ -9,7 +9,7 @@
 //  * softmax_temperature_kernel -- the fused softmax(logits / temperature) of CTC.posteriors
 //    (models/pytorch_v3/ctc/ctc.py:455-502), one warp per row, online max / sum.
 //
-// Bound: HBM for the softmax (4V read + 4V written per row); the edit distance is a latency-bound dynamic
+// Bound: HBM for the softmax (4V read, or 2V for 16-bit logits, + 4V written per row: probs are fp32 for every type); the edit distance is a latency-bound dynamic
 // programme of (R + H) dependent steps per pair and is parallel over the mini-batch.
 #include "common.cuh"
 
@@ -76,18 +76,21 @@ __global__ void __launch_bounds__(kEdThreads) edit_distance_kernel(
   }
 }
 
-// one warp per row; V-strided online softmax (two reads of the row: the second one hits L1/L2)
+// one warp per row; V-strided online softmax (two reads of the row: the second one hits L1/L2).  E: the logits' type;
+// every type keeps the fp32 element-to-lane assignment and summation order, so a 16-bit row gives bit for bit what
+// the fp32 kernel gives on its widened values.
+template <typename E>
 __global__ void __launch_bounds__(256) softmax_temperature_kernel(
-    const float* __restrict__ logits, long long stride_b, long long stride_t, int T, int V, long long rows,
+    const E* __restrict__ logits, long long stride_b, long long stride_t, int T, int V, long long rows,
     float inv_temperature, float* __restrict__ probs) {
   const int lane = threadIdx.x & 31;
   const long long row = (long long)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
   if (row >= rows) return;
   const long long b = row / T, t = row - b * T;
-  const float* x = logits + b * stride_b + t * stride_t;
+  const E* x = logits + b * stride_b + t * stride_t;
   float m = -INFINITY, s = 0.f;
   for (int v = lane; v < V; v += 32) {
-    const float z = __ldg(x + v) * inv_temperature;
+    const float z = widen(__ldg(x + v)) * inv_temperature;
     const float nm = fmaxf(m, z);
     s = s * __expf(m - nm) + __expf(z - nm);
     m = nm;
@@ -96,7 +99,7 @@ __global__ void __launch_bounds__(256) softmax_temperature_kernel(
   s = warp_sum(s * __expf(m - gm));                    // lanes that saw nothing: m = -inf, s = 0 -> 0 * exp(-inf) = 0
   const float inv = 1.0f / s;
   float* y = probs + row * V;
-  for (int v = lane; v < V; v += 32) y[v] = __expf(__ldg(x + v) * inv_temperature - gm) * inv;
+  for (int v = lane; v < V; v += 32) y[v] = __expf(widen(__ldg(x + v)) * inv_temperature - gm) * inv;
 }
 
 }  // namespace
@@ -120,13 +123,21 @@ cudaError_t launch_edit_distance(const int* refs, int ref_stride, const int* ref
   return cudaGetLastError();
 }
 
-cudaError_t launch_softmax_temperature(const float* logits, long long stride_b, long long stride_t, int T, int V, int B,
-                                       float inv_temperature, float* probs, cudaStream_t stream) {
+cudaError_t launch_softmax_temperature(const void* logits, int dtype, long long stride_b, long long stride_t, int T, int V,
+                                       int B, float inv_temperature, float* probs, cudaStream_t stream) {
   const long long rows = (long long)B * T;
   if (rows == 0) return cudaSuccess;
   const long long grid = (rows + 7) / 8;
   if (grid > 0x7fffffffLL) return cudaErrorInvalidConfiguration;
-  softmax_temperature_kernel<<<(unsigned)grid, 256, 0, stream>>>(logits, stride_b, stride_t, T, V, rows, inv_temperature, probs);
+  if (dtype == B200CTC_BFLOAT16)
+    softmax_temperature_kernel<<<(unsigned)grid, 256, 0, stream>>>(static_cast<const __nv_bfloat16*>(logits), stride_b,
+                                                                   stride_t, T, V, rows, inv_temperature, probs);
+  else if (dtype == B200CTC_FLOAT16)
+    softmax_temperature_kernel<<<(unsigned)grid, 256, 0, stream>>>(static_cast<const __half*>(logits), stride_b, stride_t,
+                                                                   T, V, rows, inv_temperature, probs);
+  else
+    softmax_temperature_kernel<<<(unsigned)grid, 256, 0, stream>>>(static_cast<const float*>(logits), stride_b, stride_t,
+                                                                   T, V, rows, inv_temperature, probs);
   return cudaGetLastError();
 }
 

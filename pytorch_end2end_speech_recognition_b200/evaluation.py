@@ -16,7 +16,7 @@ import torch
 
 from . import _lib
 from ._lib import B200CTCError
-from .decode import beam_search_decode, greedy_decode
+from .decode import DTYPES, beam_search_decode, greedy_decode
 
 
 def _padded_i32(seqs, dev):
@@ -78,18 +78,20 @@ def compute_wer(ref, hyp, normalize=False, device="cuda"):
 
 def posteriors(logits, temperature=1.0):
     """``softmax(logits / temperature)`` over the last axis in one pass (CTC.posteriors, ctc.py:486).
-    logits: CUDA fp32 ``[B, T, V]`` (any batch / time strides).  Returns a CUDA fp32 tensor ``[B, T, V]``."""
-    if not isinstance(logits, torch.Tensor) or not logits.is_cuda or logits.dtype != torch.float32 or logits.dim() != 3:
-        raise B200CTCError("logits must be a CUDA float32 tensor [B, T, V]")
+    logits: CUDA fp32, bfloat16 or float16 ``[B, T, V]`` (any batch / time strides).  Returns a CUDA fp32 tensor
+    ``[B, T, V]`` for every input type (the reference hands it to numpy, which has no bfloat16): for 16-bit logits
+    exactly ``posteriors(logits.float(), temperature)``."""
+    if not isinstance(logits, torch.Tensor) or not logits.is_cuda or logits.dtype not in DTYPES or logits.dim() != 3:
+        raise B200CTCError("logits must be a CUDA float32, bfloat16 or float16 tensor [B, T, V]")
     if logits.stride(2) != 1 and logits.size(2) > 1:
         logits = logits.contiguous()
     B, T, V = logits.shape
     out = torch.empty((B, T, V), dtype=torch.float32, device=logits.device)
     with torch.cuda.device(logits.device):
-        st = _lib.load().b200ctc_softmax_temperature(logits.data_ptr(), logits.stride(0), logits.stride(1), T, V, B,
-                                                     float(temperature), out.data_ptr(),
-                                                     torch.cuda.current_stream(logits.device).cuda_stream)
-        _lib.check(st, "b200ctc_softmax_temperature")
+        st = _lib.load().b200ctc_softmax_temperature_typed(logits.data_ptr(), DTYPES[logits.dtype], logits.stride(0),
+                                                           logits.stride(1), T, V, B, float(temperature), out.data_ptr(),
+                                                           torch.cuda.current_stream(logits.device).cuda_stream)
+        _lib.check(st, "b200ctc_softmax_temperature_typed")
     return out
 
 
@@ -97,7 +99,8 @@ def evaluate_batch(logits, x_lens, ys, y_lens, blank=0, label_offset=1, beam_wid
     """Decode (greedy for ``beam_width == 1``, else prefix beam search on ``log_softmax(logits)``, the choice
     ``CTC.decode`` makes, ctc.py:435-441) + edit distance for a whole mini-batch, device resident.
 
-    logits ``[B, T, V]`` CUDA; ys ``[B, Lmax]`` reference labels WITHOUT the blank offset (as the dataset
+    logits ``[B, T, V]`` CUDA, fp32, bfloat16 or float16 (the beam search decodes fp32 log-probabilities of the
+    widened logits, as autocast's ``log_softmax`` gives them); ys ``[B, Lmax]`` reference labels WITHOUT the blank offset (as the dataset
     stores them), y_lens ``[B]``.  The hypotheses are shifted by ``-label_offset`` exactly as ``CTC.decode`` does
     (``best_hyps -= 1``, ctc.py:444).  Returns ``(errors[B,4] int32 CUDA, hyp_tokens[B,T], hyp_lens[B])`` with
     errors = (distance, sub, ins, del) per utterance; ``errors.sum(0)`` over a data set divided by
@@ -105,7 +108,8 @@ def evaluate_batch(logits, x_lens, ys, y_lens, blank=0, label_offset=1, beam_wid
     if int(beam_width) == 1:
         tokens, hyp_lens = greedy_decode(logits, x_lens, blank)
     else:
-        tokens, hyp_lens = beam_search_decode(torch.log_softmax(logits, dim=-1), x_lens, beam_width, blank)
+        tokens, hyp_lens = beam_search_decode(torch.log_softmax(logits, dim=-1, dtype=torch.float32), x_lens, beam_width,
+                                              blank)
     hyps = tokens - int(label_offset)                       # padding (-1) becomes more negative: never read
     dev = logits.device
     refs = torch.as_tensor(ys).to(device=dev, dtype=torch.int32)
