@@ -1,6 +1,7 @@
-"""Developer aid (GPU box): where does a step's time go?  Per-step device time of the host-label call, the
-device-resident call issued eagerly, and the device-resident call replayed from a CUDA graph, next to the
-kernel times the library measures with its own events.   python tools/step_probe.py C1 C3"""
+"""Developer aid (GPU box): where does a step's time go?  Per-step device time of the host-label call (with the
+same labels every step, and with two label sets in turn, as in training, where every mini-batch brings new
+transcripts), the device-resident call issued eagerly, and the device-resident call replayed from a CUDA graph,
+next to the kernel times the library measures with its own events.   python tools/step_probe.py C1 C3"""
 import os
 import sys
 import time
@@ -33,18 +34,26 @@ for key in (sys.argv[1:] or ["C1", "C3"]):
     r = bench.Runner(wl, dev, 1, 0)
     slot = r.loss_groups[0][0:1]
 
-    def host_path(n):
+    # every symbol moved to the next one: other labels with the same lengths and repeats
+    label_sets = (wl.labels, (wl.labels % (wl.V - 1) + 1).astype(np.int32))
+
+    def host_path(n, n_sets=1):
         for i in range(n):
-            b200.ctc_loss_and_grad(r.acts_dev[i % r.n_rot], wl.labels, wl.act_lens, wl.label_lens, grads=r.grads_dev[i % r.n_rot],
-                                   costs=r.costs, loss_sum=slot)
+            b200.ctc_loss_and_grad(r.acts_dev[i % r.n_rot], label_sets[i % n_sets], wl.act_lens, wl.label_lens,
+                                   grads=r.grads_dev[i % r.n_rot], costs=r.costs, loss_sum=slot)
+
+    def host_path_alternating(n):
+        host_path(n, 2)
 
     def dev_eager(n):
         for i in range(n):
             r.one(i % r.n_rot, slot)
 
-    for fn in (host_path, dev_eager):
+    for fn in (host_path, host_path_alternating, dev_eager):
         fn(8)
-    res = {"host-label call, eager": timed(host_path, 48), "device-resident call, eager": timed(dev_eager, 48),
+    res = {"host-label call, eager": timed(host_path, 48),
+           "host-label call, two label sets": timed(host_path_alternating, 48),
+           "device-resident call, eager": timed(dev_eager, 48),
            "device-resident call, graph of %d" % r.group: timed(lambda n: r.run(n), 48)}
     for grp in (8, 16):
         bench.GROUP = grp
