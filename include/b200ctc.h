@@ -271,6 +271,51 @@ B200CTC_API int b200ctc_beam_search_typed(const void* log_probs, int dtype, int6
                         void* workspace, size_t workspace_bytes, void* stream);
 
 /*
+ * Token-level back-off n-gram language model for shallow fusion in the prefix beam search (no counterpart in the
+ * reference, whose hook is a TODO: beam_search_decoder.py:103).
+ *
+ * b200ctc_ngram_lm_create reads an ARPA file of order 1..8 whose words are the decoder's symbols: symbols[c] is the
+ * string of decoder id c (symbols[blank] is not read).  A symbol that is not a unigram of the model maps to <unk>.
+ * B200CTC_STATUS_INVALID_VALUE, before any CUDA call (so on a machine without a GPU too), when the file cannot be read
+ * or is not well-formed ARPA (no \data\ header, a count that does not match its section, an order above 8, a malformed
+ * number, an n-gram listed twice or naming a word that is not a unigram, no \end\), when an n-gram's history (its first
+ * n-1 words) is not itself an n-gram (SRILM and KenLM output always satisfies this), when <s> or </s> is not a unigram,
+ * when two non-blank symbols are equal or one is <s> or </s>, or when a symbol is neither a unigram nor covered by a
+ * <unk> unigram.  Numbers are read with strtod (correctly rounded).  N-grams that contain a word no symbol maps to
+ * (other than <s>, </s> and <unk>) can never be queried and are dropped.  The model is copied to `device` once; nothing
+ * is allocated per decoding call.  The handle is read-only after create and may be used by concurrent calls.
+ * b200ctc_ngram_lm_info: the order and, for orders 1..8, the number of n-grams kept (counts[8]).
+ */
+typedef struct b200ctc_ngram_lm b200ctc_ngram_lm;
+B200CTC_API int b200ctc_ngram_lm_create(const char* arpa_path, const char* const* symbols, int V, int blank, int device,
+                                        b200ctc_ngram_lm** lm);
+B200CTC_API int b200ctc_ngram_lm_destroy(b200ctc_ngram_lm* lm);
+B200CTC_API int b200ctc_ngram_lm_info(const b200ctc_ngram_lm* lm, int* order, long long* counts);
+
+/*
+ * b200ctc_beam_search_typed with an n-gram language model fused in (shallow fusion).  With h the last min(N-1, len)
+ * words of <s> followed by the prefix (len: their number) and p / bo the log10 numbers of the file,
+ *   log10 P(c | h) = p(h c) if "h c" is an n-gram, else bo(h) + log10 P(c | h without its first word)   (bo = 0 when
+ *   h is not an n-gram);  lnP = log10 P * ln 10;
+ *   S(empty) = 0,  S(prefix + c) = S(prefix) + (alpha * lnP(c | prefix) + beta)
+ * every * and + rounded on its own in float64.  The CTC part (p_b, p_nb) of a prefix evolves as in
+ * b200ctc_beam_search; candidates are ranked by logaddexp(p_b, p_nb) + S with the same tie order, and prefixes are
+ * identified by their token sequence.  The hypothesis is the entry of the last beam with the largest
+ * (logaddexp(p_b, p_nb) + S) + alpha * lnP(</s> | prefix), ties to the earlier entry; out_scores is that value in
+ * fp32.  With alpha = beta = 0 this is the search of b200ctc_beam_search.
+ *   lm          created for this V and blank on the current device (else B200CTC_STATUS_INVALID_VALUE)
+ *   alpha, beta finite (LM weight, insertion bonus; beta may be negative)
+ *   workspace   DEVICE, >= b200ctc_beam_search_lm_workspace(B, T, V, beam_width) bytes
+ * The other parameters are those of b200ctc_beam_search_typed.
+ */
+B200CTC_API int b200ctc_beam_search_lm_workspace(int B, int T, int V, int beam_width, size_t* bytes);
+B200CTC_API int b200ctc_beam_search_lm(const void* log_probs, int dtype, int64_t stride_b, int64_t stride_t,
+                        const int* lens, int T, int V, int B, int blank, int beam_width,
+                        const b200ctc_ngram_lm* lm, double alpha, double beta,
+                        int* out_tokens, int* out_lens, float* out_scores,
+                        void* workspace, size_t workspace_bytes, void* stream);
+
+/*
  * Batched edit distance with error counts; replaces the python loops of compute_wer
  * (utils/evaluation/edit_distance.py:53-126), which the metric code calls once per utterance
  * (examples/timit/s5/exp/metrics/phone.py:93-101 and its twins).

@@ -35,6 +35,11 @@ EXPORTED_SYMBOLS = (
     "b200ctc_beam_search_workspace",
     "b200ctc_beam_search",
     "b200ctc_beam_search_typed",
+    "b200ctc_ngram_lm_create",
+    "b200ctc_ngram_lm_destroy",
+    "b200ctc_ngram_lm_info",
+    "b200ctc_beam_search_lm_workspace",
+    "b200ctc_beam_search_lm",
     "b200ctc_edit_distance_workspace",
     "b200ctc_edit_distance",
     "b200ctc_softmax_temperature",
@@ -122,6 +127,22 @@ def declare(lib):
         ctypes.c_void_p, ctypes.c_int, ctypes.c_int64, ctypes.c_int64, ctypes.c_void_p, ctypes.c_int, ctypes.c_int,
         ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p,
         ctypes.c_size_t, ctypes.c_void_p]
+    lib.b200ctc_ngram_lm_create.restype = ctypes.c_int
+    lib.b200ctc_ngram_lm_create.argtypes = [ctypes.c_char_p, ctypes.POINTER(ctypes.c_char_p), ctypes.c_int, ctypes.c_int,
+                                            ctypes.c_int, ctypes.POINTER(ctypes.c_void_p)]
+    lib.b200ctc_ngram_lm_destroy.restype = ctypes.c_int
+    lib.b200ctc_ngram_lm_destroy.argtypes = [ctypes.c_void_p]
+    lib.b200ctc_ngram_lm_info.restype = ctypes.c_int
+    lib.b200ctc_ngram_lm_info.argtypes = [ctypes.c_void_p, ctypes.POINTER(ctypes.c_int), ctypes.POINTER(ctypes.c_longlong)]
+    lib.b200ctc_beam_search_lm_workspace.restype = ctypes.c_int
+    lib.b200ctc_beam_search_lm_workspace.argtypes = [ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_int,
+                                                     ctypes.POINTER(ctypes.c_size_t)]
+    lib.b200ctc_beam_search_lm.restype = ctypes.c_int
+    lib.b200ctc_beam_search_lm.argtypes = [
+        ctypes.c_void_p, ctypes.c_int, ctypes.c_int64, ctypes.c_int64, ctypes.c_void_p, ctypes.c_int, ctypes.c_int,
+        ctypes.c_int, ctypes.c_int, ctypes.c_int,                          # T, V, B, blank, beam_width
+        ctypes.c_void_p, ctypes.c_double, ctypes.c_double,                 # lm, alpha, beta
+        ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_size_t, ctypes.c_void_p]
     lib.b200ctc_edit_distance_workspace.restype = ctypes.c_int
     lib.b200ctc_edit_distance_workspace.argtypes = [ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.POINTER(ctypes.c_size_t)]
     lib.b200ctc_edit_distance.restype = ctypes.c_int

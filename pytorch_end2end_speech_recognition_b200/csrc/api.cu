@@ -2,6 +2,7 @@
 // warp-ctc style call with host-resident labels, by plan_kernel for the device-resident call),
 // workspace carving and kernel dispatch.  No exceptions leave this file.
 #include <algorithm>
+#include <cmath>
 #include <cstdio>
 #include <cstring>
 #include <mutex>
@@ -10,6 +11,7 @@
 #include <vector>
 
 #include "common.cuh"
+#include "ngram_lm.cuh"
 
 namespace b200ctc {
 
@@ -587,6 +589,30 @@ int b200ctc_beam_search_typed(const void* log_probs, int dtype, int64_t stride_b
   if (workspace_bytes < beam_search_workspace_bytes(B, T, V, beam_width)) return B200CTC_STATUS_WORKSPACE_TOO_SMALL;
   return status_of(launch_beam_search(log_probs, dtype, stride_b, stride_t, lens, T, V, B, blank, beam_width, out_tokens,
                                       out_lens, out_scores, workspace, reinterpret_cast<cudaStream_t>(stream_v)));
+}
+
+int b200ctc_beam_search_lm_workspace(int B, int T, int V, int beam_width, size_t* bytes) {
+  if (!bytes || B < 0 || T < 0 || V < 1 || beam_width < 1 || beam_width > 64) return B200CTC_STATUS_INVALID_VALUE;
+  *bytes = beam_search_lm_workspace_bytes(B, T, V, beam_width) + kAlign;
+  return B200CTC_STATUS_SUCCESS;
+}
+
+int b200ctc_beam_search_lm(const void* log_probs, int dtype, int64_t stride_b, int64_t stride_t, const int* lens, int T,
+                           int V, int B, int blank, int beam_width, const b200ctc_ngram_lm* lm, double alpha, double beta,
+                           int* out_tokens, int* out_lens, float* out_scores, void* workspace, size_t workspace_bytes,
+                           void* stream_v) {
+  if (T < 0 || V < 1 || B < 0 || blank < 0 || blank >= V || beam_width < 1 || beam_width > 64 || !valid_dtype(dtype) ||
+      !std::isfinite(alpha) || !std::isfinite(beta))
+    return B200CTC_STATUS_INVALID_VALUE;
+  const int st = ngram_lm_check(lm, V, blank);
+  if (st != B200CTC_STATUS_SUCCESS) return st;
+  if (B == 0) return B200CTC_STATUS_SUCCESS;
+  if (!lens || !out_lens || !workspace || (T > 0 && (!log_probs || !out_tokens))) return B200CTC_STATUS_INVALID_VALUE;
+  if ((long long)T * beam_width >= 0x3fffffffLL) return B200CTC_STATUS_UNSUPPORTED;   // trie node ids and hash slots
+  if (workspace_bytes < beam_search_lm_workspace_bytes(B, T, V, beam_width)) return B200CTC_STATUS_WORKSPACE_TOO_SMALL;
+  return status_of(launch_beam_search_lm(log_probs, dtype, stride_b, stride_t, lens, T, V, B, blank, beam_width,
+                                         ngram_lm_view(lm), alpha, beta, out_tokens, out_lens, out_scores, workspace,
+                                         reinterpret_cast<cudaStream_t>(stream_v)));
 }
 
 int b200ctc_edit_distance_workspace(int B, int max_ref, int max_hyp, size_t* bytes) {

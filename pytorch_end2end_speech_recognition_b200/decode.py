@@ -79,11 +79,17 @@ class GreedyDecoder(object):
         return out
 
 
-def beam_search_decode(log_probs, x_lens, beam_width, blank=0, return_scores=False):
-    """Batched CTC prefix beam search on the GPU (no language model).
+def beam_search_decode(log_probs, x_lens, beam_width, blank=0, return_scores=False, lm=None, alpha=0.0, beta=0.0):
+    """Batched CTC prefix beam search on the GPU.
     log_probs: CUDA fp32, bfloat16 or float16 [B,T,V] log-probabilities (any batch/time strides); x_lens [B].
     Returns device tensors (tokens[B,T] int32 padded with -1, lens[B] int32[, scores[B] fp32]); 16-bit inputs give
-    the result of ``beam_search_decode(log_probs.float(), ...)``."""
+    the result of ``beam_search_decode(log_probs.float(), ...)``.
+    lm: an ``NGramLM`` loaded for these V symbols and this blank on the device of ``log_probs``; candidates are then
+    ranked with the LM score ``S(prefix + c) = S(prefix) + alpha * ln P(c | prefix) + beta`` added, and the hypothesis
+    includes ``alpha * ln P(</s> | prefix)`` (shallow fusion; include/b200ctc.h, b200ctc_beam_search_lm), as does its
+    score.  Without an LM, alpha and beta must be 0."""
+    if lm is None and (float(alpha) != 0.0 or float(beta) != 0.0):
+        raise B200CTCError("alpha and beta weight a language model: pass lm=NGramLM(...)")
     if not isinstance(log_probs, torch.Tensor) or not log_probs.is_cuda:
         raise B200CTCError("log_probs must be a CUDA tensor: this decoder has no CPU path")
     if log_probs.dtype not in DTYPES or log_probs.dim() != 3:
@@ -106,26 +112,38 @@ def beam_search_decode(log_probs, x_lens, beam_width, blank=0, return_scores=Fal
         out_lens = torch.empty(B, dtype=torch.int32, device=dev)
         scores = torch.empty(B, dtype=torch.float32, device=dev)
         n = ctypes.c_size_t()
-        _lib.check(lib.b200ctc_beam_search_workspace(B, T, V, int(beam_width), ctypes.byref(n)), "b200ctc_beam_search_workspace")
-        ws = torch.empty(max(n.value, 1), dtype=torch.uint8, device=dev)
         stream = torch.cuda.current_stream(dev)
-        st = lib.b200ctc_beam_search_typed(log_probs.data_ptr(), DTYPES[log_probs.dtype], log_probs.stride(0),
-                                           log_probs.stride(1), lens.data_ptr(), T, V, B, int(blank), int(beam_width),
-                                           tokens.data_ptr(), out_lens.data_ptr(), scores.data_ptr(), ws.data_ptr(),
-                                           ws.numel(), stream.cuda_stream)
-        _lib.check(st, "b200ctc_beam_search_typed")
+        if lm is None:
+            _lib.check(lib.b200ctc_beam_search_workspace(B, T, V, int(beam_width), ctypes.byref(n)), "b200ctc_beam_search_workspace")
+            ws = torch.empty(max(n.value, 1), dtype=torch.uint8, device=dev)
+            st = lib.b200ctc_beam_search_typed(log_probs.data_ptr(), DTYPES[log_probs.dtype], log_probs.stride(0),
+                                               log_probs.stride(1), lens.data_ptr(), T, V, B, int(blank), int(beam_width),
+                                               tokens.data_ptr(), out_lens.data_ptr(), scores.data_ptr(), ws.data_ptr(),
+                                               ws.numel(), stream.cuda_stream)
+            _lib.check(st, "b200ctc_beam_search_typed")
+        else:
+            _lib.check(lib.b200ctc_beam_search_lm_workspace(B, T, V, int(beam_width), ctypes.byref(n)),
+                       "b200ctc_beam_search_lm_workspace")
+            ws = torch.empty(max(n.value, 1), dtype=torch.uint8, device=dev)
+            st = lib.b200ctc_beam_search_lm(log_probs.data_ptr(), DTYPES[log_probs.dtype], log_probs.stride(0),
+                                            log_probs.stride(1), lens.data_ptr(), T, V, B, int(blank), int(beam_width),
+                                            lm.handle, float(alpha), float(beta), tokens.data_ptr(), out_lens.data_ptr(),
+                                            scores.data_ptr(), ws.data_ptr(), ws.numel(), stream.cuda_stream)
+            _lib.check(st, "b200ctc_beam_search_lm")
         ws.record_stream(stream)
     return (tokens, out_lens, scores) if return_scores else (tokens, out_lens)
 
 
 class BeamSearchDecoder(object):
     """Drop-in for the reference's numpy ``BeamSearchDecoder`` (beam_search_decoder.py:22-124): same
-    constructor and call signature; ``alpha`` / ``beta`` (language-model weight, insertion bonus) are accepted
-    and, as in the reference (whose LM hook is a TODO, :103), unused."""
+    constructor and call signature.  Without ``lm``, ``alpha`` / ``beta`` (language-model weight, insertion bonus)
+    are accepted and, as in the reference (whose LM hook is a TODO, :103), unused; with an ``NGramLM`` they weight
+    it (``beam_search_decode(..., lm=lm, alpha=alpha, beta=beta)``)."""
 
-    def __init__(self, blank_index, space_index=-1):
+    def __init__(self, blank_index, space_index=-1, lm=None):
         self._blank = blank_index
         self._space = space_index
+        self._lm = lm
 
     def __call__(self, log_probs, x_lens, beam_width=1, alpha=0., beta=0., device=None):
         if isinstance(log_probs, np.ndarray):
@@ -135,7 +153,10 @@ class BeamSearchDecoder(object):
             lp = log_probs if log_probs.is_cuda else log_probs.to(device if device is not None else "cuda")
             if lp.dtype not in (torch.bfloat16, torch.float16):
                 lp = lp.float()
-        tokens, lens = beam_search_decode(lp, x_lens, beam_width, self._blank)
+        if self._lm is None:
+            tokens, lens = beam_search_decode(lp, x_lens, beam_width, self._blank)
+        else:
+            tokens, lens = beam_search_decode(lp, x_lens, beam_width, self._blank, lm=self._lm, alpha=alpha, beta=beta)
         tokens = tokens.cpu().numpy()
         lens = lens.cpu().numpy()
         hyps = [tokens[b, :lens[b]].astype(np.int64) for b in range(tokens.shape[0])]

@@ -95,7 +95,7 @@ def posteriors(logits, temperature=1.0):
     return out
 
 
-def evaluate_batch(logits, x_lens, ys, y_lens, blank=0, label_offset=1, beam_width=1):
+def evaluate_batch(logits, x_lens, ys, y_lens, blank=0, label_offset=1, beam_width=1, lm=None, alpha=0.0, beta=0.0):
     """Decode (greedy for ``beam_width == 1``, else prefix beam search on ``log_softmax(logits)``, the choice
     ``CTC.decode`` makes, ctc.py:435-441) + edit distance for a whole mini-batch, device resident.
 
@@ -104,8 +104,15 @@ def evaluate_batch(logits, x_lens, ys, y_lens, blank=0, label_offset=1, beam_wid
     stores them), y_lens ``[B]``.  The hypotheses are shifted by ``-label_offset`` exactly as ``CTC.decode`` does
     (``best_hyps -= 1``, ctc.py:444).  Returns ``(errors[B,4] int32 CUDA, hyp_tokens[B,T], hyp_lens[B])`` with
     errors = (distance, sub, ins, del) per utterance; ``errors.sum(0)`` over a data set divided by
-    ``y_lens.sum()`` gives PER / CER and its breakdown (phone.py:119-126)."""
-    if int(beam_width) == 1:
+    ``y_lens.sum()`` gives PER / CER and its breakdown (phone.py:119-126).
+    With ``lm`` (an ``NGramLM``) every beam width, 1 included, decodes with the LM-fused beam search weighted by
+    ``alpha`` and ``beta``; without one they must be 0."""
+    if lm is not None:
+        tokens, hyp_lens = beam_search_decode(torch.log_softmax(logits, dim=-1, dtype=torch.float32), x_lens, beam_width,
+                                              blank, lm=lm, alpha=alpha, beta=beta)
+    elif float(alpha) != 0.0 or float(beta) != 0.0:
+        raise B200CTCError("alpha and beta weight a language model: pass lm=NGramLM(...)")
+    elif int(beam_width) == 1:
         tokens, hyp_lens = greedy_decode(logits, x_lens, blank)
     else:
         tokens, hyp_lens = beam_search_decode(torch.log_softmax(logits, dim=-1, dtype=torch.float32), x_lens, beam_width,
