@@ -336,6 +336,32 @@ B200CTC_API int b200ctc_edit_distance(const int* refs, int ref_stride, const int
                           void* workspace, size_t workspace_bytes, void* stream);
 
 /*
+ * Word and space-free character error counts of character-level hypotheses, batched: the WER / CER of character
+ * models without a per-utterance host loop.
+ *
+ *   refs / hyps / ref_lens / hyp_lens / ref_stride / hyp_stride  as for b200ctc_edit_distance
+ *   space         the word-boundary id, in the id space of both sequences (any int; one that never occurs
+ *                 makes a non-empty sequence one word)
+ *   word4         DEVICE int32 [B,4]: b200ctc_edit_distance's (distance, sub, ins, del) over the words, where the
+ *                 words of a sequence are its maximal non-empty runs of non-`space` tokens (python's str.split()
+ *                 rule: leading, trailing and repeated spaces make no empty word) and two words are equal when
+ *                 they have the same tokens
+ *   char4         DEVICE int32 [B,4]: the same over both sequences with every `space` removed
+ *   ref_counts    DEVICE int32 [B,2]: number of reference words, number of non-space reference tokens
+ *                 (the WER / CER denominators)
+ *   workspace     DEVICE, >= b200ctc_word_errors_workspace(B, max_ref, max_hyp) bytes; its contents on entry do
+ *                 not matter
+ * max_ref <= 17000, as for b200ctc_edit_distance, and max_hyp <= 2^29 (else B200CTC_STATUS_UNSUPPORTED).  Kernel
+ * launches only (CUDA-graph capturable).
+ */
+B200CTC_API int b200ctc_word_errors_workspace(int B, int max_ref, int max_hyp, size_t* bytes);
+B200CTC_API int b200ctc_word_errors(const int* refs, int ref_stride, const int* ref_lens,
+                          const int* hyps, int hyp_stride, const int* hyp_lens,
+                          int B, int max_ref, int max_hyp, int space,
+                          int* word4, int* char4, int* ref_counts,
+                          void* workspace, size_t workspace_bytes, void* stream);
+
+/*
  * probs[b,t,:] = softmax(logits[b,t,:] / temperature): the tensor work of CTC.posteriors
  * (models/pytorch_v3/ctc/ctc.py:455-502) in one pass.  logits: DEVICE fp32, element (b,t,v) at
  * logits[b*stride_b + t*stride_t + v]; probs: DEVICE fp32 [B,T,V] contiguous.

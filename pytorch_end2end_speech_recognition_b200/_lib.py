@@ -42,6 +42,8 @@ EXPORTED_SYMBOLS = (
     "b200ctc_beam_search_lm",
     "b200ctc_edit_distance_workspace",
     "b200ctc_edit_distance",
+    "b200ctc_word_errors_workspace",
+    "b200ctc_word_errors",
     "b200ctc_softmax_temperature",
     "b200ctc_softmax_temperature_typed",
     "b200ctc_set_profiling",
@@ -149,6 +151,14 @@ def declare(lib):
     lib.b200ctc_edit_distance.argtypes = [
         ctypes.c_void_p, ctypes.c_int, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int, ctypes.c_void_p,
         ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_size_t, ctypes.c_void_p]
+    lib.b200ctc_word_errors_workspace.restype = ctypes.c_int
+    lib.b200ctc_word_errors_workspace.argtypes = [ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.POINTER(ctypes.c_size_t)]
+    lib.b200ctc_word_errors.restype = ctypes.c_int
+    lib.b200ctc_word_errors.argtypes = [
+        ctypes.c_void_p, ctypes.c_int, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int, ctypes.c_void_p,
+        ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_int,            # B, max_ref, max_hyp, space
+        ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p,                 # word4, char4, ref_counts
+        ctypes.c_void_p, ctypes.c_size_t, ctypes.c_void_p]
     lib.b200ctc_softmax_temperature.restype = ctypes.c_int
     lib.b200ctc_softmax_temperature.argtypes = [
         ctypes.c_void_p, ctypes.c_int64, ctypes.c_int64, ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_float,

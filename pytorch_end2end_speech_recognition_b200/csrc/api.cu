@@ -633,6 +633,35 @@ int b200ctc_edit_distance(const int* refs, int ref_stride, const int* ref_lens, 
                                         workspace, reinterpret_cast<cudaStream_t>(stream_v)));
 }
 
+// sizes up to 2^29 keep the word count and table size of word_errors_layout in int
+int b200ctc_word_errors_workspace(int B, int max_ref, int max_hyp, size_t* bytes) {
+  if (!bytes || B < 0 || max_ref < 0 || max_hyp < 0) return B200CTC_STATUS_INVALID_VALUE;
+  if (max_ref > (1 << 29) || max_hyp > (1 << 29)) return B200CTC_STATUS_UNSUPPORTED;
+  const size_t pair = word_errors_workspace_bytes(1, max_ref, max_hyp);
+  if (B > 0 && pair > (SIZE_MAX - kAlign) / (size_t)B) return B200CTC_STATUS_UNSUPPORTED;
+  *bytes = (size_t)B * pair + kAlign;
+  return B200CTC_STATUS_SUCCESS;
+}
+
+int b200ctc_word_errors(const int* refs, int ref_stride, const int* ref_lens, const int* hyps, int hyp_stride,
+                        const int* hyp_lens, int B, int max_ref, int max_hyp, int space, int* word4, int* char4,
+                        int* ref_counts, void* workspace, size_t workspace_bytes, void* stream_v) {
+  if (B < 0 || max_ref < 0 || max_hyp < 0 || ref_stride < max_ref || hyp_stride < max_hyp) return B200CTC_STATUS_INVALID_VALUE;
+  if (B == 0) return B200CTC_STATUS_SUCCESS;
+  if (!ref_lens || !hyp_lens || !word4 || !char4 || !ref_counts || !workspace || (max_ref > 0 && !refs) ||
+      (max_hyp > 0 && !hyps))
+    return B200CTC_STATUS_INVALID_VALUE;
+  size_t need = 0;
+  const int st = b200ctc_word_errors_workspace(B, max_ref, max_hyp, &need);
+  if (st != B200CTC_STATUS_SUCCESS) return st;
+  // the word hashes are 64-bit: the layout starts on a 16-byte boundary inside the kAlign slack of the query
+  unsigned char* ws = reinterpret_cast<unsigned char*>((reinterpret_cast<uintptr_t>(workspace) + 15) / 16 * 16);
+  const size_t lost = (size_t)(ws - reinterpret_cast<unsigned char*>(workspace));
+  if (workspace_bytes < need - kAlign + lost) return B200CTC_STATUS_WORKSPACE_TOO_SMALL;
+  return status_of(launch_word_errors(refs, ref_stride, ref_lens, hyps, hyp_stride, hyp_lens, B, max_ref, max_hyp, space,
+                                      word4, char4, ref_counts, ws, reinterpret_cast<cudaStream_t>(stream_v)));
+}
+
 int b200ctc_softmax_temperature(const float* logits, int64_t stride_b, int64_t stride_t, int T, int V, int B,
                                 float temperature, float* probs, void* stream_v) {
   return b200ctc_softmax_temperature_typed(logits, B200CTC_FLOAT32, stride_b, stride_t, T, V, B, temperature, probs,

@@ -117,6 +117,10 @@ size_t edit_distance_workspace_bytes(int B, int max_ref, int max_hyp);
 cudaError_t launch_edit_distance(const int* refs, int ref_stride, const int* ref_lens, const int* hyps, int hyp_stride,
                                  const int* hyp_lens, int B, int max_ref, int max_hyp, int* out4, void* workspace,
                                  cudaStream_t stream);
+size_t word_errors_workspace_bytes(int B, int max_ref, int max_hyp);
+cudaError_t launch_word_errors(const int* refs, int ref_stride, const int* ref_lens, const int* hyps, int hyp_stride,
+                               const int* hyp_lens, int B, int max_ref, int max_hyp, int space, int* word4, int* char4,
+                               int* ref_counts, void* workspace, cudaStream_t stream);
 // the decoders and the posterior softmax read logits / log-probabilities of element type `dtype` (b200ctc_dtype_t)
 cudaError_t launch_softmax_temperature(const void* logits, int dtype, long long stride_b, long long stride_t, int T, int V,
                                        int B, float inv_temperature, float* probs, cudaStream_t stream);

@@ -1,5 +1,6 @@
-"""Evaluation on the GPU (SURVEY 8(f) rank 4): batched edit distance with error counts, the fused
-posterior softmax, and one call that turns a mini-batch of logits into error counts.
+"""Evaluation on the GPU (SURVEY 8(f) rank 4): batched edit distance with error counts, word and space-free
+character error counts of character-level hypotheses, the fused posterior softmax, and one call that turns a
+mini-batch of logits into error counts.
 
 Mirrors of the reference (same names, argument meaning and results):
   * ``compute_wer(ref, hyp, normalize)``  -- utils/evaluation/edit_distance.py:53-126
@@ -62,6 +63,54 @@ def edit_distance(refs, ref_lens, hyps, hyp_lens):
     return out
 
 
+def _rows_i32(x, dev):
+    """``[B, L]`` -> (int32 tensor on ``dev`` with contiguous, non-overlapping rows, its row stride).  A row view of a
+    wider tensor is kept as it is."""
+    x = x.to(device=dev, dtype=torch.int32)
+    if (x.size(1) > 1 and x.stride(1) != 1) or (x.size(0) > 1 and x.stride(0) < x.size(1)):
+        x = x.contiguous()
+    return x, (x.stride(0) if x.size(0) > 1 else x.size(1))
+
+
+def word_errors(refs, ref_lens, hyps, hyp_lens, space):
+    """Word and space-free character error counts of character-level hypotheses for a whole batch, on the GPU.
+
+    refs ``[B, Rmax]`` / hyps ``[B, Hmax]`` CUDA int tensors of token ids (padded; any row stride), ref_lens /
+    hyp_lens ``[B]`` tensors or arrays; ``space`` is the word-boundary id in the same id space.  The words of a
+    sequence are its maximal runs of tokens other than ``space`` (``str.split()``: leading, trailing and repeated
+    spaces make no empty word).  Returns CUDA int32 tensors ``(word_errors[B,4], char_errors[B,4], ref_counts[B,2])``:
+    ``compute_wer`` over the words, ``compute_wer`` over both sequences with the spaces removed, and the number of
+    reference words and of non-space reference tokens.  WER = ``word_errors[:, 0].sum() / ref_counts[:, 0].sum()``,
+    CER = ``char_errors[:, 0].sum() / ref_counts[:, 1].sum()``.  No host synchronisation."""
+    if not (isinstance(refs, torch.Tensor) and refs.is_cuda and isinstance(hyps, torch.Tensor) and hyps.is_cuda):
+        raise B200CTCError("refs and hyps must be CUDA tensors: the evaluation kernels have no CPU path")
+    if refs.dim() != 2 or hyps.dim() != 2 or refs.size(0) != hyps.size(0):
+        raise B200CTCError("refs and hyps must be [B, Rmax] and [B, Hmax]")
+    if not -2 ** 31 <= int(space) < 2 ** 31:
+        raise B200CTCError("space must be an int32 token id")
+    dev = refs.device
+    (refs, ref_stride), (hyps, hyp_stride) = _rows_i32(refs, dev), _rows_i32(hyps, dev)
+    ref_lens = torch.as_tensor(ref_lens).to(device=dev, dtype=torch.int32).contiguous()
+    hyp_lens = torch.as_tensor(hyp_lens).to(device=dev, dtype=torch.int32).contiguous()
+    B, R, H = refs.size(0), refs.size(1), hyps.size(1)
+    if ref_lens.numel() != B or hyp_lens.numel() != B:
+        raise B200CTCError("ref_lens and hyp_lens must have one entry per pair")
+    lib = _lib.load()
+    word4 = torch.empty((B, 4), dtype=torch.int32, device=dev)
+    char4 = torch.empty((B, 4), dtype=torch.int32, device=dev)
+    counts = torch.empty((B, 2), dtype=torch.int32, device=dev)
+    n = ctypes.c_size_t()
+    _lib.check(lib.b200ctc_word_errors_workspace(B, R, H, ctypes.byref(n)), "b200ctc_word_errors_workspace")
+    with torch.cuda.device(dev):
+        ws = torch.empty(max(n.value, 1), dtype=torch.uint8, device=dev)
+        st = lib.b200ctc_word_errors(refs.data_ptr(), ref_stride, ref_lens.data_ptr(), hyps.data_ptr(), hyp_stride,
+                                     hyp_lens.data_ptr(), B, R, H,
+                                     int(space), word4.data_ptr(), char4.data_ptr(), counts.data_ptr(), ws.data_ptr(),
+                                     ws.numel(), torch.cuda.current_stream(dev).cuda_stream)
+        _lib.check(st, "b200ctc_word_errors")
+    return word4, char4, counts
+
+
 def compute_wer(ref, hyp, normalize=False, device="cuda"):
     """Drop-in for ``utils.evaluation.edit_distance.compute_wer`` (:53-126): ``ref`` / ``hyp`` are lists of
     hashable tokens (words, phones, characters).  Returns ``(wer, sub, ins, dele)``."""
@@ -104,7 +153,8 @@ def evaluate_batch(logits, x_lens, ys, y_lens, blank=0, label_offset=1, beam_wid
     stores them), y_lens ``[B]``.  The hypotheses are shifted by ``-label_offset`` exactly as ``CTC.decode`` does
     (``best_hyps -= 1``, ctc.py:444).  Returns ``(errors[B,4] int32 CUDA, hyp_tokens[B,T], hyp_lens[B])`` with
     errors = (distance, sub, ins, del) per utterance; ``errors.sum(0)`` over a data set divided by
-    ``y_lens.sum()`` gives PER / CER and its breakdown (phone.py:119-126).
+    ``y_lens.sum()`` gives PER / CER and its breakdown (phone.py:119-126), with spaces counted as tokens.  For the
+    WER of a character model pass ``ys`` and the returned hypotheses to ``word_errors``.
     With ``lm`` (an ``NGramLM``) every beam width, 1 included, decodes with the LM-fused beam search weighted by
     ``alpha`` and ``beta``; without one they must be 0."""
     if lm is not None:
