@@ -28,6 +28,9 @@
  *     independent (two CTC calls per step with different shapes --
  *     models/pytorch_v3/ctc/hierarchical_ctc.py:323-330 -- may share a handle
  *     because they are issued from one thread in order).
+ *   - a device workspace of at least the bytes its size query returns may
+ *     have any alignment: each call lays its regions out from the first
+ *     256-byte boundary inside the buffer.
  *   - all device work is enqueued on `stream` (a cudaStream_t passed as
  *     void*); nothing synchronises the host unless stated.
  *   - there is NO CPU fallback: if no CUDA device is usable the calls fail
@@ -140,7 +143,7 @@ B200CTC_API int b200ctc_get_workspace_bound(int T, int V, int B, int max_label_l
  *               +inf and an all-zero gradient.
  *   loss_sum    DEVICE fp32 [1] or NULL: sum_b costs[b] (ctc.py:50), fixed
  *               summation order.
- *   workspace   DEVICE, >= b200ctc_get_workspace_size bytes, 256-byte aligned.
+ *   workspace   DEVICE, >= b200ctc_get_workspace_size bytes.
  *
  * Limits: T * B rows, B * V * 4 < 2^31; label sequences of any length the fp64 safe lattice can hold in
  * shared memory (about 4000 labels); longer ones return B200CTC_STATUS_UNSUPPORTED.

@@ -22,6 +22,14 @@ constexpr int kStagingSlots = 4;
 constexpr int kGatherMinV = 129;  // V above this: the lattice reads gathered emission rows
 
 inline size_t align_up(size_t x) { return (x + kAlign - 1) / kAlign * kAlign; }
+// The caller's workspace may have any alignment: every `_workspace` query adds kAlign bytes to what the layout needs,
+// and the call lays the layout out from the first kAlign boundary of the buffer.  nullptr when fewer than `need`
+// bytes follow that boundary.
+unsigned char* aligned_workspace(void* workspace, size_t workspace_bytes, size_t need) {
+  const size_t lost = (kAlign - reinterpret_cast<uintptr_t>(workspace) % kAlign) % kAlign;
+  if (workspace_bytes < lost || workspace_bytes - lost < need) return nullptr;
+  return static_cast<unsigned char*>(workspace) + lost;
+}
 inline bool valid_dtype(int d) { return d == B200CTC_FLOAT32 || d == B200CTC_BFLOAT16 || d == B200CTC_FLOAT16; }
 
 // The call's host-prepared tables (utterance metadata, launch order, flags, labels: ~160 KB for C3) are
@@ -305,10 +313,8 @@ int b200ctc_loss_and_grad(b200ctc_handle* h, const float* acts, int64_t acts_str
   if (tot.sum_labels > 0x7fffffffLL) return B200CTC_STATUS_UNSUPPORTED;
   if ((long long)B * V * 4 > 0x7fffffffLL) return B200CTC_STATUS_UNSUPPORTED;   // frame stride of the gradient rows in bytes (int32 in the lattice)
   const WorkspaceLayout lay = make_layout(tot, T, B, V, tot.sum_labels);
-  unsigned char* ws = reinterpret_cast<unsigned char*>(
-      (reinterpret_cast<uintptr_t>(workspace) + kAlign - 1) / kAlign * kAlign);
-  const size_t lost = (size_t)(ws - reinterpret_cast<unsigned char*>(workspace));
-  if (workspace_bytes < lay.total + lost) return B200CTC_STATUS_WORKSPACE_TOO_SMALL;
+  unsigned char* ws = aligned_workspace(workspace, workspace_bytes, lay.total);
+  if (!ws) return B200CTC_STATUS_WORKSPACE_TOO_SMALL;
 
   // ---- plan cache: the same lengths and labels as the previous call on this stream? ------------
   int max_L = 0;
@@ -478,10 +484,8 @@ int b200ctc_loss_and_grad_dev_typed(b200ctc_handle* h, const void* acts, int64_t
   const bool staged = acts_dtype != B200CTC_FLOAT32 && grads;
   const WorkspaceLayout lay =
       make_layout(totals_from_bound(T, B, max_label_len), T, B, V, (long long)B * max_label_len, staged);
-  unsigned char* ws = reinterpret_cast<unsigned char*>(
-      (reinterpret_cast<uintptr_t>(workspace) + kAlign - 1) / kAlign * kAlign);
-  const size_t lost = (size_t)(ws - reinterpret_cast<unsigned char*>(workspace));
-  if (workspace_bytes < lay.total + lost) return B200CTC_STATUS_WORKSPACE_TOO_SMALL;
+  unsigned char* ws = aligned_workspace(workspace, workspace_bytes, lay.total);
+  if (!ws) return B200CTC_STATUS_WORKSPACE_TOO_SMALL;
 
   CallParams p;
   // a bfloat16 / float16 gradient is formed in fp32 in the staging region and rounded into `grads` by the last kernel
@@ -586,14 +590,15 @@ int b200ctc_beam_search_typed(const void* log_probs, int dtype, int64_t stride_b
     return B200CTC_STATUS_INVALID_VALUE;
   if (B == 0) return B200CTC_STATUS_SUCCESS;
   if (!lens || !out_lens || !workspace || (T > 0 && (!log_probs || !out_tokens))) return B200CTC_STATUS_INVALID_VALUE;
-  if (workspace_bytes < beam_search_workspace_bytes(B, T, V, beam_width)) return B200CTC_STATUS_WORKSPACE_TOO_SMALL;
+  unsigned char* ws = aligned_workspace(workspace, workspace_bytes, beam_search_workspace_bytes(B, T, V, beam_width));
+  if (!ws) return B200CTC_STATUS_WORKSPACE_TOO_SMALL;
   return status_of(launch_beam_search(log_probs, dtype, stride_b, stride_t, lens, T, V, B, blank, beam_width, out_tokens,
-                                      out_lens, out_scores, workspace, reinterpret_cast<cudaStream_t>(stream_v)));
+                                      out_lens, out_scores, ws, reinterpret_cast<cudaStream_t>(stream_v)));
 }
 
 int b200ctc_beam_search_lm_workspace(int B, int T, int V, int beam_width, size_t* bytes) {
   if (!bytes || B < 0 || T < 0 || V < 1 || beam_width < 1 || beam_width > 64) return B200CTC_STATUS_INVALID_VALUE;
-  *bytes = beam_search_lm_workspace_bytes(B, T, V, beam_width) + kAlign;
+  *bytes = beam_search_lm_workspace_bytes(B, T, V, beam_width, lm_n_words(V)) + kAlign;
   return B200CTC_STATUS_SUCCESS;
 }
 
@@ -609,9 +614,12 @@ int b200ctc_beam_search_lm(const void* log_probs, int dtype, int64_t stride_b, i
   if (B == 0) return B200CTC_STATUS_SUCCESS;
   if (!lens || !out_lens || !workspace || (T > 0 && (!log_probs || !out_tokens))) return B200CTC_STATUS_INVALID_VALUE;
   if ((long long)T * beam_width >= 0x3fffffffLL) return B200CTC_STATUS_UNSUPPORTED;   // trie node ids and hash slots
-  if (workspace_bytes < beam_search_lm_workspace_bytes(B, T, V, beam_width)) return B200CTC_STATUS_WORKSPACE_TOO_SMALL;
-  return status_of(launch_beam_search_lm(log_probs, dtype, stride_b, stride_t, lens, T, V, B, blank, beam_width,
-                                         ngram_lm_view(lm), alpha, beta, out_tokens, out_lens, out_scores, workspace,
+  const LmView view = ngram_lm_view(lm);
+  unsigned char* ws =
+      aligned_workspace(workspace, workspace_bytes, beam_search_lm_workspace_bytes(B, T, V, beam_width, view.n_words));
+  if (!ws) return B200CTC_STATUS_WORKSPACE_TOO_SMALL;
+  return status_of(launch_beam_search_lm(log_probs, dtype, stride_b, stride_t, lens, T, V, B, blank, beam_width, view,
+                                         alpha, beta, out_tokens, out_lens, out_scores, ws,
                                          reinterpret_cast<cudaStream_t>(stream_v)));
 }
 
@@ -628,9 +636,10 @@ int b200ctc_edit_distance(const int* refs, int ref_stride, const int* ref_lens, 
   if (B == 0) return B200CTC_STATUS_SUCCESS;
   if (!ref_lens || !hyp_lens || !out4 || !workspace || (max_ref > 0 && !refs) || (max_hyp > 0 && !hyps))
     return B200CTC_STATUS_INVALID_VALUE;
-  if (workspace_bytes < edit_distance_workspace_bytes(B, max_ref, max_hyp)) return B200CTC_STATUS_WORKSPACE_TOO_SMALL;
+  unsigned char* ws = aligned_workspace(workspace, workspace_bytes, edit_distance_workspace_bytes(B, max_ref, max_hyp));
+  if (!ws) return B200CTC_STATUS_WORKSPACE_TOO_SMALL;
   return status_of(launch_edit_distance(refs, ref_stride, ref_lens, hyps, hyp_stride, hyp_lens, B, max_ref, max_hyp, out4,
-                                        workspace, reinterpret_cast<cudaStream_t>(stream_v)));
+                                        ws, reinterpret_cast<cudaStream_t>(stream_v)));
 }
 
 // sizes up to 2^29 keep the word count and table size of word_errors_layout in int
@@ -654,10 +663,8 @@ int b200ctc_word_errors(const int* refs, int ref_stride, const int* ref_lens, co
   size_t need = 0;
   const int st = b200ctc_word_errors_workspace(B, max_ref, max_hyp, &need);
   if (st != B200CTC_STATUS_SUCCESS) return st;
-  // the word hashes are 64-bit: the layout starts on a 16-byte boundary inside the kAlign slack of the query
-  unsigned char* ws = reinterpret_cast<unsigned char*>((reinterpret_cast<uintptr_t>(workspace) + 15) / 16 * 16);
-  const size_t lost = (size_t)(ws - reinterpret_cast<unsigned char*>(workspace));
-  if (workspace_bytes < need - kAlign + lost) return B200CTC_STATUS_WORKSPACE_TOO_SMALL;
+  unsigned char* ws = aligned_workspace(workspace, workspace_bytes, need - kAlign);   // the layout without the query's slack
+  if (!ws) return B200CTC_STATUS_WORKSPACE_TOO_SMALL;
   return status_of(launch_word_errors(refs, ref_stride, ref_lens, hyps, hyp_stride, hyp_lens, B, max_ref, max_hyp, space,
                                       word4, char4, ref_counts, ws, reinterpret_cast<cudaStream_t>(stream_v)));
 }

@@ -116,6 +116,8 @@ __global__ void __launch_bounds__(kBeamThreads) beam_search_kernel(
   const int b = blockIdx.x, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const int n_frames = min(max(lens[b], 0), T);
   const E* lp_b = log_probs + (long long)b * stride_b;
+  // per-utterance strides of beam_layout (BeamLayout): derived here rather than passed, which keeps the kernels at
+  // their register counts without spills (a stride read from the parameters costs the LM-free kernel 10 registers)
   double* cand = cand_all + (long long)b * (kLM ? beam_width : kMaxBeam) * V;
   int2* nodes = nodes_all + (long long)b * ((long long)T * beam_width + 1);
   // ranking keys: the CTC value itself without the LM
@@ -329,93 +331,97 @@ __global__ void __launch_bounds__(kBeamThreads) beam_search_kernel(
   }
 }
 
-}  // namespace
-
-size_t beam_search_workspace_bytes(int B, int T, int V, int beam_width) {
-  const size_t cand = (size_t)B * kMaxBeam * (size_t)V * sizeof(double);
-  const size_t nodes = (size_t)B * ((size_t)T * beam_width + 1) * sizeof(int2);
-  return (cand + 255) / 256 * 256 + nodes;
-}
-
-namespace {
-
-// The LM instantiation's workspace: candidate values and keys, trie nodes, the trie's hash table, the LM rows.
-struct BeamLmLayout {
+// The workspace, for the LM-free search (n_words = 0) and the LM search (n_words: the LM's row width,
+// LmView::n_words).  Regions: the candidate values, the LM's ranking keys, the trie nodes, the LM's hash table and
+// rows; each starts on a 256-byte boundary and an LM region is empty without the LM.
+struct BeamLayout {
+  long long cand_stride;   // doubles of candidates (and of keys) per utterance
+  long long node_stride;   // trie nodes per utterance: the root and at most beam_width new ones a frame
+  long long row_stride;    // doubles of LM rows per utterance: beam_width rows of n_words
+  long long hash_cap;      // slots of the hash table per utterance: at least twice the nodes
   size_t off_keys, off_nodes, off_hash, off_rows, total;
-  long long hash_cap;
 };
 
-BeamLmLayout beam_lm_layout(int B, int T, int V, int beam_width) {
+BeamLayout beam_layout(int B, int T, int V, int beam_width, int n_words) {
   auto al = [](size_t x) { return (x + 255) / 256 * 256; };
-  BeamLmLayout l;
-  long long cap = 1;
-  while (cap < 2 * ((long long)T * beam_width + 1)) cap <<= 1;
-  l.hash_cap = cap;
-  const size_t cand = al((size_t)B * beam_width * (size_t)V * sizeof(double));
-  l.off_keys = cand;
-  l.off_nodes = l.off_keys + cand;
-  l.off_hash = l.off_nodes + al((size_t)B * ((size_t)T * beam_width + 1) * sizeof(int2));
-  l.off_rows = l.off_hash + al((size_t)B * (size_t)cap * sizeof(int));
-  l.total = l.off_rows + (size_t)B * beam_width * (size_t)(V + 3) * sizeof(double);
+  const bool lm = n_words > 0;
+  BeamLayout l;
+  l.cand_stride = (long long)(lm ? beam_width : kMaxBeam) * V;
+  l.node_stride = (long long)T * beam_width + 1;
+  l.row_stride = (long long)beam_width * n_words;
+  l.hash_cap = 0;
+  if (lm) {
+    l.hash_cap = 1;
+    while (l.hash_cap < 2 * l.node_stride) l.hash_cap <<= 1;
+  }
+  const size_t cand = (size_t)B * l.cand_stride * sizeof(double), nodes = (size_t)B * l.node_stride * sizeof(int2);
+  l.off_keys = al(cand);
+  l.off_nodes = l.off_keys + (lm ? al(cand) : 0);
+  l.off_hash = l.off_nodes + al(nodes);
+  l.off_rows = l.off_hash + al((size_t)B * l.hash_cap * sizeof(int));
+  l.total = lm ? l.off_rows + (size_t)B * l.row_stride * sizeof(double) : l.off_nodes + nodes;
   return l;
 }
 
+// lma: the LM, alpha and beta (kLM); its workspace pointers are filled in here
 template <bool kLM>
 cudaError_t launch(const void* log_probs, int dtype, long long stride_b, long long stride_t, const int* lens, int T, int V,
-                   int B, int blank, int beam_width, double* cand_all, int2* nodes_all, int* out_tokens, int* out_lens,
-                   float* out_scores, const BeamLmArgs& lma, cudaStream_t stream) {
+                   int B, int blank, int beam_width, int* out_tokens, int* out_lens, float* out_scores, void* workspace,
+                   BeamLmArgs lma, cudaStream_t stream) {
+  if (B == 0) return cudaSuccess;
+  if (beam_width < 1 || beam_width > kMaxBeam) return cudaErrorInvalidValue;
+  const BeamLayout l = beam_layout(B, T, V, beam_width, kLM ? lma.lm.n_words : 0);
+  unsigned char* ws = reinterpret_cast<unsigned char*>(workspace);
+  double* cand = reinterpret_cast<double*>(ws);
+  int2* nodes = reinterpret_cast<int2*>(ws + l.off_nodes);
+  if (kLM) {
+    lma.keys_all = reinterpret_cast<double*>(ws + l.off_keys);
+    lma.rows_all = reinterpret_cast<double*>(ws + l.off_rows);
+    lma.hash_all = reinterpret_cast<int*>(ws + l.off_hash);
+    lma.hash_cap = l.hash_cap;
+  }
   if (dtype == B200CTC_BFLOAT16)
     beam_search_kernel<__nv_bfloat16, kLM><<<B, kBeamThreads, 0, stream>>>(
-        static_cast<const __nv_bfloat16*>(log_probs), stride_b, stride_t, lens, T, V, blank, beam_width, cand_all,
-        nodes_all, out_tokens, out_lens, out_scores, lma);
+        static_cast<const __nv_bfloat16*>(log_probs), stride_b, stride_t, lens, T, V, blank, beam_width, cand,
+        nodes, out_tokens, out_lens, out_scores, lma);
   else if (dtype == B200CTC_FLOAT16)
     beam_search_kernel<__half, kLM><<<B, kBeamThreads, 0, stream>>>(
-        static_cast<const __half*>(log_probs), stride_b, stride_t, lens, T, V, blank, beam_width, cand_all, nodes_all,
-        out_tokens, out_lens, out_scores, lma);
+        static_cast<const __half*>(log_probs), stride_b, stride_t, lens, T, V, blank, beam_width, cand,
+        nodes, out_tokens, out_lens, out_scores, lma);
   else
     beam_search_kernel<float, kLM><<<B, kBeamThreads, 0, stream>>>(
-        static_cast<const float*>(log_probs), stride_b, stride_t, lens, T, V, blank, beam_width, cand_all, nodes_all,
-        out_tokens, out_lens, out_scores, lma);
+        static_cast<const float*>(log_probs), stride_b, stride_t, lens, T, V, blank, beam_width, cand,
+        nodes, out_tokens, out_lens, out_scores, lma);
   return cudaGetLastError();
 }
 
 }  // namespace
 
+size_t beam_search_workspace_bytes(int B, int T, int V, int beam_width) {
+  return beam_layout(B, T, V, beam_width, 0).total;
+}
+
 cudaError_t launch_beam_search(const void* log_probs, int dtype, long long stride_b, long long stride_t, const int* lens,
                                int T, int V, int B, int blank, int beam_width, int* out_tokens, int* out_lens,
                                float* out_scores, void* workspace, cudaStream_t stream) {
-  if (B == 0) return cudaSuccess;
-  if (beam_width < 1 || beam_width > kMaxBeam) return cudaErrorInvalidValue;
-  unsigned char* ws = reinterpret_cast<unsigned char*>(workspace);
-  const size_t cand = ((size_t)B * kMaxBeam * (size_t)V * sizeof(double) + 255) / 256 * 256;
-  return launch<false>(log_probs, dtype, stride_b, stride_t, lens, T, V, B, blank, beam_width,
-                       reinterpret_cast<double*>(ws), reinterpret_cast<int2*>(ws + cand), out_tokens, out_lens, out_scores,
-                       BeamLmArgs{}, stream);
+  return launch<false>(log_probs, dtype, stride_b, stride_t, lens, T, V, B, blank, beam_width, out_tokens, out_lens,
+                       out_scores, workspace, BeamLmArgs{}, stream);
 }
 
-size_t beam_search_lm_workspace_bytes(int B, int T, int V, int beam_width) {
-  return beam_lm_layout(B, T, V, beam_width).total;
+size_t beam_search_lm_workspace_bytes(int B, int T, int V, int beam_width, int n_words) {
+  return beam_layout(B, T, V, beam_width, n_words).total;
 }
 
 cudaError_t launch_beam_search_lm(const void* log_probs, int dtype, long long stride_b, long long stride_t,
                                   const int* lens, int T, int V, int B, int blank, int beam_width, const LmView& lm,
                                   double alpha, double beta, int* out_tokens, int* out_lens, float* out_scores,
                                   void* workspace, cudaStream_t stream) {
-  if (B == 0) return cudaSuccess;
-  if (beam_width < 1 || beam_width > kMaxBeam) return cudaErrorInvalidValue;
-  unsigned char* ws = reinterpret_cast<unsigned char*>(workspace);
-  const BeamLmLayout l = beam_lm_layout(B, T, V, beam_width);
-  BeamLmArgs a;
+  BeamLmArgs a{};
   a.lm = lm;
   a.alpha = alpha;
   a.beta = beta;
-  a.keys_all = reinterpret_cast<double*>(ws + l.off_keys);
-  a.rows_all = reinterpret_cast<double*>(ws + l.off_rows);
-  a.hash_all = reinterpret_cast<int*>(ws + l.off_hash);
-  a.hash_cap = l.hash_cap;
-  return launch<true>(log_probs, dtype, stride_b, stride_t, lens, T, V, B, blank, beam_width,
-                      reinterpret_cast<double*>(ws), reinterpret_cast<int2*>(ws + l.off_nodes), out_tokens, out_lens,
-                      out_scores, a, stream);
+  return launch<true>(log_probs, dtype, stride_b, stride_t, lens, T, V, B, blank, beam_width, out_tokens, out_lens,
+                      out_scores, workspace, a, stream);
 }
 
 }  // namespace b200ctc

@@ -129,7 +129,7 @@ cudaError_t launch_beam_search(const void* log_probs, int dtype, long long strid
                                int T, int V, int B, int blank, int beam_width, int* out_tokens, int* out_lens,
                                float* out_scores, void* workspace, cudaStream_t stream);
 struct LmView;   // ngram_lm.cuh
-size_t beam_search_lm_workspace_bytes(int B, int T, int V, int beam_width);
+size_t beam_search_lm_workspace_bytes(int B, int T, int V, int beam_width, int n_words);   // n_words: LmView::n_words
 cudaError_t launch_beam_search_lm(const void* log_probs, int dtype, long long stride_b, long long stride_t,
                                   const int* lens, int T, int V, int B, int blank, int beam_width, const LmView& lm,
                                   double alpha, double beta, int* out_tokens, int* out_lens, float* out_scores,

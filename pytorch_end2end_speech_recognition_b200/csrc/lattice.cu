@@ -10,10 +10,13 @@ namespace b200ctc {
 
 namespace {
 
-// What every utterance ends with (the CTA that owns it; at least 128 threads): the label-smoothing term of the
-// utterance and, in the CTA that finishes last, the fixed-order sum of the costs (K3).
+// What every utterance ends with (the CTA that owns it; at least kTailThreads threads): the label-smoothing term of
+// the utterance and, in the CTA that finishes last, the fixed-order sum of the costs (K3).  It reuses the dynamic
+// shared memory for kTailThreads partial sums in double.
+constexpr int kTailThreads = 128;   // the same summation order whatever the block size of the kernel variant
+constexpr size_t kTailSmemBytes = kTailThreads * sizeof(double);
 __device__ void utterance_tail(const CallParams& p, int b, const UttMeta& m, unsigned char* smem) {
-  constexpr int NT = 128;          // the same summation order whatever the block size of the kernel variant
+  constexpr int NT = kTailThreads;
   // A CTA that never needed K1's output (infeasible or empty utterance) still must not let this kernel complete
   // before K1 does: whatever follows in the stream is ordered behind THIS kernel.  A no-op for everybody else.
   pdl_wait_primary();
@@ -245,7 +248,7 @@ cudaError_t launch_apply_occupancy(const CallParams& p, cudaStream_t stream) {
 // ring grows with the label sequence, 256 * (L + 5) bytes per side), and the dynamic shared memory.
 // Longer utterances are evaluated by the fp64 safe lattice in the same launch.
 cudaError_t prepare_lattice(CallParams& p, int max_L, LatticeCfg* out) {
-  const size_t safe = safe_smem_bytes(max_L) > 256 * sizeof(double) ? safe_smem_bytes(max_L) : 256 * sizeof(double);
+  const size_t safe = safe_smem_bytes(max_L) > kTailSmemBytes ? safe_smem_bytes(max_L) : kTailSmemBytes;
   if (safe > kSmemBudget) return cudaErrorInvalidConfiguration;   // not even the safe lattice holds this label sequence
   // The deepest record ring whose shared memory still holds the longest label sequence; when none does, the
   // shallowest (largest capacity) and the longer utterances take the safe lattice.

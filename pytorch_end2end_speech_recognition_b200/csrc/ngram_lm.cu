@@ -174,7 +174,7 @@ int load_arpa(const char* path, const char* const* symbols, int V, int blank, Mo
   if (li == lines.size() || line(li) != "\\end\\") return B200CTC_STATUS_INVALID_VALUE;
 
   // ---- symbols -> words ----
-  const int BOS = V, EOS = V + 1, UNK = V + 2, NW = V + 3;
+  const int BOS = V, EOS = V + 1, UNK = V + 2, NW = lm_n_words(V);
   auto ws = word_id.find("<s>"), we = word_id.find("</s>");
   if (ws == word_id.end() || we == word_id.end()) return B200CTC_STATUS_INVALID_VALUE;
   std::vector<int> lm_word(word_id.size(), -1);   // file word -> LM word; -1: no symbol maps to it (dropped)
@@ -347,7 +347,7 @@ int b200ctc_ngram_lm_create(const char* arpa_path, const char* const* symbols, i
   h->view.uni_p = reinterpret_cast<const double*>(d + off_uni_p);
   h->view.uni_node = reinterpret_cast<const int*>(d + off_uni_node);
   h->view.word_of = reinterpret_cast<const int*>(d + off_word_of);
-  h->view.n_words = V + 3;
+  h->view.n_words = lm_n_words(V);
   h->view.order = m.order;
   h->view.bos_state = m.bos_state;
   h->view.eos = m.eos;

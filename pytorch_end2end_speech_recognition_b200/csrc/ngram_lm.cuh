@@ -14,6 +14,9 @@ namespace b200ctc {
 constexpr int kMaxLmOrder = 8;
 constexpr double kLn10 = 2.302585092994045684017991454684364208;   // the double nearest ln 10 (oracle/lm_ref.py: LN10)
 
+// The number of words of a model over V decoder symbols: the width of an LM row (LmView::n_words).
+constexpr int lm_n_words(int V) { return V + 3; }
+
 struct LmNode {
   double p;          // log10 p of the n-gram
   double bo;         // log10 back-off weight of the n-gram as a history (0 when the file gives none)
@@ -30,7 +33,7 @@ struct LmView {
   const double* uni_p;   // [n_words] log10 p of each unigram (0 for a word that is none: never read)
   const int* uni_node;   // [n_words] node of each unigram, -1 for a word that is none
   const int* word_of;    // [V] the word of each decoder id (-1 at blank)
-  int n_words;           // V + 3
+  int n_words;           // lm_n_words(V)
   int order;             // N
   int bos_state;         // the state of the empty prefix: <s> (order >= 2) or the empty history
   int eos;               // the word </s>

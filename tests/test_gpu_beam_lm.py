@@ -192,3 +192,47 @@ def test_mismatched_lm_is_rejected(tmp_path):
     lm.close()
     with pytest.raises(b200.B200CTCError):
         b200.beam_search_decode(lp, [10, 10], 4, lm=lm, alpha=1.0)                # closed
+
+
+def test_unaligned_workspace_gives_the_aligned_results(tmp_path):
+    """A C caller's workspace may have any alignment: the beam search, with and without the LM, called with the
+    queried workspace shifted by 4 bytes (and 4 bytes shorter) gives the tokens, lengths and scores of the call
+    with a 256-byte aligned one."""
+    import ctypes
+    from pytorch_end2end_speech_recognition_b200 import _lib
+    lib = _lib.load()
+    B, T, V, W = 3, 24, 12, 8
+    rng = np.random.RandomState(11)
+    path, symbols = _random_lm(tmp_path, V, 0, 3, seed=5)
+    lm = b200.NGramLM(path, symbols)
+    lp = _log_probs(rng, B, T, V, 0).cuda()
+    lens = torch.tensor([T, T - 5, 9], dtype=torch.int32, device="cuda")
+
+    def run(with_lm, shift):
+        n = ctypes.c_size_t()
+        query = lib.b200ctc_beam_search_lm_workspace if with_lm else lib.b200ctc_beam_search_workspace
+        assert query(B, T, V, W, ctypes.byref(n)) == 0
+        ws = torch.empty(n.value + 256, dtype=torch.uint8, device="cuda")
+        ptr, nbytes = ws.data_ptr() + shift, n.value - shift
+        assert ws.data_ptr() % 256 == 0
+        tokens = torch.empty((B, T), dtype=torch.int32, device="cuda")
+        out_lens = torch.empty(B, dtype=torch.int32, device="cuda")
+        scores = torch.empty(B, dtype=torch.float32, device="cuda")
+        stream = torch.cuda.current_stream().cuda_stream
+        if with_lm:
+            st = lib.b200ctc_beam_search_lm(lp.data_ptr(), 0, lp.stride(0), lp.stride(1), lens.data_ptr(), T, V, B, 0, W,
+                                            lm.handle, 0.8, 0.5, tokens.data_ptr(), out_lens.data_ptr(),
+                                            scores.data_ptr(), ptr, nbytes, stream)
+        else:
+            st = lib.b200ctc_beam_search_typed(lp.data_ptr(), 0, lp.stride(0), lp.stride(1), lens.data_ptr(), T, V, B, 0,
+                                               W, tokens.data_ptr(), out_lens.data_ptr(), scores.data_ptr(), ptr, nbytes,
+                                               stream)
+        assert st == 0
+        torch.cuda.synchronize()
+        return tokens.cpu(), out_lens.cpu(), scores.cpu()
+
+    for with_lm in (False, True):
+        aligned, shifted = run(with_lm, 0), run(with_lm, 4)
+        for a, s in zip(aligned, shifted):
+            assert torch.equal(a, s), with_lm
+    lm.close()

@@ -207,7 +207,8 @@ def test_poisoned_workspace_gives_the_clean_results():
     clean = call(torch.zeros(n.value, dtype=torch.uint8, device="cuda"))
     g = torch.Generator(device="cuda").manual_seed(17)
     poisoned = torch.randint(0, 256, (n.value,), dtype=torch.uint8, device="cuda", generator=g)
-    for ws in (poisoned, poisoned, torch.full((n.value,), 0xff, dtype=torch.uint8, device="cuda")):
+    # the last: 4 bytes past a 256-byte boundary and 4 bytes short of the query (any alignment is accepted)
+    for ws in (poisoned, poisoned, torch.full((n.value,), 0xff, dtype=torch.uint8, device="cuda"), poisoned[4:]):
         for x, y in zip(clean, call(ws)):
             assert torch.equal(x, y)
     for b in range(B):
